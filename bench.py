@@ -28,6 +28,10 @@ Legs of the CUDA arm
          resampling creates it (extent copies), with whole-grid copies (what Map::clone moves) and
          with the reference's order of work; results are identical in all modes.
   cpu_baseline  (N=1, rank 0) the CPU oracle on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what the `value` leg's filter holds after its last timed step (resample indices, argmax,
+normalised weights, all poses, published pose and map; see step_outputs) as DIR/<name>.npy. Scans and random draws
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -67,7 +71,14 @@ def parse_args():
     ap.add_argument("--c5-leg", action="store_true", help="run the configs[4] shard leg at any GPU count")
     ap.add_argument("--flags", type=int, default=0, help="slamrs_flags bits for the main run (profiling)")
     ap.add_argument("--shift-x-cells", type=int, default=0, help="experiment: move the map origin by this many cells in x")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (CUDA arm)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm")
+    return args
 
 
 # ------------------------------------------------------------------------------ helpers
@@ -204,13 +215,11 @@ def workload_config(wl, n_gpus, n_total):
 
 
 # ------------------------------------------------------------------------------ CUDA arm
-def state_hash(slam, world, dev):
-    """SHA-256 over what a step leaves behind: the resample index vector, the argmax, the poses of the whole
-    population, the published pose and the published map. Equal hashes = identical filter state."""
-    import hashlib
+def step_outputs(slam, world, dev):
+    """What a caller holds after a step: the resample index vector, the argmax, the normalised weights, the poses of
+    the whole population, the published pose and the published map (row-major, grid_w x grid_h)."""
     import torch
     import torch.distributed as dist
-    idx = slam.resample_indices()
     poses = torch.from_numpy(slam.poses()).to(dev)
     if world > 1:
         parts = [torch.empty_like(poses) for _ in range(world)]
@@ -218,10 +227,51 @@ def state_hash(slam, world, dev):
         poses = torch.cat(parts)
     ep = slam.estimated_pose()
     m = slam.estimated_likelihood().data          # collective: every rank reads the owner's grid
+    return {"resample_indices": slam.resample_indices(), "max_particle": np.array([slam.max_particle], np.uint64),
+            "weights": slam.weights()[0], "poses": poses.cpu().numpy(),
+            "estimated_pose": np.array([ep.x, ep.y, ep.theta], np.float32),
+            "estimated_likelihood": m.reshape(slam.grid_w, slam.grid_h)}
+
+
+def state_hash(outputs):
+    """SHA-256 over what a step leaves behind (step_outputs without the weights). Equal hashes = identical filter
+    state."""
+    import hashlib
     h = hashlib.sha256()
-    h.update(idx.tobytes()); h.update(np.uint64(slam.max_particle).tobytes()); h.update(poses.cpu().numpy().tobytes())
-    h.update(np.array([ep.x, ep.y, ep.theta], np.float32).tobytes()); h.update(m.tobytes())
+    for name in ("resample_indices", "max_particle", "poses", "estimated_pose", "estimated_likelihood"):
+        h.update(outputs[name].tobytes())
     return h.hexdigest()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, outputs):
+    """Writes every output as <path>/<name>.npy: float32 stays float32, everything else becomes float64 (indices
+    and counts are exact below 2**53). All files together hold at most 64 MB: an output larger than its share is
+    replaced by a fixed, seeded sample of its elements, so that two runs still compare element for element."""
+    os.makedirs(path, exist_ok=True)
+    items = sorted(outputs.items(), key=lambda kv: kv[1].nbytes)
+    left = DUMP_BYTES - 4096 * len(items)         # room for the .npy headers
+    for i, (name, a) in enumerate(items):
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            keep = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
+
+
+STEP_HISTORY = 256   # per-step records the library keeps (include/slamrs_gpu.h)
+
+
+def step_history(slam, first, count):
+    """The per-step records of steps first .. first+count-1 as float64. A run longer than the library's ring
+    repeats the records of its last STEP_HISTORY steps, so that sums over the rows still stand for `count` steps."""
+    n = min(count, STEP_HISTORY)
+    hist = slam.step_history(first + count - n, n).astype(np.float64)
+    return np.resize(hist, (count, hist.shape[1]))
 
 
 def measure_e2e_pipelined(args, wl, rank, world, local, dev, nccl_id, scans, flags):
@@ -326,10 +376,11 @@ def measure_cuda(args, wl, rank, world, local, dev, nccl_id, scans, flags, do_e2
     out = {"ms_value": e0.elapsed_time(e1), "launches": slam.launch_count - launches0, "grid_bytes": grid_bytes}
     out["phase_ms"], _ = slam.phase_ms()
     slam.set_profiling(False)
-    out["hist"] = slam.step_history(W, K).astype(np.float64)
+    out["hist"] = step_history(slam, W, K)
     out["stats"] = slam.stats()
     out["grid"] = (slam.grid_w, slam.grid_h)
-    out["state_sha256"] = state_hash(slam, world, dev)
+    out["outputs"] = step_outputs(slam, world, dev)
+    out["state_sha256"] = state_hash(out["outputs"])
 
     if do_e2e:
         pinned = torch.empty(slam.grid_w * slam.grid_h, dtype=torch.float64).pin_memory()
@@ -392,7 +443,7 @@ def measure_cuda(args, wl, rank, world, local, dev, nccl_id, scans, flags, do_e2
         e1.record(stream)
         slam.sync()
         barrier()
-        hist = slam.step_history(step0, K).astype(np.float64)
+        hist = step_history(slam, step0, K)
         out["aged"] = {"ms": e0.elapsed_time(e1), "scans_before": int(step0), "extent": slam.map_extent(),
                        "particles_integrated_per_step": float(hist[:, 4].mean()), "copy_bytes_per_step": float(hist[:, 5].mean())}
     slam.close()
@@ -663,6 +714,8 @@ def run_cuda(args, wl, rank, world, local):
                                         "values bracket it. `value` (all host threads, no dead transform) is the generous "
                                         "figure and the one the --impl reference arm reports, i.e. what the driver's "
                                         "vs_reference ratio divides by"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main["outputs"])
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

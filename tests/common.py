@@ -13,6 +13,12 @@ WEIGHT_RTOL = 1e-9   # stated tolerance of the contract is 1e-5 relative; we hol
 ODDS_RTOL = 1e-12
 
 
+def gpu_present() -> bool:
+    """Whether the CUDA driver reports a device (device node names differ between hosts and containers)."""
+    import torch
+    return torch.cuda.device_count() > 0
+
+
 def make_scans(scene_scale, n_beams, scanner_range, steps, wheel_base=0.1, speed=(0.08, 0.10)):
     sim = Simulator(reference_scene(scene_scale), n_beams=n_beams, scanner_range=scanner_range, wheel_base=wheel_base)
     return [sim.next_scan(*speed) for _ in range(steps)]

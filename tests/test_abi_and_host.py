@@ -13,6 +13,8 @@ from slamrs_b200 import _lib
 from slamrs_b200.simulator import Simulator, reference_scene, scan
 from slamrs_b200.workloads import WORKLOADS
 
+from common import gpu_present
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -49,7 +51,7 @@ def test_product_does_not_touch_the_oracle():
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), f
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="GPU present")
+@pytest.mark.skipif(gpu_present(), reason="GPU present")
 def test_no_gpu_means_loud_error_not_fallback():
     with pytest.raises(_lib.SlamrsGpuError) as e:
         slamrs_b200.GridMapSlam(slamrs_b200.GridMapSlamConfig(n_particles=4))

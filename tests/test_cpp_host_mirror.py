@@ -10,7 +10,7 @@ import pytest
 from slamrs_b200 import GridMapSlam, GridMapSlamConfig, Odometry
 from slamrs_b200 import _lib
 
-from common import make_scans
+from common import gpu_present, make_scans
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "tests", "cpp", "host_mirror_check")
@@ -26,7 +26,7 @@ def _build():
     return BIN
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="GPU present")
+@pytest.mark.skipif(gpu_present(), reason="GPU present")
 def test_cpp_mirror_builds_and_refuses_to_run_without_gpu():
     out = subprocess.run([_build(), "--no-gpu"], capture_output=True, text=True)
     assert out.returncode == 0, out.stdout + out.stderr
