@@ -230,6 +230,37 @@ int slamrs_gpu_sim_scan(slamrs_gpu_handle* h, const float* segments_xyxy, uint32
 int slamrs_gpu_get_scan(slamrs_gpu_handle* h, float* out_angle, float* out_dist, uint8_t* out_valid, uint32_t cap,
                         uint32_t* out_n);
 
+/* ------------------------------------------------------------------ localisation on a loaded map */
+
+/* Monte Carlo localisation: GridMapSlam::update (slam.rs:46-75) with the map held fixed and shared by every particle
+ * -- no integration, no per-particle grids (about 100 bytes per particle instead of a grid each). The beam term of
+ * each endpoint comes from a per-cell table built on the device at create from the loaded map and a sensor model:
+ *   SLAMRS_SENSOR_BEAM_ENDPOINT  the reference's Map::probability_of factor (map.rs:130-141): log(0.9 p + 0.1), 0 for
+ *                                p == 0.5 and for endpoints off the grid. Unknown space scores best, so this model
+ *                                cannot localise from a uniform start; it is there for parity with the SLAM step.
+ *   SLAMRS_SENSOR_LIKELIHOOD_FIELD  log(z_hit exp(-d^2 / (2 sigma^2)) + z_rand), d = distance from the endpoint's cell
+ *                                to the nearest cell with p > occupied_above (exact, in cells, times the resolution);
+ *                                log(z_rand) off the grid. The model for global localisation. */
+enum slamrs_sensor_kind { SLAMRS_SENSOR_BEAM_ENDPOINT = 0, SLAMRS_SENSOR_LIKELIHOOD_FIELD = 1 };
+typedef struct slamrs_gpu_sensor_model {
+    uint32_t struct_size;    /* = sizeof(slamrs_gpu_sensor_model) */
+    uint32_t kind;           /* enum slamrs_sensor_kind */
+    float sigma;             /* likelihood field: std. dev. of the hit Gaussian, metres */
+    float z_rand;            /* likelihood field: weight of the uniform term, (0, 1); z_hit = 1 - z_rand */
+    float occupied_above;    /* likelihood field: obstacle iff p > occupied_above, [0.5, 1) */
+} slamrs_gpu_sensor_model;
+
+/* A handle in localiser mode on the grid_w * grid_h probabilities map_probability (index row * grid_h + column, what
+ * slamrs_gpu_map_probability writes). Uses position, resolution, grid size, n_particles, seed, rng_mode, device and
+ * resample_threshold of cfg; world_size must be 1 and flags, slot_cells and spare_slots 0. Particles start at
+ * Pose::default(); place them with init_uniform or set_poses. update / step_async / pose / weights and the other
+ * particle accessors work as on a SLAM handle (step_async launches three kernels); the grid accessors (map_*,
+ * get_cells, set_cells, get_log_odds, get_extents, get_slots, get_step_history) return SLAMRS_E_INVALID_ARG. */
+int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_sensor_model* model,
+                                const double* map_probability, slamrs_gpu_handle** out);
+/* the localiser's grid_w * grid_h term table (f64, index row * grid_h + column), for tests */
+int slamrs_gpu_get_sensor_terms(slamrs_gpu_handle* h, double* out_cells);
+
 /* ------------------------------------------------------------------ introspection (tests, bench) */
 
 const char* slamrs_gpu_last_error(const slamrs_gpu_handle* h); /* never NULL; "" when none */

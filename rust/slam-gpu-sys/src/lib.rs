@@ -30,6 +30,9 @@ pub const SLAMRS_MAP_F32: u32 = 1;
 pub const SLAMRS_MAP_U8: u32 = 2;
 pub const SLAMRS_HISTORY_VALUES: usize = 8;
 
+pub const SLAMRS_SENSOR_BEAM_ENDPOINT: u32 = 0;
+pub const SLAMRS_SENSOR_LIKELIHOOD_FIELD: u32 = 1;
+
 #[repr(C)]
 pub struct slamrs_gpu_handle {
     _private: [u8; 0],
@@ -76,6 +79,16 @@ pub struct slamrs_gpu_stats {
     pub resample_exact_fallback: u64,
     pub resample_fold_rounds: u64,
     pub resampled: u64,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_sensor_model {
+    pub struct_size: u32,
+    pub kind: u32,
+    pub sigma: f32,
+    pub z_rand: f32,
+    pub occupied_above: f32,
 }
 
 extern "C" {
@@ -125,5 +138,7 @@ extern "C" {
     pub fn slamrs_gpu_get_cells(h: *mut slamrs_gpu_handle, particle: u64, out_cells: *mut u32) -> c_int;
     pub fn slamrs_gpu_set_cells(h: *mut slamrs_gpu_handle, particle: u64, cells: *const u32) -> c_int;
     pub fn slamrs_gpu_get_extents(h: *mut slamrs_gpu_handle, particle: u64, out_box_shift: *mut i32, out_bands: *mut u32, out_n_bands: *mut u32) -> c_int;
+    pub fn slamrs_gpu_create_localizer(cfg: *const slamrs_gpu_config, model: *const slamrs_gpu_sensor_model, map_probability: *const f64, out: *mut *mut slamrs_gpu_handle) -> c_int;
+    pub fn slamrs_gpu_get_sensor_terms(h: *mut slamrs_gpu_handle, out_cells: *mut f64) -> c_int;
     pub fn slamrs_gpu_get_log_odds(h: *mut slamrs_gpu_handle, particle: u64, out_cells: *mut f64) -> c_int;
 }

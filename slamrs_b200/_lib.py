@@ -34,8 +34,10 @@ EXPORTS = [
     "slamrs_gpu_effective_particles", "slamrs_gpu_sim_scan", "slamrs_gpu_get_scan", "slamrs_gpu_get_slots",
     "slamrs_gpu_get_extents", "slamrs_gpu_debug_resample", "slamrs_gpu_init_uniform",
     "slamrs_gpu_map_probability_async", "slamrs_gpu_map_wait",
+    "slamrs_gpu_create_localizer", "slamrs_gpu_get_sensor_terms",
 ]
 MAP_F64, MAP_F32, MAP_U8 = 0, 1, 2
+SENSOR_BEAM_ENDPOINT, SENSOR_LIKELIHOOD_FIELD = 0, 1
 PHASES = ["motion_likelihood", "all_gather", "resample", "materialize", "ray_update", "pull", "copy"]
 
 
@@ -51,6 +53,11 @@ class Config(C.Structure):
         ("slot_cells", C.c_uint32), ("resample_threshold", C.c_float),
         ("nccl_id", C.c_uint8 * NCCL_ID_BYTES),
     ]
+
+
+class SensorModel(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("kind", C.c_uint32), ("sigma", C.c_float), ("z_rand", C.c_float),
+                ("occupied_above", C.c_float)]
 
 
 class Stats(C.Structure):
@@ -125,6 +132,9 @@ def load():
     L.slamrs_gpu_get_slots.restype = i; L.slamrs_gpu_get_slots.argtypes = [vp, vp, vp, C.POINTER(u32)]
     L.slamrs_gpu_get_extents.restype = i; L.slamrs_gpu_get_extents.argtypes = [vp, u64, vp, vp, C.POINTER(u32)]
     L.slamrs_gpu_init_uniform.restype = i; L.slamrs_gpu_init_uniform.argtypes = [vp, vp]
+    L.slamrs_gpu_create_localizer.restype = i
+    L.slamrs_gpu_create_localizer.argtypes = [C.POINTER(Config), C.POINTER(SensorModel), vp, C.POINTER(vp)]
+    L.slamrs_gpu_get_sensor_terms.restype = i; L.slamrs_gpu_get_sensor_terms.argtypes = [vp, vp]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
     _lib = L

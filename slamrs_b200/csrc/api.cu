@@ -130,6 +130,10 @@ struct slamrs_gpu_handle {
     uint64_t launches = 0;
     uint64_t window_cells = 0;
     std::string last_error;
+    // localiser mode (slamrs_gpu_create_localizer): one shared map as a per-cell term table, no grids
+    bool localizer = false;
+    double* d_loc_terms = nullptr;   // n_cells
+    double loc_outside = 0.0;        // term of an endpoint off the grid
 };
 
 namespace {
@@ -281,7 +285,7 @@ void free_all(slamrs_gpu_handle* h) {
     cudaFree(h->d_pool);
     cudaFree(h->d_slot[0]); cudaFree(h->d_slot[1]);
     cudaFree(h->d_pose[0]); cudaFree(h->d_pose[1]);
-    cudaFree(h->d_term_table);
+    cudaFree(h->d_term_table); cudaFree(h->d_loc_terms);
     cudaFree(h->d_wnorm); cudaFree(h->d_cum); cudaFree(h->d_idx); cudaFree(h->d_fold); cudaFree(h->d_carry);
     cudaFree(h->d_angle);   // (d_dist and d_valid live in the same allocation)
     if (h->h_scan_stage) cudaFreeHost(h->h_scan_stage);
@@ -312,6 +316,8 @@ void free_all(slamrs_gpu_handle* h) {
     cudaGetLastError();
     delete h;
 }
+
+constexpr const char* NO_GRIDS = "a localizer has no particle grids";
 
 int ensure_beam_capacity(slamrs_gpu_handle* h, uint32_t n) {
     if (n <= h->beam_cap) return SLAMRS_OK;
@@ -403,6 +409,38 @@ int fetch_counters(slamrs_gpu_handle* h) {
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     CU_TRY(h, cudaGetLastError());
     h->counters_fresh = true;
+    return SLAMRS_OK;
+}
+
+// One localisation step (localiser mode): motion + likelihood against the term table, then the SLAM step's own
+// weights and resampling kernels without a survivor list -- three launches, chained by programmatic dependent launch.
+int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
+    cudaStream_t s = h->stream;
+    if (h->profiling && h->prof_recorded == PROF_RING) {
+        int prc = prof_flush(h);
+        if (prc) return prc;
+    }
+    const int cur = h->cur, nxt = cur ^ 1;
+    const ScanDevice scan = h->scan_external ? ScanDevice{h->ext_angle, h->ext_dist, h->ext_valid, h->n_beams, nullptr}
+                                             : ScanDevice{h->d_angle, h->d_dist, h->d_valid, h->n_beams, nullptr};
+    PROF_MARK(h, 0);
+    launch_loc_step(s, h->geom, od, scan, h->d_pose[cur], h->d_results, h->n_total, caller ? h->d_z : nullptr, h->cfg.seed,
+                    h->step, h->d_loc_terms, h->loc_outside, h->d_carry, h->d_counters);
+    PROF_MARK(h, 1);
+    PROF_MARK(h, 2);
+    launch_weights(s, h->d_results, h->n_total, h->d_wnorm, h->d_cum, h->d_fold, (double)h->cfg.resample_threshold, h->d_counters);
+    launch_resample_indices(s, h->d_results, h->d_cum, h->n_total, caller ? h->d_u : nullptr, h->cfg.seed, h->step, h->d_idx,
+                            h->d_pose[nxt], 0, h->n_total, false, nullptr,
+                            RayLists{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u}, h->d_wnorm, h->d_carry,
+                            h->d_counters);
+    h->launches += 3;
+    for (uint32_t m = 3; m < PROF_MARKS; ++m) PROF_MARK(h, m);
+    if (h->profiling) h->prof_recorded++;
+    CU_TRY(h, cudaGetLastError());
+    h->cur = nxt;
+    h->step++;
+    h->counters_fresh = false;
+    h->mirror_by_step = false;
     return SLAMRS_OK;
 }
 
@@ -657,6 +695,139 @@ int slamrs_gpu_create(const slamrs_gpu_config* cfg, slamrs_gpu_handle** out) {
     return SLAMRS_OK;
 }
 
+int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_sensor_model* model,
+                                const double* map_probability, slamrs_gpu_handle** out) {
+    if (!out) return fail(nullptr, SLAMRS_E_INVALID_ARG, "null output pointer");
+    *out = nullptr;
+    if (!cfg) return fail(nullptr, SLAMRS_E_INVALID_ARG, "null config");
+    if (!model) return fail(nullptr, SLAMRS_E_INVALID_ARG, "null sensor model");
+    if (!map_probability) return fail(nullptr, SLAMRS_E_INVALID_ARG, "null map_probability");
+    if (cfg->struct_size != sizeof(slamrs_gpu_config) || cfg->abi_version != SLAMRS_GPU_ABI_VERSION)
+        return fail(nullptr, SLAMRS_E_INVALID_ARG, "slamrs_gpu_config size/ABI version mismatch");
+    if (model->struct_size != sizeof(slamrs_gpu_sensor_model))
+        return fail(nullptr, SLAMRS_E_INVALID_ARG, "slamrs_gpu_sensor_model struct_size mismatch");
+    if (cfg->n_particles == 0) return fail(nullptr, SLAMRS_E_INVALID_ARG, "Must have at least one particle");
+    if (cfg->n_particles > 0x7fffffffull) return fail(nullptr, SLAMRS_E_INVALID_ARG, "too many particles");
+    if (cfg->world_size != 1 || cfg->rank != 0)
+        return fail(nullptr, SLAMRS_E_INVALID_ARG, "world_size must be 1 and rank 0: a localizer runs on one GPU");
+    if (cfg->flags != 0) return fail(nullptr, SLAMRS_E_INVALID_ARG, "flags must be 0 for a localizer");
+    if (cfg->slot_cells != 0) return fail(nullptr, SLAMRS_E_INVALID_ARG, "slot_cells must be 0 for a localizer");
+    if (cfg->spare_slots != 0) return fail(nullptr, SLAMRS_E_INVALID_ARG, "spare_slots must be 0 for a localizer");
+    if (cfg->grid_w == 0 || cfg->grid_w != cfg->grid_h)
+        return fail(nullptr, SLAMRS_E_INVALID_ARG, "grid_w and grid_h must be equal and non-zero (square grid)");
+    if ((uint64_t)cfg->grid_w * cfg->grid_h > 0x7fffffffull) return fail(nullptr, SLAMRS_E_INVALID_ARG, "grid too large");
+    if (!(cfg->resolution > 0.0f)) return fail(nullptr, SLAMRS_E_INVALID_ARG, "resolution must be positive");
+    if (cfg->rng_mode > SLAMRS_RNG_CALLER) return fail(nullptr, SLAMRS_E_INVALID_ARG, "unknown rng_mode");
+    if (!(cfg->resample_threshold >= 0.0f && cfg->resample_threshold <= 1.0f))
+        return fail(nullptr, SLAMRS_E_INVALID_ARG, "resample_threshold must be 0 (always resample) or in (0, 1]");
+    if (model->kind > SLAMRS_SENSOR_LIKELIHOOD_FIELD) return fail(nullptr, SLAMRS_E_INVALID_ARG, "unknown sensor model kind");
+    const bool field = model->kind == SLAMRS_SENSOR_LIKELIHOOD_FIELD;
+    if (field) {
+        if (!(model->sigma > 0.0f) || !isfinite(model->sigma))
+            return fail(nullptr, SLAMRS_E_INVALID_ARG, "sigma must be a positive finite number of metres");
+        if (!(model->z_rand > 0.0f && model->z_rand < 1.0f))
+            return fail(nullptr, SLAMRS_E_INVALID_ARG, "z_rand must lie in (0, 1)");
+        if (!(model->occupied_above >= 0.5f && model->occupied_above < 1.0f))
+            return fail(nullptr, SLAMRS_E_INVALID_ARG, "occupied_above must lie in [0.5, 1)");
+    }
+    const size_t n_cells = (size_t)cfg->grid_w * cfg->grid_h;
+    for (size_t i = 0; i < n_cells; ++i)
+        if (!(map_probability[i] >= 0.0 && map_probability[i] <= 1.0))
+            return fail(nullptr, SLAMRS_E_INVALID_ARG,
+                        "map_probability[" + std::to_string(i) + "] is NaN or outside [0, 1]");
+
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
+        cudaGetLastError();
+        return fail(nullptr, SLAMRS_E_NO_DEVICE, "no CUDA device visible; this library has no CPU fallback");
+    }
+    int device = cfg->device;
+    if (device < 0) cudaGetDevice(&device);
+    if (device >= n_dev) return fail(nullptr, SLAMRS_E_INVALID_ARG, "device ordinal out of range");
+
+    slamrs_gpu_handle* h = new (std::nothrow) slamrs_gpu_handle();
+    if (!h) return fail(nullptr, SLAMRS_E_OUT_OF_MEMORY, "host allocation failed");
+    h->cfg = *cfg;
+    h->localizer = true;
+    h->device = device;
+    h->n_total = h->n_local = (uint32_t)cfg->n_particles;
+    h->n_cells = (uint32_t)n_cells;
+    h->geom = make_map_geom(cfg->pos_x, cfg->pos_y, cfg->resolution, cfg->grid_w, cfg->grid_h);
+    h->loc_outside = field ? log((double)model->z_rand) : 0.0;   // ln(z_rand) / the reference's ln(1) for off-grid endpoints
+
+#define CREATE_CU(expr)                                                                                   \
+    do {                                                                                                  \
+        cudaError_t _e = (expr);                                                                          \
+        if (_e != cudaSuccess) {                                                                          \
+            const int _code = (_e == cudaErrorMemoryAllocation) ? SLAMRS_E_OUT_OF_MEMORY : SLAMRS_E_CUDA; \
+            g_create_error = std::string(#expr) + ": " + cudaGetErrorString(_e);                          \
+            cudaGetLastError();                                                                           \
+            cudaFree(scratch);                                                                            \
+            free_all(h);                                                                                  \
+            return _code;                                                                                 \
+        }                                                                                                 \
+    } while (0)
+
+    uint32_t* scratch = nullptr;   // the distance transform's column pass (freed before returning)
+    DeviceGuard guard(device);
+    cudaDeviceProp prop;
+    CREATE_CU(cudaGetDeviceProperties(&prop, device));
+    h->num_sms = prop.multiProcessorCount;
+    if (prop.major < 10) {
+        g_create_error = "this library is built for sm_100a (B200) only";
+        free_all(h);
+        return SLAMRS_E_NO_DEVICE;
+    }
+    CREATE_CU(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
+    CREATE_CU(configure_kernels());
+    // [ParticleResult x n | StepCounters], zeroed
+    h->off_counters = (sizeof(ParticleResult) * (size_t)h->n_total + 255) & ~(size_t)255;
+    const size_t pool_bytes = h->off_counters + sizeof(StepCounters);
+    CREATE_CU(cudaMalloc(&h->d_pool, pool_bytes));
+    CREATE_CU(cudaMemsetAsync(h->d_pool, 0, pool_bytes, h->stream));
+    h->d_results_base = h->d_results = (ParticleResult*)h->d_pool;
+    h->d_counters = (StepCounters*)((char*)h->d_pool + h->off_counters);
+    for (int i = 0; i < 2; ++i) {
+        CREATE_CU(cudaMalloc(&h->d_pose[i], sizeof(float) * 3 * h->n_total));
+        CREATE_CU(cudaMemsetAsync(h->d_pose[i], 0, sizeof(float) * 3 * h->n_total, h->stream));  // Pose::default()
+    }
+    CREATE_CU(cudaMalloc(&h->d_wnorm, sizeof(double) * h->n_total));
+    CREATE_CU(cudaMalloc(&h->d_cum, sizeof(double) * h->n_total));
+    CREATE_CU(cudaMalloc(&h->d_idx, sizeof(uint32_t) * h->n_total));
+    CREATE_CU(cudaMalloc(&h->d_fold, sizeof(double) * weights_scratch_doubles()));
+    if (cfg->resample_threshold > 0.0f) CREATE_CU(cudaMalloc(&h->d_carry, sizeof(double) * h->n_total));
+    CREATE_CU(cudaMemsetAsync(h->d_wnorm, 0, sizeof(double) * h->n_total, h->stream));
+    CREATE_CU(cudaMemsetAsync(h->d_idx, 0, sizeof(uint32_t) * h->n_total, h->stream));
+    if (cfg->rng_mode == SLAMRS_RNG_CALLER) {
+        CREATE_CU(cudaMalloc(&h->d_z, sizeof(double) * 2 * h->n_total));
+        CREATE_CU(cudaMalloc(&h->d_u, sizeof(double)));
+    }
+    CREATE_CU(cudaMallocHost(&h->h_counters, sizeof(StepCounters)));
+    memset(h->h_counters, 0, sizeof(StepCounters));
+    // d_export: the map's upload buffer here, sim_scan's segment scratch later (as on a SLAM handle)
+    CREATE_CU(cudaMalloc(&h->d_export, sizeof(double) * n_cells));
+    CREATE_CU(cudaMemcpyAsync(h->d_export, map_probability, sizeof(double) * n_cells, cudaMemcpyHostToDevice, h->stream));
+    CREATE_CU(cudaMalloc(&h->d_loc_terms, sizeof(double) * n_cells));
+    if (field) CREATE_CU(cudaMalloc(&scratch, sizeof(uint32_t) * n_cells));
+    CREATE_CU(launch_loc_terms(h->stream, h->d_export, cfg->grid_w, field ? 1 : 0, model->sigma, model->z_rand,
+                               model->occupied_above, cfg->resolution, scratch, h->d_loc_terms));
+    h->launches += field ? 2 : 1;
+    CREATE_CU(cudaStreamSynchronize(h->stream));
+    cudaFree(scratch);
+#undef CREATE_CU
+    *out = h;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_get_sensor_terms(slamrs_gpu_handle* h, double* out_cells) {
+    if (!h || !out_cells) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no sensor-term table (only a localizer has one)");
+    DeviceGuard g(h->device);
+    CU_TRY(h, cudaMemcpyAsync(out_cells, h->d_loc_terms, sizeof(double) * h->n_cells, cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    return SLAMRS_OK;
+}
+
 void slamrs_gpu_destroy(slamrs_gpu_handle* h) {
     if (h && getenv("SLAMRS_RAY_TRACE_PRINT")) {
         unsigned long long tr[18];
@@ -734,6 +905,7 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
         CU_TRY(h, cudaMemcpyAsync(h->d_z, z_draws, sizeof(double) * 2 * h->n_total, cudaMemcpyHostToDevice, s));
         CU_TRY(h, cudaMemcpyAsync(h->d_u, resample_u, sizeof(double), cudaMemcpyHostToDevice, s));
     }
+    if (h->localizer) return loc_step_async(h, od, caller);
     // beam order for the ray kernel (side stream, concurrent with the likelihood kernel); scans with
     // more beams than the sort handles keep scan order
     const bool sorted = h->n_beams > 32u && h->n_beams <= SORT_MAX_BEAMS;
@@ -1011,12 +1183,14 @@ int export_window(slamrs_gpu_handle* h, uint32_t format, int x0, int y0, int x1,
 
 int slamrs_gpu_map_probability(slamrs_gpu_handle* h, double* out_cells) {
     if (!h || (!out_cells && h->world == 1)) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     return export_window(h, SLAMRS_MAP_F64, 0, 0, (int)h->geom.gw, (int)h->geom.gh, out_cells);
 }
 
 int slamrs_gpu_map_probability_async(slamrs_gpu_handle* h, double* out_cells) {
     if (!h || (!out_cells && h->world == 1)) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     return export_window(h, SLAMRS_MAP_F64, 0, 0, (int)h->geom.gw, (int)h->geom.gh, out_cells, true);
 }
@@ -1035,6 +1209,7 @@ int slamrs_gpu_map_wait(slamrs_gpu_handle* h) {
 
 int slamrs_gpu_map_extent(slamrs_gpu_handle* h, int32_t out_x0y0x1y1[4]) {
     if (!h || !out_x0y0x1y1) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     if (h->world == 1 && h->step > 0 && !h->est_box_stale) {   // the step left the extent of the published map in the counters
         int rc = fetch_counters(h);
@@ -1063,6 +1238,7 @@ int slamrs_gpu_map_extent(slamrs_gpu_handle* h, int32_t out_x0y0x1y1[4]) {
 int slamrs_gpu_map_window(slamrs_gpu_handle* h, uint32_t format, int32_t x0, int32_t y0, int32_t x1, int32_t y1,
                           void* out) {
     if (!h || (!out && h->world == 1)) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     return export_window(h, format, x0, y0, x1, y1, out);
 }
@@ -1140,7 +1316,7 @@ int slamrs_gpu_get_stats(slamrs_gpu_handle* h, slamrs_gpu_stats* out) {
     out->spilled_cells = c.spilled;
     out->window_cells = h->window_cells;
     out->particles_integrated = c.n_alive;
-    out->bytes_per_grid = h->cells_per_grid * sizeof(uint32_t);
+    out->bytes_per_grid = h->localizer ? 0 : h->cells_per_grid * sizeof(uint32_t);
     out->window_overflow = c.window_overflow;
     out->copy_bytes = c.copy_bytes;
     out->resample_exact_fallback = c.fold_fallback;
@@ -1179,6 +1355,7 @@ int slamrs_gpu_get_step_history(slamrs_gpu_handle* h, uint64_t first_step, uint3
     // seven values per step: grids_copied, grids_pulled, distinct_sources, source_reads, particles_integrated,
     // copy_bytes, ray_cell_steps, ray_copy_bytes
     if (!h || !out_triples || count > STEP_HISTORY) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     std::vector<StepRecord> ring(STEP_HISTORY);
     CU_TRY(h, cudaMemcpyAsync(ring.data(), h->d_history, sizeof(StepRecord) * STEP_HISTORY, cudaMemcpyDeviceToHost, h->stream));
@@ -1206,6 +1383,7 @@ int slamrs_gpu_get_poses(slamrs_gpu_handle* h, float* out_xyt) {
 
 int slamrs_gpu_get_slots(slamrs_gpu_handle* h, int32_t* out_slot_of, int32_t* out_spare, uint32_t* out_n_spare) {
     if (!h) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     if (out_slot_of)
         CU_TRY(h, cudaMemcpyAsync(out_slot_of, h->d_slot[h->cur], sizeof(int32_t) * h->n_local, cudaMemcpyDeviceToHost, h->stream));
@@ -1282,6 +1460,7 @@ static int local_root_slot(slamrs_gpu_handle* h, uint64_t particle, int32_t* slo
 
 int slamrs_gpu_get_cells(slamrs_gpu_handle* h, uint64_t particle, uint32_t* out_cells) {
     if (!h || !out_cells) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     int32_t slot = 0;
     int rc = local_root_slot(h, particle, &slot);
@@ -1296,6 +1475,7 @@ int slamrs_gpu_get_cells(slamrs_gpu_handle* h, uint64_t particle, uint32_t* out_
 
 int slamrs_gpu_set_cells(slamrs_gpu_handle* h, uint64_t particle, const uint32_t* cells) {
     if (!h || !cells) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     int32_t slot = 0;
     int rc = unshare_all(h);
@@ -1351,6 +1531,7 @@ int slamrs_gpu_set_cells(slamrs_gpu_handle* h, uint64_t particle, const uint32_t
 int slamrs_gpu_get_extents(slamrs_gpu_handle* h, uint64_t particle, int32_t out_box_shift[5], uint32_t* out_bands,
                            uint32_t* out_n_bands) {
     if (!h || !out_box_shift) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     int32_t slot = 0;
     int rc = local_root_slot(h, particle, &slot);
@@ -1368,6 +1549,7 @@ int slamrs_gpu_get_extents(slamrs_gpu_handle* h, uint64_t particle, int32_t out_
 
 int slamrs_gpu_get_log_odds(slamrs_gpu_handle* h, uint64_t particle, double* out_cells) {
     if (!h || !out_cells) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, NO_GRIDS);
     DeviceGuard g(h->device);
     int32_t slot = 0;
     int rc = local_root_slot(h, particle, &slot);

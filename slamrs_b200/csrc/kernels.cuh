@@ -11,6 +11,8 @@
 //                          k_resample_indices  particle.rs:78-101 + survivor list;  k_plan  keep / copy lists
 //   kernels_copy.cu        k_copy, k_copy_prepare / k_copy_boxed / k_commit_boxes   particle.rs:97-100 clone()
 //   kernels_misc.cu        k_export*       slam.rs:83-88 / map.rs:50-52;  k_sim_scan  simulator/src/sim.rs:134-159
+//   kernels_localize.cu    k_loc_step      localisation on a loaded map: motion + likelihood, one warp per 32 particles;
+//                          k_loc_terms_beam / k_loc_dt_cols / k_loc_dt_rows   sensor-term table at create
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -313,6 +315,16 @@ void launch_sim_scan(cudaStream_t stream, const float* segments, uint32_t n_seg,
                      uint32_t n_beams, float scanner_range, float* angle, float* dist, uint8_t* valid,
                      uint32_t* out_count_maxbits);
 cudaError_t configure_kernels();  // per-device function attributes; call once after cudaSetDevice
+
+// localiser (kernels_localize.cu): the per-cell sensor-term table of a loaded w x w probability map (field = 0: the
+// reference's beam-endpoint model; 1: likelihood field, `scratch` = w*w uint32 for its distance transform), and one
+// step's motion + likelihood over the whole population into results[0, n) (slot = -1)
+cudaError_t launch_loc_terms(cudaStream_t stream, const double* prob, uint32_t w, int field, float sigma, float z_rand,
+                             float occupied_above, float res, uint32_t* scratch, double* terms);
+void launch_loc_step(cudaStream_t stream, MapGeom geom, OdomModel od, ScanDevice scan, const float* pose_cur,
+                     ParticleResult* results, uint32_t n, const double* z_draws, uint64_t seed, uint64_t step,
+                     const double* terms, double outside, const double* carry /* adaptive resampling, else null */,
+                     const StepCounters* counters);
 
 // test hooks
 void launch_debug_raycast(cudaStream_t stream, const float* x0, const float* y0, const float* x1, const float* y1,

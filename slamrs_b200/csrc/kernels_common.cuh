@@ -102,6 +102,65 @@ __device__ __forceinline__ double block_excl_scan_f64(double v, double* warp_tot
     return lane == 0 ? warp_tot[wid] : __dadd_rn(warp_tot[wid], within);
 }
 
+// Odometry::sample (robot.rs:170-183) and the motion log-density Odometry::probabiliy_of (robot.rs:152-167) of local
+// particle p (global index gp) moved from pose_cur: the draws come from z_draws (RNG_CALLER) or the shared stream.
+// Returns the new pose and, in `weight`, the log-density (slot is left to the caller).
+__device__ __forceinline__ ParticleResult motion_step(const OdomModel& od, const float* __restrict__ pose_cur, uint32_t p,
+                                                      uint32_t gp, const double* __restrict__ z_draws, uint64_t seed,
+                                                      uint64_t step) {
+    const float ox = pose_cur[3 * p], oy = pose_cur[3 * p + 1], otheta = pose_cur[3 * p + 2];
+    // Odometry::sample. statrs: sample = mean + std_dev * z.
+    double z1, z2;
+    if (z_draws) {
+        z1 = z_draws[2 * (size_t)gp];
+        z2 = z_draws[2 * (size_t)gp + 1];
+    } else {
+        slamrs_stream::motion_normals(seed, step, gp, &z1, &z2);
+    }
+    const float center_distance = (float)__dadd_rn(od.mean_c, __dmul_rn(od.std_c, z1));
+    const float ntheta = __fadd_rn(otheta, (float)__dadd_rn(od.mean_t, __dmul_rn(od.std_t, z2)));
+    float sn, cs;
+    slamrs_libm::sincosf_exact(ntheta, &sn, &cs);
+    const float nx = __fadd_rn(ox, __fmul_rn(cs, center_distance));
+    const float ny = __fadd_rn(oy, __fmul_rn(sn, center_distance));
+    // Odometry::probabiliy_of(old, new)
+    const float dx = __fsub_rn(ox, nx), dy = __fsub_rn(oy, ny);
+    const float moved = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+    const double ad = angle_diff((double)otheta, (double)ntheta);
+    ParticleResult r;
+    r.weight = __dadd_rn(log(normal_pdf((double)moved, od.mean_c, od.std_c)), log(normal_pdf(ad, od.mean_t, od.std_t)));
+    r.x = nx; r.y = ny; r.theta = ntheta;
+    r.slot = -1;
+    return r;
+}
+
+// Compacts the (angle, distance) pairs of the VALID beams among [b_begin, b_end), in beam order, into out[0..) and
+// returns their number to every thread. Only valid measurements contribute to Map::probability_of (map.rs:117-119);
+// one coalesced 8-byte load per beam replaces the dependent valid[] -> angle[], dist[] loads. Called by every
+// thread of a 128-thread CTA.
+__device__ __forceinline__ uint32_t block_compact_valid_beams(const ScanDevice& scan, uint32_t b_begin, uint32_t b_end,
+                                                              float2* out) {
+    __shared__ uint32_t s_cnt[4];
+    __shared__ uint32_t s_base;
+    if (threadIdx.x == 0) s_base = 0u;
+    __syncthreads();
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    for (uint32_t b0 = b_begin; b0 < b_end; b0 += 128u) {
+        const uint32_t b = b0 + threadIdx.x;
+        const bool v = b < b_end && scan.valid[b] != 0;
+        const unsigned m = __ballot_sync(0xffffffffu, v);
+        if (lane == 0) s_cnt[wid] = __popc(m);
+        __syncthreads();
+        uint32_t off = s_base;
+        for (int w = 0; w < wid; ++w) off += s_cnt[w];
+        if (v) out[off + __popc(m & ((1u << lane) - 1u))] = make_float2(scan.angle[b], scan.dist[b]);
+        __syncthreads();
+        if (threadIdx.x == 0) s_base += s_cnt[0] + s_cnt[1] + s_cnt[2] + s_cnt[3];
+        __syncthreads();
+    }
+    return s_base;
+}
+
 struct alignas(32) V8 {
     uint4 a, b;
 };

@@ -6,8 +6,8 @@ namespace slamrs {
 
 // =============================================================================== k_motion + k_likelihood
 // k_motion: one THREAD per particle. Odometry::sample (robot.rs:170-183) and the motion log-density
-// Odometry::probabiliy_of (robot.rs:152-167) need a few hundred scalar f64 operations per particle
-// and nothing else; giving them a warp or a CTA would multiply the issued instructions by 32.
+// Odometry::probabiliy_of (robot.rs:152-167) (motion_step) need a few hundred scalar f64 operations per
+// particle and nothing else; giving them a warp or a CTA would multiply the issued instructions by 32.
 // The log-density is parked in ParticleResult::weight until k_likelihood folds it in.
 __global__ void __launch_bounds__(128)
 k_motion(OdomModel od, const float* __restrict__ pose_cur, const int32_t* __restrict__ slot_of,
@@ -17,56 +17,16 @@ k_motion(OdomModel od, const float* __restrict__ pose_cur, const int32_t* __rest
     pdl_launch_dependents();   // k_likelihood may take its place on the SMs now; it waits for this grid before it reads
     // the ray update's per-step flags and counters start from zero (instead of a memset in front of the step)
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_zero; i += gridDim.x * blockDim.x) zero_words[i] = 0u;
-    // Block 0 also compacts the (angle, distance) pairs of the scan's VALID beams, in beam order, for
-    // k_likelihood: only valid measurements contribute to Map::probability_of (map.rs:117-119), and
-    // one coalesced 8-byte load per beam replaces the dependent valid[] -> angle[], dist[] loads that
-    // the likelihood kernel spent most of its stall cycles on.
+    // Block 0 also compacts the scan's VALID beams, in beam order, for k_likelihood (the likelihood kernel
+    // spent most of its stall cycles on the dependent valid[] -> angle[], dist[] loads)
     if (blockIdx.x == 0) {
-        __shared__ uint32_t s_cnt[4];
-        __shared__ uint32_t s_base;
-        if (threadIdx.x == 0) s_base = 0u;
-        __syncthreads();
-        const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-        for (uint32_t b0 = 0; b0 < scan.n_beams; b0 += 128u) {
-            const uint32_t b = b0 + threadIdx.x;
-            const bool v = b < scan.n_beams && scan.valid[b] != 0;
-            const unsigned m = __ballot_sync(0xffffffffu, v);
-            if (lane == 0) s_cnt[wid] = __popc(m);
-            __syncthreads();
-            uint32_t off = s_base;
-            for (int w = 0; w < wid; ++w) off += s_cnt[w];
-            if (v) valid_beams[off + __popc(m & ((1u << lane) - 1u))] = make_float2(scan.angle[b], scan.dist[b]);
-            __syncthreads();
-            if (threadIdx.x == 0) s_base += s_cnt[0] + s_cnt[1] + s_cnt[2] + s_cnt[3];
-            __syncthreads();
-        }
-        if (threadIdx.x == 0) *n_valid = s_base;
+        const uint32_t nv = block_compact_valid_beams(scan, 0u, scan.n_beams, valid_beams);
+        if (threadIdx.x == 0) *n_valid = nv;
     }
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_local) return;
     const uint32_t gp = first_particle + p;      // global logical index
-    const float ox = pose_cur[3 * p], oy = pose_cur[3 * p + 1], otheta = pose_cur[3 * p + 2];
-    // Odometry::sample. statrs: sample = mean + std_dev * z.
-    double z1, z2;
-    if (z_draws) {
-        z1 = z_draws[2 * (size_t)gp];
-        z2 = z_draws[2 * (size_t)gp + 1];
-    } else {
-        slamrs_stream::motion_normals(seed, step, gp, &z1, &z2);
-    }
-    const float center_distance = (float)__dadd_rn(od.mean_c, __dmul_rn(od.std_c, z1));
-    const float ntheta = __fadd_rn(otheta, (float)__dadd_rn(od.mean_t, __dmul_rn(od.std_t, z2)));
-    float sn, cs;
-    slamrs_libm::sincosf_exact(ntheta, &sn, &cs);
-    const float nx = __fadd_rn(ox, __fmul_rn(cs, center_distance));
-    const float ny = __fadd_rn(oy, __fmul_rn(sn, center_distance));
-    // Odometry::probabiliy_of(old, new)
-    const float dx = __fsub_rn(ox, nx), dy = __fsub_rn(oy, ny);
-    const float moved = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-    const double ad = angle_diff((double)otheta, (double)ntheta);
-    ParticleResult r;
-    r.weight = __dadd_rn(log(normal_pdf((double)moved, od.mean_c, od.std_c)), log(normal_pdf(ad, od.mean_t, od.std_t)));
-    r.x = nx; r.y = ny; r.theta = ntheta;
+    ParticleResult r = motion_step(od, pose_cur, p, gp, z_draws, seed, step);
     r.slot = slot_of[p];                    // physical slot, read by other ranks' planners
     results[gp] = r;
 }

@@ -27,13 +27,14 @@ __device__ __forceinline__ double cell_log_odds(uint32_t cell) {
 // LogOdds::probability, math.rs:135-137
 __device__ __forceinline__ double log_odds_probability(double l) { return 1.0 - 1.0 / (1.0 + exp(l)); }
 
-// one factor of Map::probability_of (map.rs:130-141) in log form for an informed cell:
+// one factor of Map::probability_of (map.rs:130-141) in log form for a cell of probability p:
 // log(Z_HIT * p + (1 - Z_HIT) * 1 / SENSOR_MAXDIST), or log(1/1) when p is exactly the prior
-__device__ __forceinline__ double beam_log_term(uint32_t cell) {
-    const double prob = log_odds_probability(cell_log_odds(cell));
+__device__ __forceinline__ double beam_log_term_p(double prob) {
     // Z_HIT = 0.9, SENSOR_MAXDIST = 1.0 (map.rs:108-109)
     return (prob == 0.5) ? log(1.0 / 1.0) : log(__dadd_rn(__dmul_rn(0.9, prob), (1.0 - 0.9) * 1.0 / 1.0));
 }
+// the same for an informed cell given by its hit counters
+__device__ __forceinline__ double beam_log_term(uint32_t cell) { return beam_log_term_p(log_odds_probability(cell_log_odds(cell))); }
 // The factor depends on the cell's two hit counters only. For counters below these bounds it is
 // read from a table that the same function filled on the same device at create (bit-identical
 // to evaluating it in place, without the exp, the division and the log per beam).

@@ -30,6 +30,27 @@ def reference_scene(scale: float = 1.0) -> np.ndarray:
     return (np.array(seg, np.float64) * scale).astype(np.float32)
 
 
+def scene_map(segments, config) -> np.ndarray:
+    """A probability map of the scene for a grid of `config` (a GridMapSlamConfig): 0.9 on every cell a segment
+    crosses, 0.5 (unknown) elsewhere; flat f64, index row * grid_h + column, the layout of estimated_likelihood().
+    A segment is sampled every quarter cell, both endpoints included; a sample marks the cell it falls in
+    (Map::world_to_grid and is_valid, map.rs:60-69). Deterministic, so tests and benchmarks get a map without a
+    SLAM run."""
+    from .slam import grid_cells
+    gw, gh = grid_cells(config.width, config.resolution), grid_cells(config.height, config.resolution)
+    res, px, py = f32(config.resolution), f32(config.position[0]), f32(config.position[1])
+    out = np.full(gw * gh, 0.5, np.float64)
+    for x1, y1, x2, y2 in np.asarray(segments, np.float32).reshape(-1, 4):
+        length = float(np.hypot(float(x2) - float(x1), float(y2) - float(y1)))
+        k = max(1, int(np.ceil(4.0 * length / float(res))))
+        t = np.linspace(0.0, 1.0, k + 1, dtype=np.float32)
+        gx = (x1 + (x2 - x1) * t - px) / res
+        gy = (y1 + (y2 - y1) * t - py) / res
+        ok = (gx >= 0) & (gy >= 0) & (gx < gw) & (gy < gh)
+        out[gy[ok].astype(np.int64) * gh + gx[ok].astype(np.int64)] = 0.9
+    return out
+
+
 def scan(segments: np.ndarray, pose, n_beams: int, scanner_range: float) -> Observation:
     px, py, pt = f32(pose[0]), f32(pose[1]), f32(pose[2])
     deg = np.arange(n_beams, dtype=np.float32) * f32(360.0 / n_beams)

@@ -151,6 +151,17 @@ class GridMapSlam:
             raise ValueError("Must have at least one particle")  # particle.rs:16 assert
         gw = grid_cells(config.width, config.resolution)
         gh = grid_cells(config.height, config.resolution)
+        self._create(self._config_struct(config, pl, gw, gh))
+        self.grid_w, self.grid_h = gw, gh
+        self.n_particles = int(config.n_particles)
+        self.n_local = self.n_particles // pl.world_size
+        self.first = pl.rank * self.n_local
+
+    def _create(self, cfg) -> None:
+        _lib.check(self._L.slamrs_gpu_create(C.byref(cfg), C.byref(self._h)))
+
+    @staticmethod
+    def _config_struct(config: GridMapSlamConfig, pl: GpuPlacement, gw: int, gh: int):
         cfg = _lib.Config()
         cfg.struct_size = C.sizeof(_lib.Config)
         cfg.abi_version = _lib.ABI_VERSION
@@ -170,11 +181,7 @@ class GridMapSlam:
             if pl.nccl_id is None or len(pl.nccl_id) != _lib.NCCL_ID_BYTES:
                 raise ValueError("world_size > 1 needs the 128-byte nccl_id shared by all ranks")
             C.memmove(cfg.nccl_id, pl.nccl_id, _lib.NCCL_ID_BYTES)
-        _lib.check(self._L.slamrs_gpu_create(C.byref(cfg), C.byref(self._h)))
-        self.grid_w, self.grid_h = gw, gh
-        self.n_particles = int(config.n_particles)
-        self.n_local = self.n_particles // pl.world_size
-        self.first = pl.rank * self.n_local
+        return cfg
 
     @classmethod
     def new(cls, config: GridMapSlamConfig, placement: Optional[GpuPlacement] = None) -> "GridMapSlam":
@@ -414,6 +421,57 @@ class GridMapSlam:
     def log_odds(self, particle: int) -> np.ndarray:
         out = np.zeros(self.grid_w * self.grid_h, np.float64)
         _lib.check(self._L.slamrs_gpu_get_log_odds(self._h, particle, _ptr(out)), self._h)
+        return out
+
+
+@dataclass
+class SensorModel:
+    """How a GridMapLocalizer scores a beam endpoint against its loaded map (slamrs_gpu_sensor_model).
+
+    kind SENSOR_BEAM_ENDPOINT (the default, as every extension here defaults to the reference): Map::probability_of's
+    factor (map.rs:130-141). It scores endpoints in unknown space or off the map best, so it cannot localise from a
+    uniform start; it is there for parity with the SLAM step. Global localisation needs kind SENSOR_LIKELIHOOD_FIELD:
+    log(z_hit * exp(-d^2 / (2 sigma^2)) + z_rand), d = distance to the nearest cell with p > occupied_above."""
+    kind: int = _lib.SENSOR_BEAM_ENDPOINT
+    sigma: float = 0.1            # metres
+    z_rand: float = 0.05          # z_hit = 1 - z_rand
+    occupied_above: float = 0.5
+
+    @staticmethod
+    def likelihood_field(sigma: float = 0.1, z_rand: float = 0.05, occupied_above: float = 0.5) -> "SensorModel":
+        return SensorModel(_lib.SENSOR_LIKELIHOOD_FIELD, sigma, z_rand, occupied_above)
+
+    def to_struct(self):
+        m = _lib.SensorModel()
+        m.struct_size = C.sizeof(_lib.SensorModel)
+        m.kind, m.sigma, m.z_rand, m.occupied_above = int(self.kind), float(self.sigma), float(self.z_rand), float(self.occupied_above)
+        return m
+
+
+class GridMapLocalizer(GridMapSlam):
+    """Monte Carlo localisation against a loaded occupancy map: GridMapSlam::update with the map held fixed and shared
+    by every particle (no per-particle grids). `map_probability` is the grid_w * grid_h f64 probabilities, flat or
+    2-D (index row * grid_h + column), or the GridData that GridMapSlam.estimated_likelihood() returns. Place the
+    particles with init_uniform() or set_poses(), then update() and estimated_pose() as on a GridMapSlam; the grid
+    read-outs (estimated_likelihood, cells, ...) raise. Runs on one GPU (placement.world_size must be 1)."""
+
+    def __init__(self, config: GridMapSlamConfig, map_probability, model: Optional[SensorModel] = None,
+                 placement: Optional[GpuPlacement] = None):
+        data = map_probability.data if isinstance(map_probability, GridData) else map_probability
+        self._map = np.ascontiguousarray(data, np.float64).reshape(-1)
+        self.model = model or SensorModel()
+        super().__init__(config, placement)
+
+    def _create(self, cfg) -> None:
+        if self._map.size != cfg.grid_w * cfg.grid_h:
+            raise ValueError(f"map_probability holds {self._map.size} cells, the grid {cfg.grid_w * cfg.grid_h}")
+        m = self.model.to_struct()
+        _lib.check(self._L.slamrs_gpu_create_localizer(C.byref(cfg), C.byref(m), _ptr(self._map), C.byref(self._h)))
+
+    def sensor_terms(self) -> np.ndarray:
+        """The grid_w * grid_h f64 term table the device built from the map (index row * grid_h + column)."""
+        out = np.zeros(self.grid_w * self.grid_h, np.float64)
+        _lib.check(self._L.slamrs_gpu_get_sensor_terms(self._h, _ptr(out)), self._h)
         return out
 
 
