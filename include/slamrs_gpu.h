@@ -170,8 +170,11 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
                           const double* z_draws, const double* resample_u);
 int slamrs_gpu_sync(slamrs_gpu_handle* h);
 /* Use an observation that already lives in device memory (caller-owned, must stay valid until
- * the steps that use it have completed). max_dist = largest finite distance in the scan (sizes
- * the ray kernel's shared-memory window; correctness does not depend on it). */
+ * the steps that use it have completed). max_dist = an upper bound of |distance| over every beam
+ * of the scan, in metres: it sizes the ray kernel's shared-memory window. +inf, NaN or a value <= 0
+ * mean "unknown" (pass +inf when the scan may hold non-finite distances): the step then takes the
+ * unfused ray update, which is exact for any scan. A bound that some beam exceeds can make the
+ * step fail with SLAMRS_E_INTERNAL. */
 int slamrs_gpu_set_scan_device(slamrs_gpu_handle* h, const float* angle_device, const float* dist_device,
                                const uint8_t* valid_device, uint32_t n_beams, float max_dist);
 

@@ -866,13 +866,17 @@ int slamrs_gpu_upload_scan(slamrs_gpu_handle* h, const float* angle, const float
     h->n_beams = n_beams;
     h->scan_external = false;
     h->order_valid = false;
-    // window radius for the ray kernel: farthest finite measurement, in cells, plus the two extra
-    // steps of apply_measurement (map.rs:97) and the slack that lets the ray kernel prove, per ray, that
-    // no cell leaves the window (see k_ray_update_packed). Correctness never depends on it:
-    // cells outside the window take the global-atomic path.
+    // window radius for the ray kernel: farthest measurement, in cells, plus the two extra steps of
+    // apply_measurement (map.rs:97) and the slack that lets the ray kernel prove, per ray, that no cell
+    // leaves the window (see k_ray_update_packed). A non-finite distance still casts a ray, to the grid
+    // border: its reach is unbounded, which selects the unfused ray update (cells outside the window take
+    // the global-atomic path there; the fused update can only park a bounded number of them).
     float maxd = 0.0f;
-    for (uint32_t i = 0; i < n_beams; ++i)
-        if (isfinite(dist[i]) && fabsf(dist[i]) > maxd) maxd = fabsf(dist[i]);
+    for (uint32_t i = 0; i < n_beams; ++i) {
+        const float d = fabsf(dist[i]);
+        if (!isfinite(d)) { maxd = INFINITY; break; }
+        if (d > maxd) maxd = d;
+    }
     const float cells = ceilf(maxd / h->geom.res);
     h->radius_cells = (cells < 4096.0f ? (int)cells : 4096) + 6;
     return SLAMRS_OK;
@@ -887,7 +891,9 @@ int slamrs_gpu_set_scan_device(slamrs_gpu_handle* h, const float* angle_device, 
     h->n_beams = n_beams;
     h->scan_external = true;
     h->order_valid = false;
-    const float cells = ceilf(fabsf(max_dist) / h->geom.res);
+    // max_dist bounds |distance| over the scan; +inf, NaN or <= 0 mean "unknown": the unfused ray update, which
+    // takes any scan (see slamrs_gpu.h)
+    const float cells = max_dist > 0.0f ? ceilf(max_dist / h->geom.res) : INFINITY;
     h->radius_cells = ((cells == cells && cells < 4096.0f) ? (int)cells : 4096) + 6;
     return SLAMRS_OK;
 }

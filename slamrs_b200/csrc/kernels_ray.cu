@@ -126,6 +126,31 @@ __host__ __device__ inline int ray_window_cells_upper_bound(int radius, bool vec
     return total;
 }
 
+// A zero-length ray (dx = dy = 0: the endpoint rounds back onto the start point) cannot move, so it emits its start cell
+// 1 + additional_steps = 3 times (ray.rs:96-104 with both increments 0). Every other ray emits a cell at most once,
+// which is what bounds the window's counters (n_beams hits per cell and scan), so these hits take the exact,
+// saturating path instead: a thread tallies them during its walk and sends them after it (at most 3 parked entries
+// per ray, within RAY_SPILL_CAP). Every ray of a particle starts in the same cell.
+struct ZeroLengthHits {
+    uint32_t free_hits = 0u, occ_hits = 0u;
+    __device__ __forceinline__ void tally(const RayClassifier& cls, float acc) {
+        const uint32_t inc = classify_cell(cls, acc);
+        free_hits += inc == CELL_FREE_INC ? 3u : 0u;
+        occ_hits += inc == CELL_OCC_INC ? 3u : 0u;
+    }
+    // returns the hits sent to the exact path
+    template <class ExactAdd>
+    __device__ __forceinline__ uint32_t flush(int cx0, int cy0, ExactAdd& exact_add, int* s_ext, int* s_blo, int* s_bhi,
+                                              int band0) const {
+        if (free_hits + occ_hits == 0u) return 0u;
+        for (uint32_t k = 0; k < free_hits; ++k) exact_add(cx0, cy0, CELL_FREE_INC);
+        for (uint32_t k = 0; k < occ_hits; ++k) exact_add(cx0, cy0, CELL_OCC_INC);
+        ext_add(s_ext, cx0, cy0, cx0, cy0);
+        band_add(s_blo, s_bhi, band0, cy0, cx0, cx0);
+        return free_hits + occ_hits;
+    }
+};
+
 template <bool kVector>
 __global__ void __launch_bounds__(RAY_MAX_THREADS)
 k_ray_update(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ results, uint32_t first_particle,
@@ -202,6 +227,7 @@ k_ray_update(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ r
 
     bool saturated = false;
     uint32_t spilled = 0;
+    ZeroLengthHits zero_length;
     for (uint32_t t = threadIdx.x; t < scan.n_beams; t += blockDim.x) {
         const uint32_t b = scan.order ? scan.order[t] : t;
         const float dist = scan.dist[b];
@@ -211,6 +237,12 @@ k_ray_update(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ r
         const float gy = world_to_grid(ey, geom.pos_y, geom.res);
         // measured distance in cells (map.rs:84) and the per-ray form of inverse_sensor_model
         const RayClassifier cls = make_ray_classifier(__fdiv_rn(dist, geom.res), scan.valid[b] != 0);
+        if (fabsf(__fsub_rn(gx, sx)) == 0.0f && fabsf(__fsub_rn(gy, sy)) == 0.0f) {
+            // zero-length ray (see ZeroLengthHits): its hits would overflow a 16-bit half of the window
+            const float dxs = __fsub_rn(sx, __fadd_rn((float)cx, 0.5f)), dys = __fsub_rn(sy, __fadd_rn((float)cy, 0.5f));
+            zero_length.tally(cls, __fadd_rn(__fmul_rn(dxs, dxs), __fmul_rn(dys, dys)));
+            continue;
+        }
         // apply_measurement, map.rs:88-106 (additional_steps = 2)
         ray_walk_acc(sx, sy, gx, gy, geom.gw, geom.gh, 2u, [&](int x, int y, float acc) {
             const uint32_t inc = classify_cell(cls, acc);
@@ -234,6 +266,12 @@ k_ray_update(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ r
                 }
             }
         });
+    }
+    {
+        auto exact_add = [&](int x, int y, uint32_t inc) {
+            global_cell_add(&grid[phys_index(geom, (uint32_t)x, (uint32_t)y)], inc, &saturated);
+        };
+        spilled += zero_length.flush(cx, cy, exact_add, s_ext, s_blo, s_bhi, band0);
     }
     __syncthreads();
 
@@ -382,7 +420,9 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
     uint32_t spilled = 0, cell_steps = 0;
     // A clone's own slot receives its cells only at write-back, so the (rare) hits that bypass the window --
     // the 32nd occupied hit of a cell in one scan -- are parked and applied after the write-back.
-    // At most 4 occupied cells per ray: RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS entries always suffice.
+    // At most 4 occupied cells per ray (3 hits of a zero-length ray): RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS
+    // entries suffice when the window holds every cell a ray reaches.
+    ZeroLengthHits zero_length;
     auto exact_add = [&](int x, int y, uint32_t inc) {
         if (fused) {
             const uint32_t k = atomicAdd(s_nspill_p, 1u);
@@ -452,6 +492,10 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
         float cxf = __fadd_rn((float)cx0, 0.5f), cyf = __fadd_rn((float)cy0, 0.5f);
         float dxs = __fsub_rn(sx, cxf), dys = __fsub_rn(sy, cyf);
         float dx2 = __fmul_rn(dxs, dxs), dy2 = __fmul_rn(dys, dys);
+        if (delta_x == 0.0f && delta_y == 0.0f) {   // see ZeroLengthHits
+            zero_length.tally(cls, __fadd_rn(dx2, dy2));
+            continue;
+        }
 
         // every cell of this ray inside the window and the grid?
         bool fast = false;
@@ -599,6 +643,7 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
         }
         cell_steps -= (uint32_t)remaining;   // the walk ended at the grid border
     }
+    spilled += zero_length.flush(cx0, cy0, exact_add, s_ext, s_blo, s_bhi, band0);
     if (saturated) *saturated_p = true;
     *spilled_p += spilled;
     *cell_steps_p += cell_steps;
@@ -1082,6 +1127,7 @@ __device__ __noinline__ void ray_walk_half(const MapGeom& geom, const ScanDevice
     const int gw = (int)geom.gw, gh = (int)geom.gh;
     const uint32_t win_base = (uint32_t)__cvta_generic_to_shared(s_win);
     uint32_t spilled = 0, cell_steps = 0;
+    ZeroLengthHits zero_length;
     auto exact_add = [&](int x, int y, uint32_t inc) {
         const uint32_t k = atomicAdd(s_nspill_p, 1u);
         if (k < RAY_SPILL_CAP) my_spill[k] = (uint32_t)x | ((uint32_t)y << 15) | (inc == CELL_OCC_INC ? 0x40000000u : 0u);
@@ -1144,6 +1190,10 @@ __device__ __noinline__ void ray_walk_half(const MapGeom& geom, const ScanDevice
         float cxf = __fadd_rn((float)cx0, 0.5f), cyf = __fadd_rn((float)cy0, 0.5f);
         float dxs = __fsub_rn(sx, cxf), dys = __fsub_rn(sy, cyf);
         float dx2 = __fmul_rn(dxs, dxs), dy2 = __fmul_rn(dys, dys);
+        if (delta_x == 0.0f && delta_y == 0.0f) {   // see ZeroLengthHits
+            zero_length.tally(cls, __fadd_rn(dx2, dy2));
+            continue;
+        }
 
         bool fast = false;
         if (disc_in_grid && ax < 4096ull && ay < 4096ull) {
@@ -1315,6 +1365,7 @@ __device__ __noinline__ void ray_walk_half(const MapGeom& geom, const ScanDevice
         }
         cell_steps -= (uint32_t)remaining;   // the walk ended at the grid border
     }
+    spilled += zero_length.flush(cx0, cy0, exact_add, s_ext, s_blo, s_bhi, band0);
     *spilled_p += spilled;
     *cell_steps_p += cell_steps;
 }

@@ -320,7 +320,9 @@ class GridMapSlam:
                                                  _ptr(zd), _ptr(ru)), self._h)
 
     def set_scan_device(self, angle_ptr: int, dist_ptr: int, valid_ptr: int, n_beams: int, max_dist: float) -> None:
-        """Step on an observation that already lives in device memory (raw device pointers)."""
+        """Step on an observation that already lives in device memory (raw device pointers). `max_dist` bounds
+        |distance| over every beam (it sizes the ray kernel's window); +inf, NaN or <= 0 mean unknown and are exact for
+        any scan. A bound that some beam exceeds can make the step fail with E_INTERNAL."""
         _lib.check(self._L.slamrs_gpu_set_scan_device(self._h, angle_ptr, dist_ptr, valid_ptr, n_beams, max_dist), self._h)
 
     def set_profiling(self, enabled: bool) -> None:
