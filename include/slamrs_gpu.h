@@ -105,7 +105,9 @@ typedef struct slamrs_gpu_config {
                                  tau in (0, 1]: resample only when the effective number of particles
                                  (particle.rs:59-65) is below tau * N; otherwise every particle stays in place and
                                  carries its normalised weight into the next update (SURVEY.md 8(f)4; not a
-                                 reference feature) */
+                                 reference feature). With tau > 0, N_eff is the reference's strict left fold of
+                                 the squared weights, bit for bit, so the decision is the reference's even when
+                                 N_eff lies within an ulp of tau * N; at 0 it is a re-associated sum (within 1e-9) */
     uint8_t nccl_id[SLAMRS_NCCL_ID_BYTES]; /* from slamrs_gpu_nccl_unique_id, same on all ranks */
 } slamrs_gpu_config;
 
@@ -123,8 +125,9 @@ typedef struct slamrs_gpu_stats {
     uint64_t particles_integrated; /* local particles whose grid received the scan this step */
     uint64_t copy_bytes;       /* bytes the resampling copies read + wrote in this step (device-counted) */
     uint64_t window_overflow;  /* grids whose informed extent would have outgrown a windowed slot (error) */
-    uint64_t resample_exact_fallback; /* bit 0 / 1: the weight sum / the running sum of the last step was folded by a
-                                         single thread (NaN, inf or hostile weights; the result is the same) */
+    uint64_t resample_exact_fallback; /* bit 0 / 1 / 2: the weight sum / the running sum / the sum of squares (only
+                                         with resample_threshold > 0) of the last step was folded by a single thread
+                                         (NaN, inf or hostile weights; the result is the same) */
     uint64_t resample_fold_rounds;    /* rounds the parallel exact fold needed (1 = proven at once) */
     uint64_t resampled;               /* 1 if the last update resampled (always, unless resample_threshold > 0) */
 } slamrs_gpu_stats;
@@ -350,6 +353,16 @@ int slamrs_gpu_debug_stream(int device, uint64_t seed, uint64_t step, uint64_t f
 int slamrs_gpu_debug_resample(int device, const double* raw_weights, uint32_t n, double u01, uint32_t* out_idx,
                               uint64_t* out_max_particle, double* out_norm, double* out_cum, uint64_t out_info[4],
                               float out_us[2]);
+/* slamrs_gpu_debug_resample with the adaptive-resampling threshold tau (resample_threshold, 0 or in (0, 1]).
+ * Also returns (each optional) out_n_eff = the N_eff of particle.rs:59-65 that k_weights computed, out_do_resample
+ * = 1 if N_eff < tau * N or tau = 0 (else out_idx is the identity), and out_shape = the launch k_weights used
+ * for n: {CTAs in the cluster, threads per CTA, consecutive elements per thread, 1 = elements held in registers /
+ * 0 = the generic kernel that re-reads them from global memory}. Bit 2 of out_info[3]: the sum of squares was
+ * folded by a single thread (tau > 0 only). */
+int slamrs_gpu_debug_resample_adaptive(int device, const double* raw_weights, uint32_t n, double u01, double tau,
+                                       uint32_t* out_idx, uint64_t* out_max_particle, double* out_norm, double* out_cum,
+                                       uint64_t out_info[4], float out_us[2], double* out_n_eff, uint64_t* out_do_resample,
+                                       uint64_t out_shape[4]);
 
 #ifdef __cplusplus
 }

@@ -32,7 +32,7 @@ EXPORTS = [
     "slamrs_gpu_set_scan_device", "slamrs_gpu_set_profiling", "slamrs_gpu_get_phase_ms",
     "slamrs_gpu_get_step_history", "slamrs_gpu_map_extent", "slamrs_gpu_map_window",
     "slamrs_gpu_effective_particles", "slamrs_gpu_sim_scan", "slamrs_gpu_get_scan", "slamrs_gpu_get_slots",
-    "slamrs_gpu_get_extents", "slamrs_gpu_debug_resample", "slamrs_gpu_init_uniform",
+    "slamrs_gpu_get_extents", "slamrs_gpu_debug_resample", "slamrs_gpu_debug_resample_adaptive", "slamrs_gpu_init_uniform",
     "slamrs_gpu_map_probability_async", "slamrs_gpu_map_wait",
     "slamrs_gpu_create_localizer", "slamrs_gpu_get_sensor_terms",
 ]
@@ -137,6 +137,9 @@ def load():
     L.slamrs_gpu_get_sensor_terms.restype = i; L.slamrs_gpu_get_sensor_terms.argtypes = [vp, vp]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
+    L.slamrs_gpu_debug_resample_adaptive.restype = i
+    L.slamrs_gpu_debug_resample_adaptive.argtypes = [i, vp, u32, C.c_double, C.c_double, vp, C.POINTER(u64), vp, vp, vp,
+                                                     vp, C.POINTER(C.c_double), C.POINTER(u64), vp]
     _lib = L
     return L
 

@@ -1626,7 +1626,15 @@ int slamrs_gpu_debug_stream(int device, uint64_t seed, uint64_t step, uint64_t f
 int slamrs_gpu_debug_resample(int device, const double* raw_weights, uint32_t n, double u01, uint32_t* out_idx,
                               uint64_t* out_max_particle, double* out_norm, double* out_cum, uint64_t out_info[4],
                               float out_us[2]) {
-    if (!raw_weights || !out_idx || n == 0 || n > 0x7fffffffu) return SLAMRS_E_INVALID_ARG;
+    return slamrs_gpu_debug_resample_adaptive(device, raw_weights, n, u01, 0.0, out_idx, out_max_particle, out_norm, out_cum,
+                                              out_info, out_us, nullptr, nullptr, nullptr);
+}
+
+int slamrs_gpu_debug_resample_adaptive(int device, const double* raw_weights, uint32_t n, double u01, double tau,
+                                       uint32_t* out_idx, uint64_t* out_max_particle, double* out_norm, double* out_cum,
+                                       uint64_t out_info[4], float out_us[2], double* out_n_eff, uint64_t* out_do_resample,
+                                       uint64_t out_shape[4]) {
+    if (!raw_weights || !out_idx || n == 0 || n > 0x7fffffffu || !(tau >= 0.0 && tau <= 1.0)) return SLAMRS_E_INVALID_ARG;
     int rc = debug_device(device);
     if (rc) return rc;
     DeviceGuard g(device < 0 ? 0 : device);
@@ -1648,7 +1656,7 @@ int slamrs_gpu_debug_resample(int device, const double* raw_weights, uint32_t n,
     float us[2] = {0.f, 0.f};
     for (int r = 0; r < reps; ++r) {
         cudaEventRecord(ev[0], nullptr);
-        launch_weights(nullptr, res.p, n, wn.p, cum.p, fold.p, 0.0, cnt.p);
+        launch_weights(nullptr, res.p, n, wn.p, cum.p, fold.p, tau, cnt.p);
         cudaEventRecord(ev[1], nullptr);
         launch_resample_indices(nullptr, res.p, cum.p, n, u.p, 0, 0, idx.p, nullptr, 0, 0, false, nullptr,
                                 RayLists{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u}, wn.p, nullptr, cnt.p);
@@ -1676,6 +1684,12 @@ int slamrs_gpu_debug_resample(int device, const double* raw_weights, uint32_t n,
         }
     }
     if (out_info) { out_info[0] = c.clamped; out_info[1] = c.fold_rounds; out_info[2] = c.fold_heads; out_info[3] = c.fold_fallback; }
+    if (out_n_eff) *out_n_eff = c.n_eff;
+    if (out_do_resample) *out_do_resample = c.do_resample;
+    if (out_shape) {
+        const WeightsShape sh = weights_shape(n);
+        out_shape[0] = sh.cluster; out_shape[1] = sh.threads; out_shape[2] = sh.chunk; out_shape[3] = sh.regs ? 1u : 0u;
+    }
     return SLAMRS_OK;
 }
 

@@ -192,8 +192,13 @@ cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan
                               uint32_t signal_epoch /* != 0 (half-item kernel only): every integrated slot's SlotMeta::pad0
                                                        receives it once both halves are in place (peers that pull the slot wait for it) */);
 
+// k_weights' launch for a population: a cluster of `cluster` CTAs of `threads` threads, each thread folding `chunk`
+// consecutive elements, held in registers (regs) or re-read from global memory (the generic kernel)
+struct WeightsShape { uint32_t cluster, threads, chunk; bool regs; };
+WeightsShape weights_shape(uint32_t n_total);
 // fold_scratch: weights_scratch_doubles() doubles
-// resample_tau > 0: counters->do_resample = N_eff < tau * N (adaptive resampling), else 1
+// resample_tau > 0: counters->do_resample = N_eff < tau * N (adaptive resampling; N_eff from the reference's strict
+// left fold of the squares), else 1
 void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t n_total, double* w_norm,
                     double* cum, double* fold_scratch, double resample_tau, StepCounters* counters);
 size_t weights_scratch_doubles();

@@ -482,7 +482,7 @@ k_weights(const ParticleResult* __restrict__ results, uint32_t n, double* __rest
     }
     FOLD_STAMP(4);
     double cta_sq;
-    block_excl_scan_f64(sqpart, sh.warp_f64, &cta_sq);
+    const double sq_offset = block_excl_scan_f64(sqpart, sh.warp_f64, &cta_sq);
 
     // argmax by f64::total_cmp, ties -> highest index (Iterator::max_by returns the last maximum)
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -536,6 +536,41 @@ k_weights(const ParticleResult* __restrict__ results, uint32_t n, double* __rest
         }
         fold_sync(cluster, C);
     }
+
+    // pass 4, adaptive resampling only: the sum of squares of number_of_effective_particles (particle.rs:59-65),
+    // `sum += w * w` left to right. N_eff < tau * N decides whether the filter resamples, and a re-associated sum
+    // can land on the other side of tau * N than the reference's (equal weights at tau = 1: N_eff = N +- 1 ulp),
+    // which changes the whole trajectory. The re-associated prefix of pass 2 is the estimate. With tau = 0 only
+    // the reported N_eff depends on this sum, and the re-associated one is kept (no pass on the default path).
+    FoldInfo info_sq = {0u, 0u, 0u};
+    double sq_exact = 0.0;
+    if (resample_tau > 0.0) {
+        double q_in = sq_offset;
+        if (C > 1u) {   // (every CTA has read sh.cta_part long before: pass 1 ended with cluster barriers)
+            if (threadIdx.x < C) cluster.map_shared_rank(&sh.cta_part[0], threadIdx.x)[crank] = cta_sq;
+            cluster.sync();
+            q_in = 0.0;
+            for (uint32_t r = 0; r < crank; ++r) q_in = __dadd_rn(q_in, sh.cta_part[r]);
+            q_in = __dadd_rn(q_in, sq_offset);
+        }
+        if (LREG) {
+#pragma unroll
+            for (int j = 0; j < (LREG ? LREG : 1); ++j) v[j] = __dmul_rn(v[j], v[j]);   // (the padding stays +0.0)
+        }
+        double q_lo, q_hi;
+        const bool sq_ok = exact_left_fold<LREG>(cluster, sh, n, L, cnt, all_zero, q_in, __dadd_rn(q_in, sqpart), v,
+                                                 [](uint32_t, double) {},
+                                                 [&](uint32_t i) { const double w = __ldcg(&w_norm[i]); return __dmul_rn(w, w); },
+                                                 false, fold_scratch, &q_lo, &q_hi, &sq_exact, &info_sq, 24);
+        if (!sq_ok) {   // the reference's loop as it stands (w_norm is complete: the fold passed cluster barriers)
+            info_sq.fallback = 1u;
+            if (gt == 0) {
+                double s = 0.0;
+                for (uint32_t i = 0; i < n; ++i) { const double w = __ldcg(&w_norm[i]); s = __dadd_rn(s, __dmul_rn(w, w)); }
+                sq_exact = s;
+            }
+        }
+    }
     // (a proven pass 3 ended with a cluster barrier: the peers' argmax candidates and sums of squares are in CTA 0)
     if (gt == 0) {
         long long bk = 0; uint32_t bi = 0; bool h = false;
@@ -546,29 +581,42 @@ k_weights(const ParticleResult* __restrict__ results, uint32_t n, double* __rest
         counters->max_particle = bi;
         counters->sum = sum;
         // number_of_effective_particles (particle.rs:59-65) of the normalised weights, before resampling
-        double sq = 0.0;
-        for (uint32_t r = 0; r < C; ++r) sq = __dadd_rn(sq, s_sq[r]);
+        double sq = sq_exact;
+        if (!(resample_tau > 0.0)) {
+            sq = 0.0;
+            for (uint32_t r = 0; r < C; ++r) sq = __dadd_rn(sq, s_sq[r]);
+        }
         counters->n_eff = __ddiv_rn(1.0, sq);
         // adaptive resampling (not in the reference, which always resamples): only when N_eff < tau * N
         counters->do_resample = (resample_tau > 0.0 && !(__ddiv_rn(1.0, sq) < __dmul_rn(resample_tau, (double)n))) ? 0ull : 1ull;
-        counters->fold_rounds = (unsigned long long)max(info_sum.rounds, info_cum.rounds);
-        counters->fold_heads = (unsigned long long)max(info_sum.heads, info_cum.heads);
-        counters->fold_fallback = (unsigned long long)(info_sum.fallback | (info_cum.fallback << 1));
+        counters->fold_rounds = (unsigned long long)max(max(info_sum.rounds, info_cum.rounds), info_sq.rounds);
+        counters->fold_heads = (unsigned long long)max(max(info_sum.heads, info_cum.heads), info_sq.heads);
+        counters->fold_fallback = (unsigned long long)(info_sum.fallback | (info_cum.fallback << 1) | (info_sq.fallback << 2));
     }
     FOLD_STAMP(7);
 }
 
 static size_t weights_tile_bytes() { return sizeof(double) * FOLD_THREADS * (FOLD_LREG + 1); }
 // cluster size by population: 512 threads x 16 elements per CTA, 1 / 2 / 4 / 8 CTAs up to 65,536 particles;
-// beyond that the generic kernel (8 CTAs x 1024 threads, chunks re-read from global memory)
-void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t n_total, double* w_norm,
-                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters) {
+// beyond that the generic kernel (8 CTAs x 1024 threads, chunks of ceil(N / 8192) re-read from global memory)
+WeightsShape weights_shape(uint32_t n_total) {
     uint32_t c = 1u;
     while (c < (uint32_t)W_CLUSTER && (uint64_t)c * FOLD_THREADS * FOLD_LREG < n_total) c <<= 1;
-    const bool regs = (uint64_t)c * FOLD_THREADS * FOLD_LREG >= n_total;
+    WeightsShape s;
+    s.cluster = c;
+    s.regs = (uint64_t)c * FOLD_THREADS * FOLD_LREG >= n_total;
+    s.threads = s.regs ? (uint32_t)FOLD_THREADS : (uint32_t)FOLD_GENERIC_THREADS;
+    s.chunk = s.regs ? (uint32_t)FOLD_LREG : (uint32_t)(((uint64_t)n_total + c * s.threads - 1u) / (c * s.threads));
+    return s;
+}
+void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t n_total, double* w_norm,
+                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters) {
+    const WeightsShape shape = weights_shape(n_total);
+    const uint32_t c = shape.cluster;
+    const bool regs = shape.regs;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(c, 1, 1);
-    cfg.blockDim = dim3(regs ? FOLD_THREADS : FOLD_GENERIC_THREADS, 1, 1);
+    cfg.blockDim = dim3(shape.threads, 1, 1);
     cfg.dynamicSmemBytes = regs ? weights_tile_bytes() : 0;
     cfg.stream = stream;
     cudaLaunchAttribute attr[2];

@@ -502,18 +502,25 @@ def debug_stream(seed, step, first, count, device=0):
     return z, float(u[0])
 
 
-def debug_resample(raw_weights, u01: float, device=0, timing=False):
+def debug_resample(raw_weights, u01: float, device=0, timing=False, tau=0.0):
     """normalize_weights + argmax + resample indices on the device for caller-supplied raw weights
-    (the step's own k_weights / k_resample_indices). Returns a dict: idx, max_particle, norm, cum,
-    clamped, fold_rounds, fold_heads, fold_fallback (+ us = (k_weights, k_resample_indices) with timing)."""
+    (the step's own k_weights / k_resample_indices) with the adaptive-resampling threshold tau
+    (resample_threshold). Returns a dict: idx, max_particle, norm, cum, clamped, fold_rounds, fold_heads,
+    fold_fallback, n_eff, do_resample, and the launch k_weights used: cluster (CTAs), threads (per CTA), chunk
+    (elements per thread), regs (elements in registers, else the generic kernel) (+ us = (k_weights,
+    k_resample_indices) with timing)."""
     w = np.ascontiguousarray(raw_weights, np.float64).reshape(-1)
     n = w.size
     idx = np.zeros(n, np.uint32); norm = np.zeros(n, np.float64); cum = np.zeros(n, np.float64)
     info = np.zeros(4, np.uint64); us = np.zeros(2, np.float32); mp = C.c_uint64(0)
-    _lib.check(_lib.load().slamrs_gpu_debug_resample(device, _ptr(w), n, float(u01), _ptr(idx), C.byref(mp), _ptr(norm),
-                                                     _ptr(cum), _ptr(info), _ptr(us) if timing else None))
+    n_eff = C.c_double(0.0); do_resample = C.c_uint64(0); shape = np.zeros(4, np.uint64)
+    _lib.check(_lib.load().slamrs_gpu_debug_resample_adaptive(
+        device, _ptr(w), n, float(u01), float(tau), _ptr(idx), C.byref(mp), _ptr(norm), _ptr(cum), _ptr(info),
+        _ptr(us) if timing else None, C.byref(n_eff), C.byref(do_resample), _ptr(shape)))
     out = dict(idx=idx, max_particle=int(mp.value), norm=norm, cum=cum, clamped=int(info[0]), fold_rounds=int(info[1]),
-               fold_heads=int(info[2]), fold_fallback=int(info[3]))
+               fold_heads=int(info[2]), fold_fallback=int(info[3]), n_eff=float(n_eff.value),
+               do_resample=bool(do_resample.value), cluster=int(shape[0]), threads=int(shape[1]), chunk=int(shape[2]),
+               regs=bool(shape[3]))
     if timing:
         out["us"] = (float(us[0]), float(us[1]))
     return out
