@@ -236,6 +236,34 @@ int slamrs_gpu_sim_scan(slamrs_gpu_handle* h, const float* segments_xyxy, uint32
 int slamrs_gpu_get_scan(slamrs_gpu_handle* h, float* out_angle, float* out_dist, uint8_t* out_valid, uint32_t cap,
                         uint32_t* out_n);
 
+/* ------------------------------------------------------------------ scan-matching pose refinement */
+
+/* Not in the reference (the slam.rs:60 TODO). Off by default; while it is off the step is unchanged. When it is on,
+ * each sampled pose is moved onto its particle's own pre-update grid before the likelihood, by a hill climb on an
+ * integer score, bit-exact against the CPU oracle:
+ *   S(pose) = sum over valid beams of max((r+1)^2 - (dx^2 + dy^2)) over the occupied cells (counters' log-odds > 0)
+ *             at offsets (dx, dy) in [-r, r]^2 of the endpoint's cell (0 when there is none or the endpoint is off
+ *             the grid);
+ *   for level = 0 .. levels-1 (steps step_xy * 2^-level, step_theta * 2^-level), while moves < max_moves: score
+ *   (x+d, y, t), (x-d, y, t), (x, y+d, t), (x, y-d, t), (x, y, t+dt), (x, y, t-dt); move to the first best one if it
+ *   scores more than the current pose, else go to the next level.
+ * The refined pose replaces the sample, and the motion log-density is recomputed from the old pose to it. The scan is
+ * then weighted and integrated at the refined pose. One more kernel per step. */
+typedef struct slamrs_gpu_scan_match {
+    uint32_t struct_size;   /* = sizeof(slamrs_gpu_scan_match) */
+    uint32_t radius;        /* 0..2 cells */
+    float step_xy;          /* metres, finite, > 0 */
+    float step_theta;       /* radians, finite, > 0 */
+    uint32_t levels;        /* 1..8 */
+    uint32_t max_moves;     /* 1..1024 */
+} slamrs_gpu_scan_match;
+/* Takes effect at the next step; NULL turns the matcher off. With world_size > 1 every rank sets the same value before
+ * the same step. A localiser handle returns SLAMRS_E_INVALID_ARG. */
+int slamrs_gpu_set_scan_match(slamrs_gpu_handle* h, const slamrs_gpu_scan_match* m);
+/* Of this rank's particles in the last step: {particles that moved, total moves, poses scored (start poses included),
+ * particles that stopped at max_moves}. All zero when the last step ran without the matcher. Synchronises. */
+int slamrs_gpu_get_scan_match_stats(slamrs_gpu_handle* h, uint64_t out[4]);
+
 /* ------------------------------------------------------------------ localisation on a loaded map */
 
 /* Monte Carlo localisation: GridMapSlam::update (slam.rs:46-75) with the map held fixed and shared by every particle

@@ -91,6 +91,17 @@ pub struct slamrs_gpu_sensor_model {
     pub occupied_above: f32,
 }
 
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_scan_match {
+    pub struct_size: u32,
+    pub radius: u32,
+    pub step_xy: f32,
+    pub step_theta: f32,
+    pub levels: u32,
+    pub max_moves: u32,
+}
+
 extern "C" {
     pub fn slamrs_gpu_grid_cells(extent: f32, resolution: f32, out_cells: *mut u32) -> c_int;
     pub fn slamrs_gpu_nccl_unique_id(out: *mut u8) -> c_int;
@@ -141,4 +152,6 @@ extern "C" {
     pub fn slamrs_gpu_create_localizer(cfg: *const slamrs_gpu_config, model: *const slamrs_gpu_sensor_model, map_probability: *const f64, out: *mut *mut slamrs_gpu_handle) -> c_int;
     pub fn slamrs_gpu_get_sensor_terms(h: *mut slamrs_gpu_handle, out_cells: *mut f64) -> c_int;
     pub fn slamrs_gpu_get_log_odds(h: *mut slamrs_gpu_handle, particle: u64, out_cells: *mut f64) -> c_int;
+    pub fn slamrs_gpu_set_scan_match(h: *mut slamrs_gpu_handle, m: *const slamrs_gpu_scan_match) -> c_int;
+    pub fn slamrs_gpu_get_scan_match_stats(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
 }

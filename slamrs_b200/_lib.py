@@ -35,6 +35,7 @@ EXPORTS = [
     "slamrs_gpu_get_extents", "slamrs_gpu_debug_resample", "slamrs_gpu_debug_resample_adaptive", "slamrs_gpu_init_uniform",
     "slamrs_gpu_map_probability_async", "slamrs_gpu_map_wait",
     "slamrs_gpu_create_localizer", "slamrs_gpu_get_sensor_terms",
+    "slamrs_gpu_set_scan_match", "slamrs_gpu_get_scan_match_stats",
 ]
 MAP_F64, MAP_F32, MAP_U8 = 0, 1, 2
 SENSOR_BEAM_ENDPOINT, SENSOR_LIKELIHOOD_FIELD = 0, 1
@@ -58,6 +59,11 @@ class Config(C.Structure):
 class SensorModel(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("kind", C.c_uint32), ("sigma", C.c_float), ("z_rand", C.c_float),
                 ("occupied_above", C.c_float)]
+
+
+class ScanMatch(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("radius", C.c_uint32), ("step_xy", C.c_float), ("step_theta", C.c_float),
+                ("levels", C.c_uint32), ("max_moves", C.c_uint32)]
 
 
 class Stats(C.Structure):
@@ -135,6 +141,8 @@ def load():
     L.slamrs_gpu_create_localizer.restype = i
     L.slamrs_gpu_create_localizer.argtypes = [C.POINTER(Config), C.POINTER(SensorModel), vp, C.POINTER(vp)]
     L.slamrs_gpu_get_sensor_terms.restype = i; L.slamrs_gpu_get_sensor_terms.argtypes = [vp, vp]
+    L.slamrs_gpu_set_scan_match.restype = i; L.slamrs_gpu_set_scan_match.argtypes = [vp, C.POINTER(ScanMatch)]
+    L.slamrs_gpu_get_scan_match_stats.restype = i; L.slamrs_gpu_get_scan_match_stats.argtypes = [vp, vp]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
     L.slamrs_gpu_debug_resample_adaptive.restype = i

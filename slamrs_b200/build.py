@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libslamrs_gpu.so")
 SOURCES = ["kernels_likelihood.cu", "kernels_ray.cu", "kernels_resample.cu", "kernels_copy.cu", "kernels_misc.cu",
-           "kernels_localize.cu", "comm.cu", "api.cu"]
+           "kernels_localize.cu", "kernels_scan_match.cu", "comm.cu", "api.cu"]
 HEADERS = ["kernels.cuh", "kernels_common.cuh", "slam_device.cuh", "libm_f32.cuh", "shared_stream.cuh", "comm.h",
            os.path.join("..", "..", "include", "slamrs_gpu.h")]
 

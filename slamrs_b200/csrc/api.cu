@@ -134,6 +134,12 @@ struct slamrs_gpu_handle {
     bool localizer = false;
     double* d_loc_terms = nullptr;   // n_cells
     double loc_outside = 0.0;        // term of an endpoint off the grid
+    // scan-matching pose refinement (slamrs_gpu_set_scan_match)
+    bool match_on = false;
+    ScanMatchParams match{};
+    uint2* d_match_stats = nullptr;  // n_local x {moves, poses scored} of the last step that ran the matcher
+    bool match_last_step = false;    // the last issued step ran it
+    uint32_t match_last_max_moves = 0;
 };
 
 namespace {
@@ -305,6 +311,7 @@ void free_all(slamrs_gpu_handle* h) {
     if (h->ev_plan) cudaEventDestroy(h->ev_plan);
     if (h->ev_sort) cudaEventDestroy(h->ev_sort);
     cudaFree(h->d_order); cudaFree(h->d_valid_list); cudaFree(h->d_n_valid);
+    cudaFree(h->d_match_stats);
     if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
     for (int k = 0; k < 2; ++k) {
         cudaFree(h->d_export_async[k]);
@@ -828,6 +835,49 @@ int slamrs_gpu_get_sensor_terms(slamrs_gpu_handle* h, double* out_cells) {
     return SLAMRS_OK;
 }
 
+int slamrs_gpu_set_scan_match(slamrs_gpu_handle* h, const slamrs_gpu_scan_match* m) {
+    if (!h) return SLAMRS_E_INVALID_ARG;
+    if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a localizer does not scan-match");
+    if (!m) {
+        h->match_on = false;
+        return SLAMRS_OK;
+    }
+    if (m->struct_size != sizeof(slamrs_gpu_scan_match))
+        return fail(h, SLAMRS_E_INVALID_ARG, "slamrs_gpu_scan_match struct_size mismatch");
+    if (m->radius > 2u) return fail(h, SLAMRS_E_INVALID_ARG, "scan match radius must be 0, 1 or 2 cells");
+    if (!(m->step_xy > 0.0f) || !isfinite(m->step_xy))
+        return fail(h, SLAMRS_E_INVALID_ARG, "scan match step_xy must be a positive finite number of metres");
+    if (!(m->step_theta > 0.0f) || !isfinite(m->step_theta))
+        return fail(h, SLAMRS_E_INVALID_ARG, "scan match step_theta must be a positive finite number of radians");
+    if (m->levels < 1u || m->levels > 8u) return fail(h, SLAMRS_E_INVALID_ARG, "scan match levels must lie in 1..8");
+    if (m->max_moves < 1u || m->max_moves > 1024u)
+        return fail(h, SLAMRS_E_INVALID_ARG, "scan match max_moves must lie in 1..1024");
+    if (!h->d_match_stats) {
+        DeviceGuard g(h->device);
+        CU_TRY(h, cudaMalloc(&h->d_match_stats, sizeof(uint2) * h->n_local));
+    }
+    h->match = ScanMatchParams{m->radius, m->step_xy, m->step_theta, m->levels, m->max_moves};
+    h->match_on = true;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_get_scan_match_stats(slamrs_gpu_handle* h, uint64_t out[4]) {
+    if (!h || !out) return SLAMRS_E_INVALID_ARG;
+    out[0] = out[1] = out[2] = out[3] = 0;
+    if (!h->match_last_step) return SLAMRS_OK;
+    DeviceGuard g(h->device);
+    std::vector<uint2> per(h->n_local);
+    CU_TRY(h, cudaMemcpyAsync(per.data(), h->d_match_stats, sizeof(uint2) * h->n_local, cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    for (const uint2& v : per) {
+        out[0] += v.x > 0u;
+        out[1] += v.x;
+        out[2] += v.y;
+        out[3] += v.x == h->match_last_max_moves;
+    }
+    return SLAMRS_OK;
+}
+
 void slamrs_gpu_destroy(slamrs_gpu_handle* h) {
     if (h && getenv("SLAMRS_RAY_TRACE_PRINT")) {
         unsigned long long tr[18];
@@ -956,8 +1006,10 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     launch_motion_likelihood(s, h->geom, od, scan, h->d_pose[cur], h->d_slot[cur], h->defer ? h->d_alias : nullptr, h->d_cells, h->d_meta, h->cells_per_grid,
                              h->d_results, h->first, h->n_local, caller ? h->d_z : nullptr, h->cfg.seed, h->step, h->d_term_table, h->d_valid_list, h->d_n_valid,
                              h->d_carry, h->d_counters, h->p2p_exchange ? h->d_peer_results : nullptr, res_off, h->rank, h->world,
-                             h->d_readers, (uint32_t)n_zero);
-    h->launches += 2;   // k_motion + k_likelihood
+                             h->d_readers, (uint32_t)n_zero, h->match_on ? &h->match : nullptr, h->d_match_stats);
+    h->launches += h->match_on ? 3 : 2;   // k_motion (+ k_scan_match) + k_likelihood
+    h->match_last_step = h->match_on;
+    h->match_last_max_moves = h->match.max_moves;
     // 2. the one exchange step: every GPU needs every particle's weight, pose and slot. Default:
     //    k_likelihood has already stored each record into every peer (NVLink), only the barrier is
     //    left. SLAMRS_FLAG_NCCL_EXCHANGE: ncclAllGather of the shard instead.

@@ -7,6 +7,8 @@
 //                                          results stored into every peer GPU; k_peer_barrier
 //   kernels_ray.cu         k_ray_update*   map.rs:71-106 + ray.rs:21-110 + map.rs:148-172 (integrate):
 //                                          one CTA per surviving particle, shared-memory disc window
+//   kernels_scan_match.cu  k_scan_match    scan-matching pose refinement (extension, off by default): one warp
+//                                          per particle, between k_motion and k_likelihood
 //   kernels_resample.cu    k_weights       particle.rs:40-56, 59-65 + the running sum of :85-91 (8-CTA cluster)
 //                          k_resample_indices  particle.rs:78-101 + survivor list;  k_plan  keep / copy lists
 //   kernels_copy.cu        k_copy, k_copy_prepare / k_copy_boxed / k_commit_boxes   particle.rs:97-100 clone()
@@ -149,6 +151,12 @@ __device__ __forceinline__ RayItem ray_item_at(const RayItem* __restrict__ clone
     return owners[n_local - 1u - (k - n_ro)];
 }
 // ---- launch wrappers (all asynchronous on `stream`) ----
+// scan-matching pose refinement (slamrs_gpu_scan_match), between k_motion and k_likelihood
+struct ScanMatchParams {
+    uint32_t radius;
+    float step_xy, step_theta;
+    uint32_t levels, max_moves;
+};
 void launch_motion_likelihood(cudaStream_t stream, MapGeom geom, OdomModel od, ScanDevice scan,
                               const float* pose_cur, const int32_t* slot_of, const int32_t* alias_of /* may be null */,
                               const uint32_t* cells,
@@ -161,8 +169,14 @@ void launch_motion_likelihood(cudaStream_t stream, MapGeom geom, OdomModel od, S
                               ParticleResult* const* peer_results /* null: no fused exchange */,
                               uint32_t peer_offset /* records in front of this step's generation */, uint32_t rank,
                               uint32_t world, uint32_t* zero_words /* n_zero words that k_motion clears (may be null with 0) */,
-                              uint32_t n_zero);
+                              uint32_t n_zero, const ScanMatchParams* match /* null: no scan matching */,
+                              uint2* match_stats /* with match: n_local x {moves, poses scored} */);
 void launch_fill_term_table(cudaStream_t stream, double* table);
+void launch_scan_match(cudaStream_t stream, MapGeom geom, ScanMatchParams mp, OdomModel od, const float* pose_cur,
+                       const int32_t* alias_of /* may be null */, const uint32_t* cells, const SlotMeta* meta,
+                       size_t cells_per_grid, ParticleResult* results, uint32_t first_particle, uint32_t n_local,
+                       const float2* valid_beams, const uint32_t* n_valid,
+                       uint2* stats /* n_local x {moves, poses scored} */);
 constexpr uint32_t PEER_MAX_WORLD = 64;
 void launch_peer_barrier(cudaStream_t stream, unsigned long long* const* peer_flags, unsigned long long* my_flags,
                          uint32_t rank, uint32_t world, unsigned long long epoch, unsigned long long timeout_ns,

@@ -102,6 +102,15 @@ __device__ __forceinline__ double block_excl_scan_f64(double v, double* warp_tot
     return lane == 0 ? warp_tot[wid] : __dadd_rn(warp_tot[wid], within);
 }
 
+// The motion log-density Odometry::probabiliy_of (robot.rs:152-167) of a move from (ox, oy, otheta) to (nx, ny, ntheta)
+__device__ __forceinline__ double motion_log_density(const OdomModel& od, float ox, float oy, float otheta, float nx,
+                                                     float ny, float ntheta) {
+    const float dx = __fsub_rn(ox, nx), dy = __fsub_rn(oy, ny);
+    const float moved = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+    const double ad = angle_diff((double)otheta, (double)ntheta);
+    return __dadd_rn(log(normal_pdf((double)moved, od.mean_c, od.std_c)), log(normal_pdf(ad, od.mean_t, od.std_t)));
+}
+
 // Odometry::sample (robot.rs:170-183) and the motion log-density Odometry::probabiliy_of (robot.rs:152-167) of local
 // particle p (global index gp) moved from pose_cur: the draws come from z_draws (RNG_CALLER) or the shared stream.
 // Returns the new pose and, in `weight`, the log-density (slot is left to the caller).
@@ -123,12 +132,8 @@ __device__ __forceinline__ ParticleResult motion_step(const OdomModel& od, const
     slamrs_libm::sincosf_exact(ntheta, &sn, &cs);
     const float nx = __fadd_rn(ox, __fmul_rn(cs, center_distance));
     const float ny = __fadd_rn(oy, __fmul_rn(sn, center_distance));
-    // Odometry::probabiliy_of(old, new)
-    const float dx = __fsub_rn(ox, nx), dy = __fsub_rn(oy, ny);
-    const float moved = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-    const double ad = angle_diff((double)otheta, (double)ntheta);
     ParticleResult r;
-    r.weight = __dadd_rn(log(normal_pdf((double)moved, od.mean_c, od.std_c)), log(normal_pdf(ad, od.mean_t, od.std_t)));
+    r.weight = motion_log_density(od, ox, oy, otheta, nx, ny, ntheta);   // Odometry::probabiliy_of(old, new)
     r.x = nx; r.y = ny; r.theta = ntheta;
     r.slot = -1;
     return r;

@@ -114,9 +114,12 @@ void launch_motion_likelihood(cudaStream_t stream, MapGeom geom, OdomModel od, S
                               const double* term_table, float2* valid_beams, uint32_t* n_valid,
                               const double* carry, const StepCounters* counters,
                               ParticleResult* const* peer_results, uint32_t peer_offset, uint32_t rank, uint32_t world,
-                              uint32_t* zero_words, uint32_t n_zero) {
+                              uint32_t* zero_words, uint32_t n_zero, const ScanMatchParams* match, uint2* match_stats) {
     k_motion<<<(n_local + 127u) / 128u, 128, 0, stream>>>(od, pose_cur, slot_of, results, first_particle, n_local,
                                                          z_draws, seed, step, scan, valid_beams, n_valid, zero_words, n_zero);
+    if (match)   // refines the sampled poses in results[] before the likelihood reads them
+        launch_scan_match(stream, geom, *match, od, pose_cur, alias_of, cells, meta, cells_per_grid, results, first_particle,
+                          n_local, valid_beams, n_valid, match_stats);
     launch_pdl(k_likelihood, dim3((n_local + LK_WARPS - 1) / LK_WARPS), dim3(LK_WARPS * 32), 0, stream, geom, scan, alias_of, cells,
                meta, cells_per_grid, results, first_particle, n_local, term_table, valid_beams, n_valid, carry, counters,
                peer_results, peer_offset, rank, world);

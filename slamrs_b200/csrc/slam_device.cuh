@@ -24,6 +24,8 @@ __device__ __forceinline__ double cell_log_odds(uint32_t cell) {
     const double no = (double)(cell >> 16);
     return __dadd_rn(__dmul_rn(nf, SLAMRS_L_FREE), __dmul_rn(no, SLAMRS_L_OCC));
 }
+// the scan matcher's occupancy test: log-odds > 0. No occupied hit means log-odds <= 0, so only cells with one read f64.
+__device__ __forceinline__ bool cell_occupied(uint32_t cell) { return (cell >> 16) != 0u && cell_log_odds(cell) > 0.0; }
 // LogOdds::probability, math.rs:135-137
 __device__ __forceinline__ double log_odds_probability(double l) { return 1.0 - 1.0 / (1.0 + exp(l)); }
 

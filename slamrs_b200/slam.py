@@ -121,6 +121,27 @@ class GpuPlacement:
     slot_cells: int = 0      # 0 = whole-grid slots; power of two >= 256 = windowed slots (see slamrs_gpu.h)
 
 
+@dataclass
+class ScanMatcher:
+    """Scan-matching pose refinement of the SLAM step (slamrs_gpu_scan_match; not in the reference, off by default).
+    Each sampled pose climbs, before the likelihood, to the pose whose beam endpoints lie nearest to occupied cells of
+    its particle's own map: `radius` cells around each endpoint are searched (0..2), the climb tries steps of
+    `step_xy` metres and `step_theta` radians, halves them `levels` - 1 times (1..8) and stops after `max_moves`
+    accepted moves (1..1024). The defaults are what the quality measurement in DESIGN.md used."""
+    radius: int = 1
+    step_xy: float = 0.1
+    step_theta: float = 0.05
+    levels: int = 4
+    max_moves: int = 32
+
+    def to_struct(self):
+        m = _lib.ScanMatch()
+        m.struct_size = C.sizeof(_lib.ScanMatch)
+        m.radius, m.levels, m.max_moves = int(self.radius), int(self.levels), int(self.max_moves)
+        m.step_xy, m.step_theta = float(self.step_xy), float(self.step_theta)
+        return m
+
+
 def grid_cells(extent: float, resolution: float) -> int:
     """Map::new grid sizing (map.rs:28-31) as the library computes it."""
     out = C.c_uint32(0)
@@ -351,6 +372,20 @@ class GridMapSlam:
     @property
     def launch_count(self) -> int:
         return int(self._L.slamrs_gpu_launch_count(self._h))
+
+    # ------------------------------------------------------------------ scan matching (extension)
+    def set_scan_matcher(self, matcher: Optional[ScanMatcher]) -> None:
+        """Refine every sampled pose by scan matching from the next update on; None turns it off (the default).
+        Multi-GPU: every rank sets the same matcher before the same update."""
+        m = None if matcher is None else matcher.to_struct()
+        _lib.check(self._L.slamrs_gpu_set_scan_match(self._h, None if m is None else C.byref(m)), self._h)
+
+    def scan_match_stats(self) -> dict:
+        """Of this rank's particles in the last update: moved (particles), moves (total), scored (poses, start poses
+        included), capped (particles that stopped at max_moves). All zero after an update without the matcher."""
+        out = np.zeros(4, np.uint64)
+        _lib.check(self._L.slamrs_gpu_get_scan_match_stats(self._h, _ptr(out)), self._h)
+        return dict(zip(("moved", "moves", "scored", "capped"), (int(v) for v in out)))
 
     # ------------------------------------------------------------------ introspection (tests / bench)
     def stats(self) -> dict:
