@@ -42,7 +42,7 @@ enum slamrs_status {
     SLAMRS_E_STAGING = -6,       /* cross-GPU migration needed more free grid slots than exist */
     SLAMRS_E_NOT_LOCAL = -7,     /* debug accessor asked for a particle owned by another rank */
     SLAMRS_E_INTERNAL = -8,
-    SLAMRS_E_WINDOW = -9         /* a grid's informed extent outgrew its windowed slot (slot_cells too small) */
+    SLAMRS_E_WINDOW = -9         /* a scan could not be proven to fit a grid's windowed slot (see slot_cells) */
 };
 
 enum slamrs_rng_mode {
@@ -99,8 +99,17 @@ typedef struct slamrs_gpu_config {
     uint32_t slot_cells;   /* 0: every particle's slot holds the whole grid. Otherwise a power of two >= 256:
                               a slot holds a slot_cells x slot_cells torus of the grid, enough for the informed
                               extent of one particle's map (everything else is the prior). Memory per particle
-                              drops from 4*W*H to 4*slot_cells^2 bytes; an extent that outgrows it is reported
-                              as SLAMRS_E_WINDOW. */
+                              drops from 4*W*H to 4*slot_cells^2 bytes. Before a grid receives a scan, the step
+                              proves that its extent will still fit, conservatively: with reach = ceil(m / resolution)
+                              + 6 cells, m the largest |distance| over EVERY beam of the scan, valid or not (a
+                              non-finite distance is unbounded; a device-resident scan uses its max_dist), the square
+                              of side 2*reach + 1 around the start cell (columns widened to multiples of 8, clipped to
+                              the grid) united with the informed extent must fit slot_cells x slot_cells. Otherwise
+                              that grid is left as it was and the step reports SLAMRS_E_WINDOW, even where the cells
+                              the rays would write fit: one long beam (e.g. an invalid reading at 13 m on 5 cm cells
+                              with slot_cells = 512) refuses the step for every particle, and a scan without beams
+                              still has reach 6. set_cells refuses an image whose extent, columns widened to
+                              multiples of 8, does not fit. */
     float resample_threshold; /* 0 (default): resample after every update, as the reference does (slam.rs:74).
                                  tau in (0, 1]: resample only when the effective number of particles
                                  (particle.rs:59-65) is below tau * N; otherwise every particle stays in place and

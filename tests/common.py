@@ -1,6 +1,8 @@
 """Shared helpers of the parity tests: lockstep drivers for the GPU path and the CPU oracle."""
 from __future__ import annotations
 
+import os
+
 import numpy as np
 
 from slamrs_b200 import GpuPlacement, GridMapSlam, GridMapSlamConfig, Observation, Odometry
@@ -31,6 +33,18 @@ def at_scale_config(n):
 
 def at_scale_scans(steps):
     return make_scans(10.0, 360, 6.0, steps)
+
+
+def host_gib() -> float:
+    """MemAvailable of this host in GiB (0 when unknown): the oracle's tiles at full populations need tens of GiB."""
+    try:
+        with open("/proc/meminfo") as f:
+            for line in f:
+                if line.startswith("MemAvailable"):
+                    return int(line.split()[1]) / 2 ** 20
+    except OSError:
+        pass
+    return 0.0
 
 
 def oracle_slam(O, cfg: GridMapSlamConfig, track_counts=True):
@@ -116,3 +130,95 @@ def lockstep(O, cfg: GridMapSlamConfig, scans, rng_mode=_lib.RNG_SHARED_STREAM, 
         gpu.close()
         osl.close()
     return errs
+
+
+def install_cells(gpu: GridMapSlam, osl, particle: int, cells) -> None:
+    """Installs one hand-built grid on both sides: packed hit counters (free | occupied << 16, index
+    row * grid_h + column) into the device's slot and the same counters, with their log-odds, into the oracle
+    (an oracle.scan_match_oracle.ScanMatchOracle; without a matcher set it is the plain oracle)."""
+    c = np.ascontiguousarray(cells, np.uint32).reshape(-1)
+    gpu.set_cells(particle, c)
+    osl.set_counts(particle, (c & 0xFFFF).astype(np.uint16), (c >> 16).astype(np.uint16))
+
+
+def lockstep_following_device_weights(O, cfg, scans, probes, check_map=True, flags=0, slot_cells=0, pre_step=None):
+    """Lockstep of one sparse oracle with one device handle per entry of `flags` (an int or a sequence of flag
+    sets), all on the same scans and seed. The device's exp/log differ from glibc's in the last bit, so raw weights
+    agree to ~1e-12 relative, not bit for bit, and at large populations a resampling threshold lands that close to
+    a prefix sum often enough to matter. Each step therefore (1) compares the oracle's own raw weights with the
+    device's against WEIGHT_RTOL and (2) lets the oracle resample on the device's raw weights: on identical numbers
+    the index vector, the argmax, every pose and every probed grid must then match bit for bit, on every handle.
+
+    probes(step, idx, gpu) -> particles whose counters are compared (gpu: the first handle); pre_step(step, gpus,
+    osl) runs before each step. Returns (worst relative weight error, distinct survivors per step, per step the
+    list of every handle's stats())."""
+    modes = list(flags) if isinstance(flags, (list, tuple)) else [flags]
+    osl = O.OracleSlam(cfg.position, cfg.width, cfg.height, cfg.resolution, cfg.n_particles, True, sparse=True)
+    osl.set_threads(os.cpu_count() or 1)
+    worst_w = 0.0
+    survivors, stats = [], []
+    gpus = []
+    try:
+        for f in modes:
+            gpus.append(GridMapSlam(cfg, GpuPlacement(seed=SEED, flags=f, slot_cells=slot_cells)))
+        for step, (obs, odo) in enumerate(scans):
+            if pre_step is not None:
+                pre_step(step, gpus, osl)
+            for g in gpus:
+                g.update(obs, odo)
+            w_gpu, raw_gpu = gpus[0].weights()
+            for g in gpus[1:]:
+                assert np.array_equal(g.weights()[1].view(np.int64), raw_gpu.view(np.int64)), (step, g.placement.flags)
+            osl.set_weight_override(raw_gpu)
+            rc, _, _ = oracle_step(O, osl, obs, odo, step)
+            assert rc == 0
+            own = osl.own_raw_weights()
+            rel = np.max(np.abs(own - raw_gpu) / np.maximum(np.abs(own), 1e-300))
+            worst_w = max(worst_w, float(rel))
+            assert rel < WEIGHT_RTOL, (step, rel)
+            w_ref, _ = osl.weights()
+            idx_ref = osl.indices().astype(np.int64)
+            survivors.append(len(np.unique(idx_ref)))
+            p_ref = osl.poses().view(np.uint32)
+            ep_ref = osl.estimated_pose().view(np.uint32)
+            m_ref = osl.estimated_likelihood() if check_map else None
+            picked = probes(step, idx_ref, gpus[0])
+            counts_ref = {int(p): osl.counts(int(p)) for p in picked}
+            step_stats = []
+            for g in gpus:
+                w_gpu = g.weights()[0]
+                assert np.array_equal(w_ref.view(np.int64), w_gpu.view(np.int64)), "normalised weights differ on identical raw weights"
+                idx_gpu = g.resample_indices().astype(np.int64)
+                assert np.array_equal(idx_ref, idx_gpu), (step, g.placement.flags, np.nonzero(idx_ref != idx_gpu)[0][:8])
+                assert g.max_particle == osl.max_particle
+                assert np.array_equal(p_ref, g.poses().view(np.uint32)), (step, g.placement.flags)
+                st = g.stats()
+                assert st["resample_clamped"] == 0 and st["resample_exact_fallback"] == 0, st
+                ep = g.estimated_pose()
+                assert np.array_equal(ep_ref, np.array([ep.x, ep.y, ep.theta], np.float32).view(np.uint32))
+                if check_map:
+                    assert np.max(np.abs(m_ref - g.estimated_likelihood().data)) < 1e-12
+                for p, (nf, no) in counts_ref.items():
+                    gf, go = g.counts(p)
+                    assert np.array_equal(nf, gf) and np.array_equal(no, go), (step, g.placement.flags, p)
+                step_stats.append(st)
+            stats.append(step_stats)
+    finally:
+        for g in gpus:
+            g.close()
+        osl.close()
+    return worst_w, survivors, stats
+
+
+def cloned_probes(n):
+    """Probes for lockstep_following_device_weights: fixed particles, the most-cloned source's first and last
+    copy, and a particle cloned exactly once."""
+    def pick(step, idx, gpu=None):
+        src, first, counts = np.unique(idx, return_index=True, return_counts=True)
+        big = int(np.argmax(counts))
+        out = {0, n // 2, n - 1, int(first[big]), int(first[big] + counts[big] - 1)}
+        single = np.nonzero(counts == 1)[0]
+        if single.size:
+            out.add(int(first[single[0]]))
+        return sorted(out)
+    return pick

@@ -13,22 +13,23 @@ from slamrs_b200 import _lib
 from common import gpu_present, make_scans
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "tests", "cpp", "host_mirror_check")
 
 
-def _build():
+def _build(out_dir):
+    """Compiles the check program into out_dir (a test's temporary directory: the source tree may be read-only)."""
     _lib.load()
     libdir = os.path.join(ROOT, "slamrs_b200")
     src = os.path.join(ROOT, "tests", "cpp", "host_mirror_check.cpp")
-    cmd = ["g++", "-std=c++17", "-O2", src, "-o", BIN, "-L" + libdir, "-lslamrs_gpu", "-Wl,-rpath," + libdir]
+    exe = os.path.join(str(out_dir), "host_mirror_check")
+    cmd = ["g++", "-std=c++17", "-O2", src, "-o", exe, "-L" + libdir, "-lslamrs_gpu", "-Wl,-rpath," + libdir]
     env = dict(os.environ); env.pop("CXX", None)
     subprocess.run(cmd, check=True, env=env)
-    return BIN
+    return exe
 
 
 @pytest.mark.skipif(gpu_present(), reason="GPU present")
-def test_cpp_mirror_builds_and_refuses_to_run_without_gpu():
-    out = subprocess.run([_build(), "--no-gpu"], capture_output=True, text=True)
+def test_cpp_mirror_builds_and_refuses_to_run_without_gpu(tmp_path):
+    out = subprocess.run([_build(tmp_path), "--no-gpu"], capture_output=True, text=True)
     assert out.returncode == 0, out.stdout + out.stderr
     assert "no CPU fallback" in out.stdout
 
@@ -40,7 +41,7 @@ def test_cpp_mirror_matches_python_binding(tmp_path):
     with open(scan, "w") as f:
         for a, d, v in zip(obs.angle, obs.distance, obs.valid):
             f.write(f"{float(np.float32(a))!r} {float(np.float32(d))!r} {int(v)}\n")
-    out = subprocess.run([_build(), str(scan)], capture_output=True, text=True)
+    out = subprocess.run([_build(tmp_path), str(scan)], capture_output=True, text=True)
     assert out.returncode == 0, out.stdout + out.stderr
     lines = [ln.split() for ln in out.stdout.strip().splitlines()]
     assert len(lines) == 6

@@ -9,79 +9,14 @@ Each step therefore (1) compares the oracle's own weights with the device's agai
 (2) lets the oracle resample on the device's raw weights -- on identical numbers the index vector, the
 argmax, every pose and every probed grid must then match bit for bit (tests/test_gpu_resample_exact.py
 covers the index kernels on adversarial weights)."""
-import os
-
-import numpy as np
 import pytest
 
-from slamrs_b200 import GpuPlacement, GridMapSlam, GridMapSlamConfig
+from slamrs_b200 import GridMapSlamConfig
 from slamrs_b200.workloads import WORKLOADS
 
-from common import SEED, WEIGHT_RTOL, oracle_step
+from common import cloned_probes, host_gib, lockstep_following_device_weights
 
 pytestmark = pytest.mark.gpu
-
-
-def _host_gib():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable"):
-                    return int(line.split()[1]) / 2 ** 20
-    except OSError:
-        pass
-    return 0.0
-
-
-def _lockstep_following_device_weights(oracle, cfg, scans, probes, check_map=True, flags=0):
-    osl = oracle.OracleSlam(cfg.position, cfg.width, cfg.height, cfg.resolution, cfg.n_particles, True, sparse=True)
-    osl.set_threads(os.cpu_count() or 1)
-    worst_w = 0.0
-    survivors = []
-    with GridMapSlam(cfg, GpuPlacement(seed=SEED, flags=flags)) as gpu:
-        for step, (obs, odo) in enumerate(scans):
-            gpu.update(obs, odo)
-            w_gpu, raw_gpu = gpu.weights()
-            osl.set_weight_override(raw_gpu)
-            rc, _, _ = oracle_step(oracle, osl, obs, odo, step)
-            assert rc == 0
-            own = osl.own_raw_weights()
-            rel = np.max(np.abs(own - raw_gpu) / np.maximum(np.abs(own), 1e-300))
-            worst_w = max(worst_w, float(rel))
-            assert rel < WEIGHT_RTOL, (step, rel)
-            w_ref, _ = osl.weights()
-            assert np.array_equal(w_ref.view(np.int64), w_gpu.view(np.int64)), "normalised weights differ on identical raw weights"
-            idx_ref = osl.indices().astype(np.int64)
-            idx_gpu = gpu.resample_indices().astype(np.int64)
-            assert np.array_equal(idx_ref, idx_gpu), (step, np.nonzero(idx_ref != idx_gpu)[0][:8])
-            survivors.append(len(np.unique(idx_ref)))
-            assert gpu.max_particle == osl.max_particle
-            assert np.array_equal(osl.poses().view(np.uint32), gpu.poses().view(np.uint32))
-            st = gpu.stats()
-            assert st["resample_clamped"] == 0 and st["resample_exact_fallback"] == 0, st
-            ep = gpu.estimated_pose()
-            assert np.array_equal(osl.estimated_pose().view(np.uint32), np.array([ep.x, ep.y, ep.theta], np.float32).view(np.uint32))
-            if check_map:
-                assert np.max(np.abs(osl.estimated_likelihood() - gpu.estimated_likelihood().data)) < 1e-12
-            for p in probes(step, idx_ref):
-                nf, no = osl.counts(int(p))
-                gf, go = gpu.counts(int(p))
-                assert np.array_equal(nf, gf) and np.array_equal(no, go), (step, p)
-    osl.close()
-    return worst_w, survivors
-
-
-def _probes(n):
-    def pick(step, idx):
-        # fixed probes, the most-cloned source's first and last copy, a particle cloned exactly once
-        src, first, counts = np.unique(idx, return_index=True, return_counts=True)
-        big = int(np.argmax(counts))
-        out = {0, n // 2, n - 1, int(first[big]), int(first[big] + counts[big] - 1)}
-        single = np.nonzero(counts == 1)[0]
-        if single.size:
-            out.add(int(first[single[0]]))
-        return sorted(out)
-    return pick
 
 
 def test_lockstep_configs1_full_population(oracle):
@@ -90,32 +25,32 @@ def test_lockstep_configs1_full_population(oracle):
     cfg = wl.slam_config()
     sim = wl.simulator()
     scans = [sim.next_scan(wl.speed_left, wl.speed_right) for _ in range(5)]
-    worst, surv = _lockstep_following_device_weights(oracle, cfg, scans, _probes(cfg.n_particles))
+    worst, surv, _ = lockstep_following_device_weights(oracle, cfg, scans, cloned_probes(cfg.n_particles))
     assert surv[-1] < cfg.n_particles
 
 
 def test_lockstep_configs2_full_population(oracle):
     """configs[2]: 8,192 particles x 360 beams, 1024^2 grid, 4 scans (aliases, deferred copies and the
     survivors-only ray update all at the benchmark's own shape)."""
-    if _host_gib() < 24:
+    if host_gib() < 24:
         pytest.skip("needs ~24 GiB of host memory for the oracle's tiles")
     wl = WORKLOADS["c3"]
     cfg = wl.slam_config()
     sim = wl.simulator()
     scans = [sim.next_scan(wl.speed_left, wl.speed_right) for _ in range(4)]
-    worst, surv = _lockstep_following_device_weights(oracle, cfg, scans, _probes(cfg.n_particles), check_map=True)
+    worst, surv, _ = lockstep_following_device_weights(oracle, cfg, scans, cloned_probes(cfg.n_particles), check_map=True)
     assert 1 < surv[-1] < cfg.n_particles
 
 
 def test_lockstep_configs3_population_in_one_handle(oracle):
     """65,536 particles (the population of configs[3]) in one handle on a small grid: the exact left folds,
     the index search and the planner at the 8-GPU population; 3 scans."""
-    if _host_gib() < 16:
+    if host_gib() < 16:
         pytest.skip("needs ~16 GiB of host memory for the oracle's tiles")
     from slamrs_b200.simulator import Simulator, reference_scene
     n = 65536
     cfg = GridMapSlamConfig(position=(-6.4, -6.4), width=12.8, height=12.8, resolution=0.2, n_particles=n)
     sim = Simulator(reference_scene(5.0), n_beams=360, scanner_range=3.0, wheel_base=0.1)
     scans = [sim.next_scan(0.08, 0.10) for _ in range(3)]
-    worst, surv = _lockstep_following_device_weights(oracle, cfg, scans, _probes(n), check_map=True)
+    worst, surv, _ = lockstep_following_device_weights(oracle, cfg, scans, cloned_probes(n), check_map=True)
     assert 1 < surv[-1] < n
