@@ -884,8 +884,8 @@ void slamrs_gpu_destroy(slamrs_gpu_handle* h) {
         DeviceGuard g(h->device);
         cudaStreamSynchronize(h->stream);
         if (ray_trace(tr) == 0) {
-            fprintf(stderr, "ray trace: items fused %llu in-place %llu; cycles pop %llu setup %llu walk %llu fused_total %llu wait %llu inplace_wb %llu | fused: prepass %llu loop %llu barrier %llu\n",
-                    tr[16], tr[17], tr[0], tr[1], tr[2], tr[3], tr[4], tr[5], tr[8], tr[9], tr[10]);
+            fprintf(stderr, "ray trace: items fused %llu in-place %llu; cycles pop %llu setup %llu walk %llu fused_total %llu wait %llu inplace_wb %llu\n",
+                    tr[16], tr[17], tr[0], tr[1], tr[2], tr[3], tr[4], tr[5]);
             fprintf(stderr, "ray trace raw:");
             for (int k = 0; k < 18; ++k) fprintf(stderr, " [%d]%llu", k, tr[k]);
             fprintf(stderr, "\n");
@@ -918,7 +918,7 @@ int slamrs_gpu_upload_scan(slamrs_gpu_handle* h, const float* angle, const float
     h->order_valid = false;
     // window radius for the ray kernel: farthest measurement, in cells, plus the two extra steps of
     // apply_measurement (map.rs:97) and the slack that lets the ray kernel prove, per ray, that no cell
-    // leaves the window (see k_ray_update_packed). A non-finite distance still casts a ray, to the grid
+    // leaves the window (see ray_walk_packed). A non-finite distance still casts a ray, to the grid
     // border: its reach is unbounded, which selects the unfused ray update (cells outside the window take
     // the global-atomic path there; the fused update can only park a bounded number of them).
     float maxd = 0.0f;

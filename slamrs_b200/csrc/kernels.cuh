@@ -116,7 +116,7 @@ struct CopyItem {
 };
 
 // One work item of the ray update: a surviving local particle, its slot and the slot whose cells it
-// logically holds (root != slot: a clone that k_ray_update_packed makes private while it integrates the scan)
+// logically holds (root != slot: a clone that k_ray_update_half makes private while it integrates the scan)
 struct RayItem {
     uint32_t particle;
     int32_t slot, root;
@@ -191,7 +191,7 @@ size_t ray_half_xchg_bytes();               // per surviving particle: what its 
 int ray_trace(unsigned long long* out18);   // tuning builds (-DSLAMRS_RAY_TRACE): cycles per phase, summed over CTAs   // scratch of the fused path (uint32 words)
 // returns the shared-memory window size in cells through *window_cells
 // alive_list / counters->n_alive select the local particles to integrate (see launch_mark_alive); with the work
-// lists of RayLists (clones, owners) the packed kernel fuses the clones' copies into its write-back (readers /
+// lists of RayLists (clones, owners) the half-particle kernel fuses the clones' copies into its write-back (readers /
 // done: per-slot counters, zeroed by the caller before launch_resample_indices)
 cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan, const ParticleResult* results,
                               uint32_t first_particle, uint32_t n_local, const uint32_t* alive_list,

@@ -1,6 +1,9 @@
-// k_ray_update / k_ray_update_packed: Map::integrate (map.rs:71-106) with GridRayIterator
-// (ray.rs:21-110) and the inverse sensor model (map.rs:148-172); hit counters accumulated in a
-// shared-memory disc window, written back with 128-bit read-modify-writes.
+// The ray update: Map::integrate (map.rs:71-106) with GridRayIterator (ray.rs:21-110) and the inverse
+// sensor model (map.rs:148-172); hit counters accumulated in a shared-memory disc window, then added to the
+// grid. k_ray_update: 32-bit window cells, one CTA per particle (any beam count and grid side).
+// k_ray_update_packed / k_ray_update_half: 16-bit window cells and one walk (ray_walk_packed); a whole
+// particle per work item written back in place (row-major or windowed slots), or half a particle per work
+// item whose write-back also makes a clone's grid private (whole-grid tiled slots).
 #include "kernels_common.cuh"
 #include <cstdio>
 #include <cstdlib>
@@ -373,7 +376,7 @@ __host__ __device__ inline int ray_window_cells_upper_bound_packed(int radius) {
     return total;
 }
 
-// Facts the packed kernel's fast walk relies on (see DESIGN.md):
+// Facts the packed kernels' fast walk relies on (see DESIGN.md):
 //  * |x0 - centre_x| and |y0 - centre_y| never decrease along a walk (x only moves by x_inc, y
 //    only by y_inc, away from the start cell), IEEE rounding is monotone, so
 //    acc = fl(fl(dx^2) + fl(dy^2)) is non-decreasing along the ray. The inverse sensor model is
@@ -405,33 +408,39 @@ __device__ __forceinline__ unsigned ray_smid() { unsigned r; asm volatile("mov.u
 #define RAY_LOG_V(w, k, v) do { } while (0)
 #endif
 
-// The walk of every beam of one particle into the shared-memory window (GridRayIterator, ray.rs:21-110, with
-// the inverse sensor model of map.rs:148-172). Out of line on purpose: compiled on its own the free-run
-// loop stays the 25-instruction predicated block tools/sass_hot_loop.py checks for.
-__device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevice& scan, float px, float py, float ptheta, float sx,
-                                            float sy, int cx0, int cy0, int rad, int wy0, int wh, int band0, uint32_t* s_win,
-                                            const int2* s_row, const uint32_t* s_rowb, int* s_blo, int* s_bhi, int* s_ext,
-                                            uint32_t* __restrict__ grid, uint32_t* __restrict__ bands, bool fused,
-                                            uint32_t* s_nspill_p, uint32_t* __restrict__ my_spill, bool* saturated_p,
-                                            uint32_t* spilled_p, uint32_t* cell_steps_p) {
+// The walk of one particle's beams into the 16-bit shared-memory window (GridRayIterator, ray.rs:21-110, with the
+// inverse sensor model of map.rs:148-172), shared by k_ray_update_packed (every beam, `beams` = scan.order or null
+// for identity order) and k_ray_update_half (this half's list). `disc_in_grid`: the window holds every in-grid cell
+// within `rad` of the start cell in the rows this walk can reach. Out of line on purpose: compiled on its own the
+// free-run loop stays the 25-instruction predicated block tools/sass_hot_loop.py checks for.
+//
+// Hits that bypass the window (the 32nd occupied hit of a cell in one scan, zero-length rays, and cells outside
+// the window) take the exact path. kParkBypass: they are parked in my_spill and applied after the write-back --
+// a clone's own slot receives its cells only then; at most 4 occupied cells per ray (3 hits of a zero-length ray),
+// so RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS entries suffice when the window holds every cell a ray reaches.
+// Otherwise they go straight to the grid with a saturating CAS, widening the slot's band table where the window's
+// bands do not cover them.
+template <bool kParkBypass>
+__device__ __noinline__ void ray_walk_packed(const MapGeom& geom, const ScanDevice& scan, const uint16_t* beams, uint32_t n_walk,
+                                             float px, float py, float ptheta, float sx, float sy, int cx0, int cy0, int rad,
+                                             bool disc_in_grid, int wy0, int wh, int band0, uint32_t* s_win, const int2* s_row,
+                                             const uint32_t* s_rowb, int* s_blo, int* s_bhi, int* s_ext,
+                                             uint32_t* __restrict__ grid, uint32_t* __restrict__ bands, uint32_t* s_nspill_p,
+                                             uint32_t* __restrict__ my_spill, bool* saturated_p, uint32_t* spilled_p,
+                                             uint32_t* cell_steps_p) {
     const int gw = (int)geom.gw, gh = (int)geom.gh;
     const uint32_t win_base = (uint32_t)__cvta_generic_to_shared(s_win);
     bool saturated = false;
     uint32_t spilled = 0, cell_steps = 0;
-    // A clone's own slot receives its cells only at write-back, so the (rare) hits that bypass the window --
-    // the 32nd occupied hit of a cell in one scan -- are parked and applied after the write-back.
-    // At most 4 occupied cells per ray (3 hits of a zero-length ray): RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS
-    // entries suffice when the window holds every cell a ray reaches.
     ZeroLengthHits zero_length;
     auto exact_add = [&](int x, int y, uint32_t inc) {
-        if (fused) {
+        if constexpr (kParkBypass) {
             const uint32_t k = atomicAdd(s_nspill_p, 1u);
             if (k < RAY_SPILL_CAP) my_spill[k] = (uint32_t)x | ((uint32_t)y << 15) | (inc == CELL_OCC_INC ? 0x40000000u : 0u);
         } else {
             global_cell_add(&grid[phys_index(geom, (uint32_t)x, (uint32_t)y)], inc, &saturated);
         }
     };
-    const bool disc_in_grid = cx0 - rad >= 0 && cx0 + rad < gw && cy0 - rad >= 0 && cy0 + rad < gh;
     // The row table is read at every y-step of the walk. Its shared address is kept in a register the
     // compiler cannot re-derive: left to itself ptxas may rebuild it inside the loop (S2UR + ULEA per
     // step, seen in SASS after an unrelated change elsewhere in the kernel), which costs the walk ~15 %.
@@ -442,9 +451,8 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
         asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(rowb_base + 4u * (uint32_t)row) : "memory");
         return v;
     };
-    const uint32_t n_beams_walk = scan.n_beams;
-    for (uint32_t t = threadIdx.x; t < n_beams_walk; t += blockDim.x) {
-        const uint32_t b = scan.order ? scan.order[t] : t;   // similar ray lengths within a warp
+    for (uint32_t t = threadIdx.x; t < n_walk; t += blockDim.x) {
+        const uint32_t b = beams ? beams[t] : t;
         const float dist = scan.dist[b];
         float ex, ey;
         beam_endpoint(px, py, ptheta, scan.angle[b], dist, &ex, &ey);
@@ -508,8 +516,36 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
             const uint32_t x_inc2 = (uint32_t)(2 * x_inc);
             int ly = cy0 - wy0;
             uint32_t rb = load_rowb(ly);
-            // free run
-            while (remaining > 0) {
+            // The first cells of a walk are free whatever its direction: the cell reached after k steps is k cells from
+            // the start cell in the Manhattan sense, the start point lies inside the start cell, so both offsets to the
+            // cell centre are at most (cells + 0.5) and acc <= (k + 0.5)^2 + 0.25 < K^2 for k < K; with K^2 <= 0.999 x
+            // free_below (the margin dwarfs the f32 rounding of acc) those K cells pass `acc < free_below` without
+            // evaluating it. They take a loop without the distance arithmetic; the distance state is then rebuilt from
+            // the cell position -- cxf and cyf only ever held (integer + 0.5) exactly, so the rebuilt values are the
+            // accumulated ones bit for bit -- and the free run continues with the test.
+            {
+                const float kf = floorf(__fsqrt_rn(__fmul_rn(cls.free_below, 0.999f)));
+                int safe = (kf >= 1.0f && kf < 1.0e6f) ? (int)kf : 0;      // (NaN and tiny thresholds: none)
+                safe = min(safe, remaining);
+                remaining -= safe;
+                for (; safe > 0; --safe) {
+                    const uint32_t c2 = rb + x2;
+                    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(c2 & ~3u), "r"((c2 & 2u) ? 0x10000u : 1u) : "memory");
+                    if (error > 0.0f) {
+                        error = __fsub_rn(error, delta_x);
+                        ly += y_inc;
+                        rb = load_rowb(ly);
+                    } else {
+                        error = __fadd_rn(error, delta_y);
+                        x2 += x_inc2;
+                    }
+                }
+                cxf = __fadd_rn((float)(x2 >> 1), 0.5f);
+                cyf = __fadd_rn((float)(wy0 + ly), 0.5f);
+                dxs = __fsub_rn(sx, cxf); dys = __fsub_rn(sy, cyf);
+                dx2 = __fmul_rn(dxs, dxs); dy2 = __fmul_rn(dys, dys);
+            }
+            while (remaining > 0) {                    // free run
                 const float acc = __fadd_rn(dx2, dy2);
                 if (!(acc < cls.free_below)) break;
                 const uint32_t c2 = rb + x2;           // shared byte address of the 16-bit window cell
@@ -530,8 +566,7 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
                 }
                 remaining -= 1;
             }
-            // occupied run (hits only): bounded 5-bit field per scan, exact global path beyond it
-            if (cls.mid_inc != 0u) {
+            if (cls.mid_inc != 0u) {                   // occupied run (hits only): bounded 5-bit field, exact path beyond it
                 while (remaining > 0) {
                     const float acc = __fadd_rn(dx2, dy2);
                     if (acc > cls.prior_above) break;
@@ -609,13 +644,12 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
                         exact_add(x, y, is_free ? CELL_FREE_INC : CELL_OCC_INC);
                         ext_add(s_ext, x, y, x, y);
                         band_add(s_blo, s_bhi, band0, y, x, x);
-                        band_add_global(bands, geom, band0, x, y);
+                        if constexpr (!kParkBypass) band_add_global(bands, geom, band0, x, y);
                         spilled++;
                     }
                 }
             }
-            // GridRayIterator::next (ray.rs:96-104)
-            if (error > 0.0f) {
+            if (error > 0.0f) {                    // GridRayIterator::next (ray.rs:96-104)
                 y += y_inc;
                 error = __fsub_rn(error, delta_x);
                 cyf = __fadd_rn(cyf, y_step);
@@ -649,193 +683,40 @@ __device__ __noinline__ void ray_walk_beams(const MapGeom& geom, const ScanDevic
     *cell_steps_p += cell_steps;
 }
 
-// Fused copy + write-back of one clone (see k_ray_update_packed): reads the root slot's tiles, adds the
-// window, writes the clone's own slot, clears what the slot's previous tenant had informed elsewhere,
-// applies the parked exact-path hits, commits extents and announces that the root has been read.
-// Kept out of line: inlined, its live ranges push the ray walk's loop off its tight form.
-__device__ __noinline__ void ray_fused_writeback(const MapGeom& geom, int32_t slot, int32_t root, uint32_t* __restrict__ cells,
-                                                 SlotMeta* __restrict__ meta, uint32_t* __restrict__ bands_all,
-                                                 size_t cells_per_grid, const uint32_t* s_win, const int2* s_row, int* s_blo,
-                                                 int* s_bhi, int* s_ext, const uint32_t* s_nspill_p, const uint32_t* my_spill,
-                                                 int wy0, int wh, int band0, uint32_t* __restrict__ done, StepCounters* counters,
-                                                 bool* saturated_p, uint32_t* moved_p) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
-    const int gw = (int)geom.gw;
-    const uint32_t n_bands_slot = bands_per_slot(geom);
-    uint32_t* grid = cells + (size_t)slot * cells_per_grid;
-    uint32_t* bands = bands_all + (size_t)slot * n_bands_slot;
-    bool saturated = false;
-    uint32_t moved = 0;
-#ifdef SLAMRS_RAY_TRACE
-    long long t_prev = clock64();
-#endif
-    const uint4* win4 = reinterpret_cast<const uint4*>(s_win);
-    auto unpack = [](uint32_t packed16) { return (packed16 & PK_FREE_MASK) | ((packed16 >> PK_FREE_BITS) << 16); };
-    auto merge_group = [&](uint4& va, uint4& vb, const uint4& d) {
-        const uint32_t high_any = (va.x | va.y | va.z | va.w | vb.x | vb.y | vb.z | vb.w) & 0x80008000u;
-        if (high_any == 0u) {
-            va.x += unpack(d.x & 0xffffu); va.y += unpack(d.x >> 16);
-            va.z += unpack(d.y & 0xffffu); va.w += unpack(d.y >> 16);
-            vb.x += unpack(d.z & 0xffffu); vb.y += unpack(d.z >> 16);
-            vb.z += unpack(d.w & 0xffffu); vb.w += unpack(d.w >> 16);
-        } else {
-            va.x = cell_sat_add(va.x, unpack(d.x & 0xffffu), &saturated); va.y = cell_sat_add(va.y, unpack(d.x >> 16), &saturated);
-            va.z = cell_sat_add(va.z, unpack(d.y & 0xffffu), &saturated); va.w = cell_sat_add(va.w, unpack(d.y >> 16), &saturated);
-            vb.x = cell_sat_add(vb.x, unpack(d.z & 0xffffu), &saturated); vb.y = cell_sat_add(vb.y, unpack(d.z >> 16), &saturated);
-            vb.z = cell_sat_add(vb.z, unpack(d.w & 0xffffu), &saturated); vb.w = cell_sat_add(vb.w, unpack(d.w >> 16), &saturated);
-        }
-    };
-    // ---- fused copy + write-back (whole-grid tiled slots: logical cell = physical cell).
-    // Pre-pass: per band of the window the columns that really received hits. A lane scans one window row,
-    // a warp four bands at a time; the eight lanes of a band combine their ranges with shuffles.
-    {
-        const int rr = lane & 7, bq = lane >> 3;
-        int wxmin = 0x7fffffff, wymin = 0x7fffffff, wxmax = -1, wymax = -1;
-        const int n_wbands = (wy0 + wh - 1) / BAND_ROWS - band0 + 1;
-        for (int q = warp; 4 * q < n_wbands; q += n_warps) {
-            const int lb = 4 * q + bq;
-            const int y = (band0 + lb) * BAND_ROWS + rr, ly = y - wy0;
-            int first = 0x7fffffff, last = -1, rx0 = 0;
-            int2 row = make_int2(0, 0);
-            if (lb < n_wbands && (unsigned)ly < (unsigned)wh) { row = s_row[ly]; rx0 = row.y & 0xffff; }
-            const int groups = row.y >> 19;
-            for (int g = 0; g < 34; ++g) {                 // (a window row is at most 34 groups wide)
-                if (__all_sync(0xffffffffu, g >= groups)) break;
-                if (g < groups) {
-                    const uint4 d = win4[(row.x >> 3) + g];
-                    if ((d.x | d.y | d.z | d.w) != 0u) { first = min(first, g); last = g; }
-                }
-            }
-            int xlo = last >= 0 ? rx0 + 8 * first : 0x7fffffff, xhi = last >= 0 ? rx0 + 8 * last + 7 : -1;
-            const int ylo = last >= 0 ? y : 0x7fffffff, yhi = last >= 0 ? y : -1;
-            wymin = min(wymin, ylo); wymax = max(wymax, yhi);
-#pragma unroll
-            for (int o = 1; o < 8; o <<= 1) {
-                xlo = min(xlo, __shfl_xor_sync(0xffffffffu, xlo, o));
-                xhi = max(xhi, __shfl_xor_sync(0xffffffffu, xhi, o));
-            }
-            wxmin = min(wxmin, xlo); wxmax = max(wxmax, xhi);
-            if (rr == 0 && xhi >= xlo && (unsigned)lb < (unsigned)RAY_MAX_BANDS) { atomicMin(&s_blo[lb], xlo); atomicMax(&s_bhi[lb], xhi); }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            wxmin = min(wxmin, __shfl_xor_sync(0xffffffffu, wxmin, o)); wxmax = max(wxmax, __shfl_xor_sync(0xffffffffu, wxmax, o));
-            wymin = min(wymin, __shfl_xor_sync(0xffffffffu, wymin, o)); wymax = max(wymax, __shfl_xor_sync(0xffffffffu, wymax, o));
-        }
-        if (lane == 0) ext_add(s_ext, wxmin, wymin, wxmax, wymax);
+// Adds one 8-cell group of the packed window (d: eight 16-bit cells) to the grid's eight counters (va, vb). The
+// window value is unpacked without a branch; only a grid counter at or above 2^15 (which one scan's increment could
+// saturate) takes the saturating form.
+__device__ __forceinline__ uint32_t unpack_window_cell(uint32_t packed16) {
+    return (packed16 & PK_FREE_MASK) | ((packed16 >> PK_FREE_BITS) << 16);
+}
+__device__ __forceinline__ void merge_window_group(uint4& va, uint4& vb, const uint4& d, bool* saturated) {
+    const uint32_t high_any = (va.x | va.y | va.z | va.w | vb.x | vb.y | vb.z | vb.w) & 0x80008000u;
+    if (high_any == 0u) {
+        va.x += unpack_window_cell(d.x & 0xffffu); va.y += unpack_window_cell(d.x >> 16);
+        va.z += unpack_window_cell(d.y & 0xffffu); va.w += unpack_window_cell(d.y >> 16);
+        vb.x += unpack_window_cell(d.z & 0xffffu); vb.y += unpack_window_cell(d.z >> 16);
+        vb.z += unpack_window_cell(d.w & 0xffffu); vb.w += unpack_window_cell(d.w >> 16);
+    } else {
+        va.x = cell_sat_add(va.x, unpack_window_cell(d.x & 0xffffu), saturated); va.y = cell_sat_add(va.y, unpack_window_cell(d.x >> 16), saturated);
+        va.z = cell_sat_add(va.z, unpack_window_cell(d.y & 0xffffu), saturated); va.w = cell_sat_add(va.w, unpack_window_cell(d.y >> 16), saturated);
+        vb.x = cell_sat_add(vb.x, unpack_window_cell(d.z & 0xffffu), saturated); vb.y = cell_sat_add(vb.y, unpack_window_cell(d.z >> 16), saturated);
+        vb.z = cell_sat_add(vb.z, unpack_window_cell(d.w & 0xffffu), saturated); vb.w = cell_sat_add(vb.w, unpack_window_cell(d.w >> 16), saturated);
     }
-    __syncthreads();
-    RAY_STAMP(8);
-    const uint32_t* src = cells + (size_t)root * cells_per_grid;
-    const uint32_t* src_bands = bands_all + (size_t)root * n_bands_slot;
-    const SlotMeta sm = meta[root], om = meta[slot];
-    // bands to visit: the source's rows, the rows the slot's previous tenant had informed, the touched window rows
-    int by0 = 0x7fffffff, by1 = -1;
-    if (sm.x1 > sm.x0 && sm.y1 > sm.y0) { by0 = min(by0, sm.y0 / BAND_ROWS); by1 = max(by1, (sm.y1 - 1) / BAND_ROWS); }
-    if (om.x1 > om.x0 && om.y1 > om.y0) { by0 = min(by0, om.y0 / BAND_ROWS); by1 = max(by1, (om.y1 - 1) / BAND_ROWS); }
-    if (s_ext[3] >= s_ext[1] && s_ext[2] >= s_ext[0]) { by0 = min(by0, s_ext[1] / BAND_ROWS); by1 = max(by1, s_ext[3] / BAND_ROWS); }
-    const uint32_t tpr = geom.tiles_per_row;
-    constexpr int FUSE_DEPTH = 4;              // tiles in flight per warp
-    const int rr = lane >> 2, uu = lane & 3;   // this lane's row of the band and 32-byte unit of the tile row
-    // bands go to the warps round-robin: every warp gets narrow (top, bottom) and wide (middle) bands alike
-    for (int bnd = by0 + warp; bnd <= by1; bnd += n_warps) {
-        const uint32_t es = src_bands[bnd], eo = bands[bnd];
-        const int lb = bnd - band0;
-        const bool touched = (unsigned)lb < (unsigned)RAY_MAX_BANDS && s_bhi[lb] >= s_blo[lb];
-        uint32_t n0 = es ? (es & 0xffffu) : 0xffffu, n1 = es ? (es >> 16) : 0u;     // new extent: source + touched
-        if (touched) { n0 = min(n0, (uint32_t)s_blo[lb] & ~7u); n1 = max(n1, min(geom.gw, ((uint32_t)s_bhi[lb] + 8u) & ~7u)); }
-        uint32_t u0 = n0, u1 = n1;                                                   // to write: new + old (to clear)
-        if (eo) { u0 = min(u0, eo & 0xffffu); u1 = max(u1, eo >> 16); }
-        __syncwarp();                                   // every lane has read the old entry
-        if (lane == 0) bands[bnd] = n1 > n0 ? (n0 | (n1 << 16)) : 0u;
-        if (u1 <= u0) continue;
-        const int t_lo = (int)(u0 / TILE_COLS), t_hi = (int)((u1 + TILE_COLS - 1u) / TILE_COLS);
-        // this lane's window row, if the band has one
-        const int y = bnd * BAND_ROWS + rr, ly = y - wy0;
-        int wfirst = 0, wx0 = 0, ww = 0;
-        if (touched && (unsigned)ly < (unsigned)wh) { const int2 row = s_row[ly]; wfirst = row.x; wx0 = row.y & 0xffff; ww = row.y >> 16; }
-        const uint32_t sx0 = es & 0xffffu, sx1 = es >> 16;                           // (0, 0 when the source has nothing here)
-        const size_t band_off = (size_t)bnd * tpr * TILE_CELLS + 8u * (uint32_t)lane;
-        for (int t0 = t_lo; t0 < t_hi; t0 += FUSE_DEPTH) {
-            uint4 va[FUSE_DEPTH], vb[FUSE_DEPTH];
-#pragma unroll
-            for (int k = 0; k < FUSE_DEPTH; ++k) {
-                const int t = t0 + k;
-                const uint32_t x = (uint32_t)t * TILE_COLS + 8u * (uint32_t)uu;
-                va[k] = make_uint4(0u, 0u, 0u, 0u); vb[k] = va[k];
-                if (t < t_hi && x >= sx0 && x < sx1) {
-                    const V8 s8 = ld_stream_v8(reinterpret_cast<const V8*>(src + band_off + (size_t)t * TILE_CELLS));
-                    va[k] = s8.a; vb[k] = s8.b;
-                    moved++;
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < FUSE_DEPTH; ++k) {
-                const int t = t0 + k;
-                if (t >= t_hi) break;
-                const int lx = t * (int)TILE_COLS + 8 * uu - wx0;
-                if ((unsigned)lx < (unsigned)ww) {
-                    const uint4 d = win4[(wfirst + lx) >> 3];
-                    if ((d.x | d.y | d.z | d.w) != 0u) merge_group(va[k], vb[k], d);
-                }
-                V8 o8; o8.a = va[k]; o8.b = vb[k];
-                st_stream_v8(reinterpret_cast<V8*>(grid + band_off + (size_t)t * TILE_CELLS), o8);
-                moved++;
-            }
-        }
-    }
-    RAY_STAMP(9);
-    __syncthreads();
-    RAY_STAMP(10);
-    {   // the parked exact-path hits, now that the slot holds its cells
-        const uint32_t ns = *s_nspill_p;
-        if (ns > RAY_SPILL_CAP && threadIdx.x == 0) atomicAdd(&counters->fuse_overflow, 1ull);
-        for (uint32_t k = threadIdx.x; k < min(ns, RAY_SPILL_CAP); k += blockDim.x) {
-            const uint32_t e = my_spill[k];
-            global_cell_add(&grid[phys_index(geom, e & 0x7fffu, (e >> 15) & 0x7fffu)],
-                            (e & 0x40000000u) ? CELL_OCC_INC : CELL_FREE_INC, &saturated);
-        }
-    }
-    if (threadIdx.x == 0) {
-        // the slot now holds the source's extent plus what this scan touched
-        SlotMeta nm = sm;
-        if (!(nm.x1 > nm.x0 && nm.y1 > nm.y0)) { nm.x0 = nm.y0 = nm.x1 = nm.y1 = 0; }
-        meta[slot] = nm;
-        ext_commit(s_ext, &meta[slot], gw);
-        __threadfence();
-        atomicAdd(&done[root], 1u);        // the root has been read: its owner may write it
-    }
-    if (saturated) *saturated_p = true;
-    *moved_p += moved;
 }
 
-// Work distribution. The kernel is launched with as many CTAs as are resident at once (two per SM at a
-// 6 m / 5 cm window) and every CTA pops work items from an atomic counter until the list is empty: the
-// list holds the few hundred particles that survive this step's resampling, not the whole population.
+// Work distribution of both packed kernels. A kernel is launched with as many CTAs as are resident at once and
+// every CTA pops work items from an atomic counter until the list is empty: the list holds the few hundred
+// particles that survive this step's resampling, not the whole population.
 //
-// Fused copies (deferred copies, whole-grid tiled slots). A surviving particle whose grid is still an
-// alias of its source's slot ("clone") would first need its own copy of the source's cells (k_copy_boxed)
-// and then read them again to add the scan. Here its CTA does both in one pass: it reads the ROOT slot's
-// tiles, adds the window, writes its OWN slot (and clears what the slot's previous tenant had informed
-// outside the new extent). The copy kernels and their pass over the grids disappear from the step.
-// The hazard is the root's owner integrating the scan in place while a clone still reads the root:
-// k_resample_indices lists the clones first and the particles that own their slot after them, counts the clones per root (readers[]), every clone announces when it has read its root
-// (done[]), and an owner waits for its readers before it writes. Items are popped in list order by CTAs
-// that are all resident, so every reader an owner waits for is already running: no deadlock.
-struct RayJob {      // what a CTA works on, resolved once per item
-    uint32_t particle;
-    int32_t slot, root;   // root != slot: fused copy
-};
-
+// k_ray_update_packed: a whole particle per work item (two CTAs per SM at a 6 m / 5 cm window), for row-major and
+// windowed slots. Its items come from the survivor list alone; the particle's slot is its own, so the window is
+// written back into it in place.
 __global__ void __maxnreg__(80)   // 2 CTAs of 384 threads per SM; blocks have at most RAY_MAX_THREADS threads
 k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ results, uint32_t first_particle,
-                    const uint32_t* __restrict__ alive_list, const RayItem* __restrict__ clones, const RayItem* __restrict__ owners,
-                    const uint32_t* __restrict__ readers, uint32_t* __restrict__ done, uint32_t* __restrict__ spill_scratch,
-                    const int32_t* __restrict__ slot_of, uint32_t* __restrict__ cells, SlotMeta* __restrict__ meta,
-                    uint32_t* __restrict__ bands_all, size_t cells_per_grid, int radius, int reach, StepCounters* counters,
-                    uint32_t n_local) {
+                    const uint32_t* __restrict__ alive_list, const int32_t* __restrict__ slot_of, uint32_t* __restrict__ cells,
+                    SlotMeta* __restrict__ meta, uint32_t* __restrict__ bands_all, size_t cells_per_grid, int radius, int reach,
+                    StepCounters* counters) {
     extern __shared__ __align__(16) uint32_t s_win[];   // two 16-bit cells per word
-    __shared__ uint32_t s_nspill;
     __shared__ int s_blo[RAY_MAX_BANDS], s_bhi[RAY_MAX_BANDS];
     __shared__ int2 s_row[RAY_MAX_ROWS + 1];            // .x = first window cell of the row, .y = x0 | width << 16
     __shared__ uint32_t s_rowb[RAY_MAX_ROWS];           // shared byte address of column x = 0 of the row
@@ -849,7 +730,6 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
     bool saturated = false;
     uint32_t spilled = 0;
     uint32_t cell_steps = 0;   // iterator steps of this thread's rays (SURVEY.md 8(d): C_p, the unit of the ray update's bytes)
-    uint32_t moved = 0;        // 32-byte units read + written by the fused copies (this thread)
 
 #ifdef SLAMRS_RAY_TRACE
     long long t_prev = clock64();
@@ -861,18 +741,10 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
         __syncthreads();
         const unsigned long long item = s_next;
         if (item >= n_items) break;
-        RayJob job;
-        if (clones) {   // clones first: an owner is popped only after every clone that reads its slot
-            const RayItem it = ray_item_at(clones, owners, n_local, counters, item);
-            job.particle = it.particle; job.slot = it.slot; job.root = it.root;
-        }
-        else { job.particle = alive_list[item]; job.slot = slot_of[job.particle]; job.root = job.slot; }
-        const bool fused = job.root != job.slot;
-        const uint32_t p = job.particle;
-        uint32_t* grid = cells + (size_t)job.slot * cells_per_grid;
+        const uint32_t p = alive_list[item];
+        const int32_t slot = slot_of[p];
+        uint32_t* grid = cells + (size_t)slot * cells_per_grid;
         ext_init(s_ext);
-        if (threadIdx.x == 0) s_nspill = 0u;
-        uint32_t* my_spill = spill_scratch + (size_t)blockIdx.x * RAY_SPILL_CAP;
         const ParticleResult r = results[first_particle + p];
         const float px = r.x, py = r.y, ptheta = r.theta;
 
@@ -881,24 +753,22 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
         const long long lcx = f32_as_isize(floorf(sx)), lcy = f32_as_isize(floorf(sy));
         // every ray starts in the same cell; outside the grid nothing is emitted (ray.rs:88-92)
         const bool start_inside = !(lcx < 0 || lcx >= (long long)geom.gw || lcy < 0 || lcy >= (long long)geom.gh);
-        if (!start_inside && !fused) continue;
-        // (a clone whose pose left the grid integrates nothing but still gets its own cells: window of radius 0 at cell 0)
-        const int cx0 = start_inside ? (int)lcx : 0, cy0 = start_inside ? (int)lcy : 0;
-        const int rad = start_inside ? radius : 0;
-        if (window_would_overflow(geom, &meta[job.slot], cx0, cy0, reach)) {   // windowed slots only (never fused)
+        if (!start_inside) continue;
+        const int cx0 = (int)lcx, cy0 = (int)lcy;
+        if (window_would_overflow(geom, &meta[slot], cx0, cy0, reach)) {   // windowed slots only
             if (threadIdx.x == 0) atomicAdd(&counters->window_overflow, 1ull);
             continue;   // the grid is left as it was; the step reports SLAMRS_E_WINDOW
         }
-        uint32_t* bands = bands_all + (size_t)job.slot * n_bands_slot;
+        uint32_t* bands = bands_all + (size_t)slot * n_bands_slot;
         band_init(s_blo, s_bhi);
 
         // ---- row table of the disc window (x ranges aligned to 8 cells = one 128-bit group)
-        const int wy0 = max(0, cy0 - rad), wy1 = min(gh, cy0 + rad + 1);
+        const int wy0 = max(0, cy0 - radius), wy1 = min(gh, cy0 + radius + 1);
         const int band0 = wy0 / BAND_ROWS;
         const int wh = wy1 - wy0;
         for (int ly = threadIdx.x; ly < wh; ly += blockDim.x) {
             const int dy = wy0 + ly - cy0;
-            const int hw = isqrt_small(rad * rad - dy * dy);
+            const int hw = isqrt_small(radius * radius - dy * dy);
             const int x0 = max(0, cx0 - hw) & ~7;
             const int x1 = min(gw, (min(gw, cx0 + hw + 1) + 7) & ~7);
             s_row[ly].y = x0 | ((x1 - x0) << 16);
@@ -933,61 +803,18 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
         __syncthreads();
 
         RAY_STAMP(1);
-        if (start_inside)
-            ray_walk_beams(geom, scan, px, py, ptheta, sx, sy, cx0, cy0, rad, wy0, wh, band0, s_win, s_row, s_rowb, s_blo, s_bhi, s_ext,
-                           grid, bands, fused, &s_nspill, my_spill, &saturated, &spilled, &cell_steps);
+        const bool disc_in_grid = cx0 - radius >= 0 && cx0 + radius < gw && cy0 - radius >= 0 && cy0 + radius < gh;
+        ray_walk_packed<false>(geom, scan, scan.order, scan.n_beams, px, py, ptheta, sx, sy, cx0, cy0, radius, disc_in_grid, wy0,
+                               wh, band0, s_win, s_row, s_rowb, s_blo, s_bhi, s_ext, grid, bands, nullptr, nullptr, &saturated,
+                               &spilled, &cell_steps);
         __syncthreads();
         RAY_STAMP(2);
 
-        const uint4* win4 = reinterpret_cast<const uint4*>(s_win);
-        auto unpack = [](uint32_t packed16) { return (packed16 & PK_FREE_MASK) | ((packed16 >> PK_FREE_BITS) << 16); };
-        auto merge_group = [&](uint4& va, uint4& vb, const uint4& d) {
-            const uint32_t high_any = (va.x | va.y | va.z | va.w | vb.x | vb.y | vb.z | vb.w) & 0x80008000u;
-            if (high_any == 0u) {
-                va.x += unpack(d.x & 0xffffu); va.y += unpack(d.x >> 16);
-                va.z += unpack(d.y & 0xffffu); va.w += unpack(d.y >> 16);
-                vb.x += unpack(d.z & 0xffffu); vb.y += unpack(d.z >> 16);
-                vb.z += unpack(d.w & 0xffffu); vb.w += unpack(d.w >> 16);
-            } else {
-                va.x = cell_sat_add(va.x, unpack(d.x & 0xffffu), &saturated); va.y = cell_sat_add(va.y, unpack(d.x >> 16), &saturated);
-                va.z = cell_sat_add(va.z, unpack(d.y & 0xffffu), &saturated); va.w = cell_sat_add(va.w, unpack(d.y >> 16), &saturated);
-                vb.x = cell_sat_add(vb.x, unpack(d.z & 0xffffu), &saturated); vb.y = cell_sat_add(vb.y, unpack(d.z >> 16), &saturated);
-                vb.z = cell_sat_add(vb.z, unpack(d.w & 0xffffu), &saturated); vb.w = cell_sat_add(vb.w, unpack(d.w >> 16), &saturated);
-            }
-        };
-
-        if (fused) {
-            ray_fused_writeback(geom, job.slot, job.root, cells, meta, bands_all, cells_per_grid, s_win, s_row, s_blo, s_bhi, s_ext,
-                                &s_nspill, my_spill, wy0, wh, band0, done, counters, &saturated, &moved);
-            RAY_STAMP(3);
-#ifdef SLAMRS_RAY_TRACE
-            if (threadIdx.x == 0) atomicAdd(&g_ray_trace_items[0], 1ull);
-#endif
-            continue;
-        }
-
-        // ---- in-place write-back. The owner of a slot that clones read in this step waits for them first.
-        if (readers != nullptr) {
-            if (threadIdx.x == 0) {
-                const uint32_t want = readers[job.slot];
-                if (want != 0u) {
-                    uint32_t seen;
-                    for (;;) {
-                        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(done + job.slot) : "memory");
-                        if (seen >= want) break;
-                        __nanosleep(100);
-                    }
-                }
-            }
-            __syncthreads();
-            RAY_STAMP(4);
-        }
-        // A window row is at most 34 groups of 8 cells (one 128-bit shared load each); a
+        // ---- in-place write-back. A window row is at most 34 groups of 8 cells (one 128-bit shared load each); a
         // non-empty group is two 128-bit global read-modify-writes. Main pass: one warp per row, lane g
         // takes group g < 32, RAY_WB_ROWS rows in flight per warp. Tail pass: the (at most two) groups
-        // beyond the 32nd of each row, one thread per row. One code path per group: the packed window
-        // value is unpacked without a branch; only a grid counter at or above 2^15 (which one scan's
-        // increment could saturate) takes the saturating form.
+        // beyond the 32nd of each row, one thread per row.
+        const uint4* win4 = reinterpret_cast<const uint4*>(s_win);
         constexpr int RAY_WB_ROWS = 2;   // (measured on a configs[4] shard: 2 -> 0.770 ms per step, 4 -> 0.800: four rows spilled)
         int exmin = 0x7fffffff, eymin = 0x7fffffff, exmax = -1, eymax = -1;   // this thread's touched extent
         for (int ly0 = warp; ly0 < wh; ly0 += n_warps * RAY_WB_ROWS) {
@@ -1027,7 +854,7 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
 #pragma unroll
             for (int j = 0; j < RAY_WB_ROWS; ++j) {
                 if (nz[j]) {
-                    merge_group(va[j], vb[j], d[j]);
+                    merge_window_group(va[j], vb[j], d[j], &saturated);
                     st_group_v8(gp[j], va[j], vb[j]);
                 }
             }
@@ -1043,7 +870,7 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
                 band_add(s_blo, s_bhi, band0, wy0 + ly, gx0, gx0 + 7);
                 uint4* gpt = reinterpret_cast<uint4*>(grid + phys_index(geom, (uint32_t)gx0, (uint32_t)(wy0 + ly)));
                 uint4 ta = gpt[0], tb = gpt[1];
-                merge_group(ta, tb, dd);
+                merge_window_group(ta, tb, dd, &saturated);
                 gpt[0] = ta;
                 gpt[1] = tb;
             }
@@ -1051,7 +878,7 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
         ext_add(s_ext, exmin, eymin, exmax, eymax);
         __syncthreads();
         band_commit(s_blo, s_bhi, band0, bands, geom);
-        if (threadIdx.x == 0) ext_commit(s_ext, &meta[job.slot], (int)geom.gw);
+        if (threadIdx.x == 0) ext_commit(s_ext, &meta[slot], (int)geom.gw);
         RAY_STAMP(5);
 #ifdef SLAMRS_RAY_TRACE
         if (threadIdx.x == 0) atomicAdd(&g_ray_trace_items[1], 1ull);
@@ -1060,12 +887,8 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
     if (saturated) atomicAdd(&counters->saturated, 1ull);
     if (spilled) atomicAdd(&counters->spilled, (unsigned long long)spilled);
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { cell_steps += __shfl_down_sync(0xffffffffu, cell_steps, o); moved += __shfl_down_sync(0xffffffffu, moved, o); }
+    for (int o = 16; o > 0; o >>= 1) cell_steps += __shfl_down_sync(0xffffffffu, cell_steps, o);
     if ((threadIdx.x & 31) == 0 && cell_steps) atomicAdd(&counters->ray_cell_steps, (unsigned long long)cell_steps);
-    if ((threadIdx.x & 31) == 0 && moved) {
-        atomicAdd(&counters->copy_bytes, (unsigned long long)moved * 32ull);
-        atomicAdd(&counters->ray_copy_bytes, (unsigned long long)moved * 32ull);
-    }
 }
 
 // =============================================================================== k_ray_update_half
@@ -1085,9 +908,17 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
 // The lower half is listed right before the upper half, so the upper CTA only ever waits for a CTA that
 // is already running.
 //
-// One write-back path for clones and owners: read the ROOT slot's tiles (a clone's source; an owner's own
-// slot), add the window, write the particle's OWN slot -- see k_ray_update_packed for the clone / owner
-// protocol (readers / done), which is unchanged except that a clone counts as two readers.
+// Fused copies (deferred copies). A surviving particle whose grid is still an alias of its source's slot
+// ("clone") would first need its own copy of the source's cells (k_copy_boxed) and then read them again to
+// add the scan. Here its CTAs do both in one pass: one write-back path for clones and owners reads the ROOT
+// slot's tiles (a clone's source; an owner's own slot), adds the window and writes the particle's OWN slot
+// (and clears what the slot's previous tenant had informed outside the new extent). The copy kernels and
+// their pass over the grids disappear from the step. The hazard is the root's owner integrating the scan in
+// place while a clone still reads the root: k_resample_indices lists the clones first and the particles that
+// own their slot after them and counts the readers of each root (readers[]; each half of a clone is one),
+// every clone half announces when it has read its root (done[]), and an owner waits for its readers before it
+// writes. Items are popped in list order by CTAs that are all resident, so every reader an owner waits for is
+// already running: no deadlock.
 constexpr int HALF_MAX_ROWS = RAY_MAX_RADIUS + 1;
 constexpr int HALF_MAX_BANDS = HALF_MAX_ROWS / BAND_ROWS + 2;
 constexpr uint32_t HALF_XCHG_GROUPS = 36;
@@ -1117,259 +948,6 @@ __host__ __device__ inline int ray_window_cells_upper_bound_half(int radius) {
     return worst;
 }
 
-// The walk of this half's beams (s_beam: indices into the scan) into the half-disc window. Same arithmetic as
-// ray_walk_beams; hits that bypass the window are always parked (the slot receives its cells at write-back).
-__device__ __noinline__ void ray_walk_half(const MapGeom& geom, const ScanDevice& scan, const uint16_t* s_beam, uint32_t n_mine,
-                                           float px, float py, float ptheta, float sx, float sy, int cx0, int cy0, int rad,
-                                           bool upper, int wy0, int wh, int band0, uint32_t* s_win, const int2* s_row,
-                                           const uint32_t* s_rowb, int* s_blo, int* s_bhi, int* s_ext, uint32_t* s_nspill_p,
-                                           uint32_t* __restrict__ my_spill, uint32_t* spilled_p, uint32_t* cell_steps_p) {
-    const int gw = (int)geom.gw, gh = (int)geom.gh;
-    const uint32_t win_base = (uint32_t)__cvta_generic_to_shared(s_win);
-    uint32_t spilled = 0, cell_steps = 0;
-    ZeroLengthHits zero_length;
-    auto exact_add = [&](int x, int y, uint32_t inc) {
-        const uint32_t k = atomicAdd(s_nspill_p, 1u);
-        if (k < RAY_SPILL_CAP) my_spill[k] = (uint32_t)x | ((uint32_t)y << 15) | (inc == CELL_OCC_INC ? 0x40000000u : 0u);
-    };
-    // the window holds every in-grid cell within `rad` of the start in this half's rows
-    const bool disc_in_grid = cx0 - rad >= 0 && cx0 + rad < gw && (upper ? cy0 + rad < gh : cy0 - rad >= 0);
-    uint32_t rowb_base = (uint32_t)__cvta_generic_to_shared(s_rowb);
-    asm volatile("" : "+r"(rowb_base));
-    auto load_rowb = [&](int row) {
-        uint32_t v;
-        asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(rowb_base + 4u * (uint32_t)row) : "memory");
-        return v;
-    };
-    for (uint32_t t = threadIdx.x; t < n_mine; t += blockDim.x) {
-        const uint32_t b = s_beam[t];
-        const float dist = scan.dist[b];
-        float ex, ey;
-        beam_endpoint(px, py, ptheta, scan.angle[b], dist, &ex, &ey);
-        const float x1 = world_to_grid(ex, geom.pos_x, geom.res);
-        const float y1 = world_to_grid(ey, geom.pos_y, geom.res);
-        const RayClassifier cls = make_ray_classifier(__fdiv_rn(dist, geom.res), scan.valid[b] != 0);
-
-        // GridRayIterator::new (ray.rs:21-77) -- identical arithmetic to ray_walk_acc
-        const float delta_x = fabsf(__fsub_rn(x1, sx)), delta_y = fabsf(__fsub_rn(y1, sy));
-        const float fx0 = floorf(sx), fy0 = floorf(sy);
-        unsigned long long n = 1ull + 2ull;   // additional_steps = 2 (map.rs:97)
-        unsigned long long ax = 0ull, ay = 0ull;   // |endpoint cell - start cell| per axis
-        int x_inc, y_inc;
-        float error;
-        if (delta_x == 0.0f) {
-            x_inc = 0;
-            error = __int_as_float(0x7f800000);
-        } else if (x1 > sx) {
-            x_inc = 1;
-            ax = (unsigned long long)f32_as_isize(__fsub_rn(floorf(x1), (float)cx0));
-            error = __fmul_rn(__fsub_rn(__fadd_rn(fx0, 1.0f), sx), delta_y);
-        } else {
-            x_inc = -1;
-            ax = (unsigned long long)(long long)cx0 - (unsigned long long)f32_as_isize(floorf(x1));
-            error = __fmul_rn(__fsub_rn(sx, fx0), delta_y);
-        }
-        if (delta_y == 0.0f) {
-            y_inc = 0;
-            error = __fsub_rn(error, __int_as_float(0x7f800000));
-        } else if (y1 > sy) {
-            y_inc = 1;
-            ay = (unsigned long long)f32_as_isize(floorf(y1)) - (unsigned long long)(long long)cy0;
-            error = __fsub_rn(error, __fmul_rn(__fsub_rn(__fadd_rn(fy0, 1.0f), sy), delta_x));
-        } else {
-            y_inc = -1;
-            ay = (unsigned long long)(long long)cy0 - (unsigned long long)f32_as_isize(floorf(y1));
-            error = __fsub_rn(error, __fmul_rn(__fsub_rn(sy, fy0), delta_x));
-        }
-        n += ax + ay;   // wrapping isize arithmetic, then `as usize`
-        const unsigned long long cap = (unsigned long long)geom.gw + geom.gh + 8ull;
-        int remaining = (int)(n < cap ? n : cap);
-        cell_steps += (uint32_t)remaining;
-
-        const float x_step = (float)x_inc, y_step = (float)y_inc;
-        float cxf = __fadd_rn((float)cx0, 0.5f), cyf = __fadd_rn((float)cy0, 0.5f);
-        float dxs = __fsub_rn(sx, cxf), dys = __fsub_rn(sy, cyf);
-        float dx2 = __fmul_rn(dxs, dxs), dy2 = __fmul_rn(dys, dys);
-        if (delta_x == 0.0f && delta_y == 0.0f) {   // see ZeroLengthHits
-            zero_length.tally(cls, __fadd_rn(dx2, dy2));
-            continue;
-        }
-
-        bool fast = false;
-        if (disc_in_grid && ax < 4096ull && ay < 4096ull) {
-            const int cxa = (int)ax + 2, cya = (int)ay + 2;
-            fast = cxa * cxa + cya * cya <= rad * rad;
-        }
-        if (fast) {
-            uint32_t x2 = 2u * (uint32_t)cx0;         // twice the current column
-            const uint32_t x_inc2 = (uint32_t)(2 * x_inc);
-            int ly = cy0 - wy0;
-            uint32_t rb = load_rowb(ly);
-            // The first cells of a walk are free whatever its direction: the cell reached after k steps is k cells from
-            // the start cell in the Manhattan sense, the start point lies inside the start cell, so both offsets to the
-            // cell centre are at most (cells + 0.5) and acc <= (k + 0.5)^2 + 0.25 < K^2 for k < K; with K^2 <= 0.999 x
-            // free_below (the margin dwarfs the f32 rounding of acc) those K cells pass `acc < free_below` without
-            // evaluating it. They take a loop without the distance arithmetic; the distance state is then rebuilt from
-            // the cell position -- cxf and cyf only ever held (integer + 0.5) exactly, so the rebuilt values are the
-            // accumulated ones bit for bit -- and the free run continues with the test.
-            {
-                const float kf = floorf(__fsqrt_rn(__fmul_rn(cls.free_below, 0.999f)));
-                int safe = (kf >= 1.0f && kf < 1.0e6f) ? (int)kf : 0;      // (NaN and tiny thresholds: none)
-                safe = min(safe, remaining);
-                remaining -= safe;
-                for (; safe > 0; --safe) {
-                    const uint32_t c2 = rb + x2;
-                    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(c2 & ~3u), "r"((c2 & 2u) ? 0x10000u : 1u) : "memory");
-                    if (error > 0.0f) {
-                        error = __fsub_rn(error, delta_x);
-                        ly += y_inc;
-                        rb = load_rowb(ly);
-                    } else {
-                        error = __fadd_rn(error, delta_y);
-                        x2 += x_inc2;
-                    }
-                }
-                cxf = __fadd_rn((float)(x2 >> 1), 0.5f);
-                cyf = __fadd_rn((float)(wy0 + ly), 0.5f);
-                dxs = __fsub_rn(sx, cxf); dys = __fsub_rn(sy, cyf);
-                dx2 = __fmul_rn(dxs, dxs); dy2 = __fmul_rn(dys, dys);
-            }
-            while (remaining > 0) {                    // free run
-                const float acc = __fadd_rn(dx2, dy2);
-                if (!(acc < cls.free_below)) break;
-                const uint32_t c2 = rb + x2;           // shared byte address of the 16-bit window cell
-                asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(c2 & ~3u), "r"((c2 & 2u) ? 0x10000u : 1u) : "memory");
-                if (error > 0.0f) {
-                    error = __fsub_rn(error, delta_x);
-                    cyf = __fadd_rn(cyf, y_step);
-                    dys = __fsub_rn(sy, cyf);
-                    dy2 = __fmul_rn(dys, dys);
-                    ly += y_inc;
-                    rb = load_rowb(ly);
-                } else {
-                    error = __fadd_rn(error, delta_y);
-                    cxf = __fadd_rn(cxf, x_step);
-                    dxs = __fsub_rn(sx, cxf);
-                    dx2 = __fmul_rn(dxs, dxs);
-                    x2 += x_inc2;
-                }
-                remaining -= 1;
-            }
-            if (cls.mid_inc != 0u) {                   // occupied run (hits only)
-                while (remaining > 0) {
-                    const float acc = __fadd_rn(dx2, dy2);
-                    if (acc > cls.prior_above) break;
-                    const uint32_t c2 = rb + x2;
-                    const uint32_t shift = ((c2 & 2u) << 3) + PK_FREE_BITS;
-                    uint32_t old;
-                    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(old) : "r"(c2 & ~3u) : "memory");
-                    bool done_here = false;
-                    for (;;) {
-                        if (((old >> shift) & PK_OCC_MAX) == PK_OCC_MAX) break;
-                        uint32_t seen;
-                        asm volatile("atom.shared.cas.b32 %0, [%1], %2, %3;"
-                                     : "=r"(seen) : "r"(c2 & ~3u), "r"(old), "r"(old + (1u << shift)) : "memory");
-                        if (seen == old) { done_here = true; break; }
-                        old = seen;
-                    }
-                    if (!done_here) {
-                        const int x = (int)(x2 >> 1), y = wy0 + ly;
-                        exact_add(x, y, CELL_OCC_INC);
-                        ext_add(s_ext, x, y, x, y);
-                        band_add(s_blo, s_bhi, band0, y, x, x);
-                        spilled++;
-                    }
-                    if (error > 0.0f) {
-                        error = __fsub_rn(error, delta_x);
-                        cyf = __fadd_rn(cyf, y_step);
-                        dys = __fsub_rn(sy, cyf);
-                        dy2 = __fmul_rn(dys, dys);
-                        ly += y_inc;
-                        rb = load_rowb(ly);
-                    } else {
-                        error = __fadd_rn(error, delta_y);
-                        cxf = __fadd_rn(cxf, x_step);
-                        dxs = __fsub_rn(sx, cxf);
-                        dx2 = __fmul_rn(dxs, dxs);
-                        x2 += x_inc2;
-                    }
-                    remaining -= 1;
-                }
-            }
-            continue;
-        }
-
-        // general walk: per-cell window and grid tests (rays that may leave the window or the grid)
-        int x = cx0, y = cy0;
-        int ly = y - wy0;
-        int2 row = s_row[ly];                      // the start cell is always inside the window
-        int lx = x - (row.y & 0xffff);
-        int row_w = row.y >> 16;
-        bool inside = true;
-        while (remaining > 0 && inside) {
-            const float acc = __fadd_rn(dx2, dy2);
-            const bool is_free = acc < cls.free_below;
-            const bool is_mid = !is_free && !(acc > cls.prior_above) && (cls.mid_inc != 0u);
-            if (is_free | is_mid) {
-                const bool in_win = (unsigned)lx < (unsigned)row_w;
-                const int cell = row.x + lx;
-                const uint32_t addr = win_base + ((uint32_t)(cell >> 1) << 2);
-                const uint32_t shift = (cell & 1) << 4;
-                if (is_free & in_win) {
-                    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(addr), "r"(1u << shift) : "memory");
-                } else {
-                    bool done_here = false;
-                    if (in_win) {
-                        uint32_t* wp = &s_win[cell >> 1];
-                        uint32_t old = *wp;
-                        for (;;) {
-                            if (((old >> (shift + PK_FREE_BITS)) & PK_OCC_MAX) == PK_OCC_MAX) break;
-                            const uint32_t seen = atomicCAS(wp, old, old + (1u << (shift + PK_FREE_BITS)));
-                            if (seen == old) { done_here = true; break; }
-                            old = seen;
-                        }
-                    }
-                    if (!done_here) {
-                        exact_add(x, y, is_free ? CELL_FREE_INC : CELL_OCC_INC);
-                        ext_add(s_ext, x, y, x, y);
-                        band_add(s_blo, s_bhi, band0, y, x, x);
-                        spilled++;
-                    }
-                }
-            }
-            if (error > 0.0f) {                    // GridRayIterator::next (ray.rs:96-104)
-                y += y_inc;
-                error = __fsub_rn(error, delta_x);
-                cyf = __fadd_rn(cyf, y_step);
-                dys = __fsub_rn(sy, cyf);
-                dy2 = __fmul_rn(dys, dys);
-                inside = (unsigned)y < (unsigned)gh;
-                ly += y_inc;
-                if ((unsigned)ly < (unsigned)wh) {
-                    row = s_row[ly];
-                    row_w = row.y >> 16;
-                    lx = x - (row.y & 0xffff);
-                } else {
-                    row_w = 0;
-                }
-            } else {
-                x += x_inc;
-                error = __fadd_rn(error, delta_y);
-                cxf = __fadd_rn(cxf, x_step);
-                dxs = __fsub_rn(sx, cxf);
-                dx2 = __fmul_rn(dxs, dxs);
-                inside = (unsigned)x < (unsigned)gw;
-                lx += x_inc;
-            }
-            remaining -= 1;
-        }
-        cell_steps -= (uint32_t)remaining;   // the walk ended at the grid border
-    }
-    spilled += zero_length.flush(cx0, cy0, exact_add, s_ext, s_blo, s_bhi, band0);
-    *spilled_p += spilled;
-    *cell_steps_p += cell_steps;
-}
-
 // write-back of one half item: root tiles + window -> own slot, for the rows this half owns
 __device__ __noinline__ void ray_half_writeback(const MapGeom& geom, const RayItem& it, bool upper, int cy0, bool walked,
                                                 uint32_t* __restrict__ cells, SlotMeta* __restrict__ meta,
@@ -1388,21 +966,6 @@ __device__ __noinline__ void ray_half_writeback(const MapGeom& geom, const RayIt
     bool saturated = false;
     uint32_t moved = 0;
     const uint4* win4 = reinterpret_cast<const uint4*>(s_win);
-    auto unpack = [](uint32_t packed16) { return (packed16 & PK_FREE_MASK) | ((packed16 >> PK_FREE_BITS) << 16); };
-    auto merge_group = [&](uint4& va, uint4& vb, const uint4& d) {
-        const uint32_t high_any = (va.x | va.y | va.z | va.w | vb.x | vb.y | vb.z | vb.w) & 0x80008000u;
-        if (high_any == 0u) {
-            va.x += unpack(d.x & 0xffffu); va.y += unpack(d.x >> 16);
-            va.z += unpack(d.y & 0xffffu); va.w += unpack(d.y >> 16);
-            vb.x += unpack(d.z & 0xffffu); vb.y += unpack(d.z >> 16);
-            vb.z += unpack(d.w & 0xffffu); vb.w += unpack(d.w >> 16);
-        } else {
-            va.x = cell_sat_add(va.x, unpack(d.x & 0xffffu), &saturated); va.y = cell_sat_add(va.y, unpack(d.x >> 16), &saturated);
-            va.z = cell_sat_add(va.z, unpack(d.y & 0xffffu), &saturated); va.w = cell_sat_add(va.w, unpack(d.y >> 16), &saturated);
-            vb.x = cell_sat_add(vb.x, unpack(d.z & 0xffffu), &saturated); vb.y = cell_sat_add(vb.y, unpack(d.z >> 16), &saturated);
-            vb.z = cell_sat_add(vb.z, unpack(d.w & 0xffffu), &saturated); vb.w = cell_sat_add(vb.w, unpack(d.w >> 16), &saturated);
-        }
-    };
     // rows this half owns: the lower half everything below the start row, the upper half the rest
     const int own_lo = upper ? cy0 : 0, own_hi = upper ? (int)geom.gh : cy0;     // [own_lo, own_hi)
     if (own_hi <= own_lo) { *moved_p += 0; return; }
@@ -1478,12 +1041,12 @@ __device__ __noinline__ void ray_half_writeback(const MapGeom& geom, const RayIt
             for (int k = 0; k < DEPTH; ++k) {
                 if (!need[k]) continue;
                 const int t = tt + k;
-                if ((d[k].x | d[k].y | d[k].z | d[k].w) != 0u) merge_group(va[k], vb[k], d[k]);
+                if ((d[k].x | d[k].y | d[k].z | d[k].w) != 0u) merge_window_group(va[k], vb[k], d[k], &saturated);
                 if (start_row) {
                     const int lx = t * (int)TILE_COLS + 8 * uu - wx0;
                     if ((unsigned)lx < (unsigned)ww && (uint32_t)(lx >> 3) < HALF_XCHG_GROUPS) {
                         const uint4 dl = s_lrow[lx >> 3];
-                        if ((dl.x | dl.y | dl.z | dl.w) != 0u) merge_group(va[k], vb[k], dl);
+                        if ((dl.x | dl.y | dl.z | dl.w) != 0u) merge_window_group(va[k], vb[k], dl, &saturated);
                     }
                 }
                 V8 o8; o8.a = va[k]; o8.b = vb[k];
@@ -1693,9 +1256,13 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
             flush_pending();
             pop_next();   // (s_next, s_item, s_pose are read only after the barrier that ends this item)
         }
-        if (walked)
-            ray_walk_half(geom, scan, s_beam, s_nmine, px, py, ptheta, sx, sy, cx0, cy0, rad, upper, wy0, wh, band0, s_win, s_row,
-                          s_rowb, s_blo, s_bhi, s_ext, &s_nspill, my_spill, &spilled, &cell_steps);
+        if (walked) {
+            // the window holds every in-grid cell within `rad` of the start in this half's rows
+            const bool disc_in_grid = cx0 - rad >= 0 && cx0 + rad < gw && (upper ? cy0 + rad < gh : cy0 - rad >= 0);
+            ray_walk_packed<true>(geom, scan, s_beam, s_nmine, px, py, ptheta, sx, sy, cx0, cy0, rad, disc_in_grid, wy0, wh, band0,
+                                  s_win, s_row, s_rowb, s_blo, s_bhi, s_ext, nullptr, nullptr, &s_nspill, my_spill, nullptr,
+                                  &spilled, &cell_steps);
+        }
 #ifdef SLAMRS_RAY_TRACE
         if (threadIdx.x == 0) atomicAdd(&g_ray_trace[12], (unsigned long long)(clock64() - t_prev));   // warp 0's own walk (longest beams)
 #endif
@@ -2016,12 +1583,11 @@ cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan
         cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ray_update_packed, threads, wmax * 2);
         if (e != cudaSuccess) return e;
         if (per_sm < 1) per_sm = 1;
-        if (per_sm > 4) per_sm = 4;   // (the spill scratch is sized for 4 CTAs per SM)
+        if (per_sm > 4) per_sm = 4;
         uint32_t grid = (uint32_t)(per_sm * num_sms);
         if (grid > n_local) grid = n_local;
-        k_ray_update_packed<<<grid, threads, wmax * 2, stream>>>(geom, scan, results, first_particle, alive_list, nullptr, nullptr, nullptr,
-                                                                 nullptr, spill_scratch, slot_of, cells, meta, bands, cells_per_grid, radius,
-                                                                 radius_cells, counters, n_local);
+        k_ray_update_packed<<<grid, threads, wmax * 2, stream>>>(geom, scan, results, first_particle, alive_list, slot_of, cells, meta,
+                                                                 bands, cells_per_grid, radius, radius_cells, counters);
         return cudaSuccess;
     }
     const bool vec = (geom.gw % 4u == 0u) && (cells_per_grid % 4u == 0u);

@@ -110,17 +110,19 @@ def test_simulator_odometry_and_workloads():
 
 
 def test_ray_walk_loop_compiled_to_the_tight_form():
-    """The free-run loop of k_ray_update_packed must stay one predicated block without the in-loop rebuild of
-    the row table's shared address (tools/sass_hot_loop.py; the slow form cost 15 % of the kernel on B200)."""
+    """The tested free-run loop of the walk in both packed kernels must stay one predicated block without the
+    in-loop rebuild of the row table's shared address (tools/sass_hot_loop.py; the slow form cost 15 % of the
+    kernel on B200)."""
     import shutil
     import sys
     if shutil.which("cuobjdump") is None:
         pytest.skip("cuobjdump not installed")
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     from sass_hot_loop import hot_loop
-    r = hot_loop(os.path.join(ROOT, "slamrs_b200", "libslamrs_gpu.so"))
-    assert not r["s2ur"] and not r["local_memory"], r["body"]
-    assert r["instructions"] <= 27, r["instructions"]
+    for kernel in ("k_ray_update_packed", "k_ray_update_half"):
+        r = hot_loop(os.path.join(ROOT, "slamrs_b200", "libslamrs_gpu.so"), kernel)
+        assert not r["s2ur"] and not r["local_memory"], (kernel, r["body"])
+        assert r["instructions"] <= 27, (kernel, r["instructions"])
 
 
 def test_bindings_agree_with_the_header_on_flags_phases_and_history():

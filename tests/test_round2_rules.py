@@ -4,7 +4,7 @@
   selects it (that rank pulls the grid; the item is listed first and the ray update signals its completion):
   either the first selector belongs to another rank, or the run of selectors crosses the end of the owner's
   range (kernels_resample.cu, `remote`).
-* ray_walk_half skips the free test for the first K cells of a walk: the cell reached after k steps of the
+* ray_walk_packed skips the free test for the first K cells of a walk: the cell reached after k steps of the
   reference's ray iterator (ray.rs:83-110) satisfies acc <= (k + 0.5)^2 + 0.25, whatever the direction."""
 import numpy as np
 import pytest
