@@ -60,7 +60,7 @@ struct StepCounters {
     unsigned long long ray_items_back;   // ray work list: slot owners whose grid a peer GPU pulls (first among the owners)
     unsigned long long ray_items_front_local;  // the other clones (behind the pulled ones)
     unsigned long long ray_items_back_local;   // the other slot owners (last)
-    unsigned long long fuse_overflow;    // fused ray update: more parked hits than its scratch holds (error, cannot happen by its bound)
+    unsigned long long fuse_overflow;    // fused ray update: more parked hits than its scratch holds (error; cannot happen by RAY_OCC_PER_RAY_MAX, kernels_ray.cu)
     unsigned long long do_resample;      // k_weights: this step resamples (always 1 unless adaptive resampling is on)
     unsigned long long carry_active;     // the weights of the last step were carried over (it did not resample)
     unsigned long long fold_rounds;      // k_weights: rounds the exact left fold needed (1 = proven at once)

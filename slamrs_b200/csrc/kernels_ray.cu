@@ -386,7 +386,25 @@ __host__ __device__ inline int ray_window_cells_upper_bound_packed(int radius) {
 //  * a ray whose endpoint cell is (ax, ay) cells away from the start cell visits only cells within
 //    (ax + 2, ay + 2) of it; if that corner is inside the disc window and the disc is inside the
 //    grid, no per-cell window or grid test is needed.
-constexpr uint32_t RAY_SPILL_CAP = 4u * RAY_PACKED_MAX_BEAMS;
+//
+// At most RAY_OCC_PER_RAY_MAX = 7 cells of one ray are occupied. In cell units, let S be the start point, u the
+// unit direction of the ray, d the measured distance, E the endpoint (|E - S| = d). The iterator visits the cells the
+// line S + t u passes through, in order of t, one grid line per step: up to the endpoint cell the cells it meets for
+// t in [0, d], then additional_steps = 2 more. A cell is occupied when its centre c has |c - S| in [d - 1, d + 1]
+// (map.rs:148-172, tolerance 2). Every point p of the cell is within sqrt(2)/2 of c, so the line meets an occupied
+// cell at some t = |p - S| >= d - 1 - sqrt(2)/2. The occupied cells up to the endpoint cell therefore all meet the
+// line in [d - 1.71, d]: one cell plus one per grid line crossed inside that interval, which holds fewer than
+// 1.71 |u_x| + 1 vertical and 1.71 |u_y| + 1 horizontal lines, at most 1.71 sqrt(2) + 2 = 4.42 together: at most
+// 4 crossings, 5 cells. With the 2 cells after the endpoint cell: 7. A zero-length ray parks 3 hits. The walk's f32
+// rounding moves a step by far less than a cell at these distances; tests/test_ray_bypass_bounds.py searches a lattice
+// of start offsets, headings and distances with the reference's walk and finds at most 5.
+//
+// So one work item parks at most 7 hits per ray of its half: RAY_SPILL_CAP entries. The lower half's parked hits on
+// the start row, all of them occupied hits of window cells, travel to the upper half as 16-bit counts per start-row
+// cell (HalfXchg::occ): at most 7 x 2,047 < 65,536 of them.
+constexpr uint32_t RAY_OCC_PER_RAY_MAX = 7;
+constexpr uint32_t RAY_SPILL_CAP = RAY_OCC_PER_RAY_MAX * RAY_PACKED_MAX_BEAMS;
+static_assert(RAY_SPILL_CAP <= 0xffffu, "a start-row count of parked hits is 16 bits");
 // SLAMRS_RAY_TRACE (tuning builds): thread 0 of every CTA adds the cycles it spent per phase of an item
 #ifdef SLAMRS_RAY_TRACE
 __device__ unsigned long long g_ray_trace[16];
@@ -416,8 +434,8 @@ __device__ __forceinline__ unsigned ray_smid() { unsigned r; asm volatile("mov.u
 //
 // Hits that bypass the window (the 32nd occupied hit of a cell in one scan, zero-length rays, and cells outside
 // the window) take the exact path. kParkBypass: they are parked in my_spill and applied after the write-back --
-// a clone's own slot receives its cells only then; at most 4 occupied cells per ray (3 hits of a zero-length ray),
-// so RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS entries suffice when the window holds every cell a ray reaches.
+// a clone's own slot receives its cells only then; at most RAY_OCC_PER_RAY_MAX occupied cells per ray (3 hits of a
+// zero-length ray), so RAY_SPILL_CAP entries suffice when the window holds every cell a ray reaches.
 // Otherwise they go straight to the grid with a saturating CAS, widening the slot's band table where the window's
 // bands do not cover them.
 template <bool kParkBypass>
@@ -922,14 +940,13 @@ k_ray_update_packed(MapGeom geom, ScanDevice scan, const ParticleResult* __restr
 constexpr int HALF_MAX_ROWS = RAY_MAX_RADIUS + 1;
 constexpr int HALF_MAX_BANDS = HALF_MAX_ROWS / BAND_ROWS + 2;
 constexpr uint32_t HALF_XCHG_GROUPS = 36;
-constexpr uint32_t HALF_XCHG_HITS = 60;
 struct alignas(16) HalfXchg {           // lower half -> upper half of the same particle
     uint4 row[HALF_XCHG_GROUPS];        // the lower CTA's window row for the start row (packed 16-bit cells, 8 per group)
     int band_lo, band_hi;               // columns the lower half touched in its rows of the shared band (hi < lo: none)
-    uint32_t n_hits;                    // exact-path hits of lower rays on the start row (applied by the upper CTA)
+    uint32_t n_hits;                    // parked hits of lower rays on the start row (applied by the upper CTA)
     uint32_t pad;
     int ext[4];                         // what the lower half touched {xmin, ymin, xmax, ymax} (the upper half commits the slot's box)
-    uint32_t hits[HALF_XCHG_HITS];
+    uint4 occ[HALF_XCHG_GROUPS];        // those hits: occupied count per start-row window cell (16 bits, cells as in `row`)
 };
 static_assert(sizeof(HalfXchg) % 16 == 0, "exchange records are accessed as 16-byte pieces");
 
@@ -1069,7 +1086,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
                   uint32_t* __restrict__ xdone, uint32_t n_local, uint32_t signal_epoch) {
     extern __shared__ __align__(16) uint32_t s_win[];   // two 16-bit cells per word; behind the window: this half's beam list
     uint16_t* s_beam = reinterpret_cast<uint16_t*>(reinterpret_cast<unsigned char*>(s_win) + window_bytes);
-    __shared__ uint32_t s_nspill, s_nmine, s_eo_shared;
+    __shared__ uint32_t s_nspill, s_nmine, s_eo_shared, s_nxhits;
     __shared__ int s_blo[HALF_MAX_BANDS], s_bhi[HALF_MAX_BANDS];
     __shared__ int2 s_row[HALF_MAX_ROWS + 1];           // .x = first window cell of the row, .y = x0 | width << 16
     __shared__ uint32_t s_rowb[HALF_MAX_ROWS];          // shared byte address of column x = 0 of the row
@@ -1171,7 +1188,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
         const int rad = walked ? radius : 0;
         ext_init(s_ext);
         if (threadIdx.x == 0) {
-            s_nspill = 0u; s_nmine = 0u; s_xinfo[0] = 0x7fffffff; s_xinfo[1] = -1; s_eo_shared = 0u;
+            s_nspill = 0u; s_nmine = 0u; s_xinfo[0] = 0x7fffffff; s_xinfo[1] = -1; s_eo_shared = 0u; s_nxhits = 0u;
             s_lext[0] = s_lext[1] = 0x7fffffff; s_lext[2] = s_lext[3] = -1;
         }
         for (int i = threadIdx.x; i < HALF_MAX_BANDS; i += blockDim.x) { s_blo[i] = 0x7fffffff; s_bhi[i] = -1; }
@@ -1319,23 +1336,35 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
             HalfXchg* x = xchg + item;
             const int2 row = s_row[wh - 1];                        // the start row is this window's last
             const int groups = row.y >> 19;
-            if (threadIdx.x < HALF_XCHG_GROUPS)
+            // parked hits of lower rays on the start row travel too (the upper half writes that row), as 16-bit
+            // counts per cell in s_lrow, which the lower half does not use otherwise
+            {
+                uint32_t* s_occ = reinterpret_cast<uint32_t*>(s_lrow);
+                const uint32_t rx0 = (uint32_t)(row.y & 0xffff), ns = min(s_nspill, RAY_SPILL_CAP);
+                for (uint32_t k = threadIdx.x; k < ns; k += blockDim.x) {
+                    const uint32_t e = my_spill[k];
+                    if ((int)((e >> 15) & 0x7fffu) != cy0) continue;
+                    const uint32_t lx = (e & 0x7fffu) - rx0;
+                    if ((e & 0x40000000u) && lx < 8u * HALF_XCHG_GROUPS) {
+                        atomicAdd(&s_occ[lx >> 1], 1u << ((lx & 1u) << 4));
+                        atomicAdd(&s_nxhits, 1u);
+                    } else {
+                        atomicAdd(&counters->fuse_overflow, 1ull);   // (a lower ray parks only occupied hits of window cells)
+                    }
+                }
+            }
+            __syncthreads();
+            if (threadIdx.x < HALF_XCHG_GROUPS) {
                 x->row[threadIdx.x] = (int)threadIdx.x < groups ? win4[(row.x >> 3) + threadIdx.x] : make_uint4(0u, 0u, 0u, 0u);
+                x->occ[threadIdx.x] = s_lrow[threadIdx.x];
+            }
             if (threadIdx.x == 0) {
                 const int lb = shared_band - band0;
                 const bool any = shared_band >= 0 && (unsigned)lb < (unsigned)HALF_MAX_BANDS && s_bhi[lb] >= s_blo[lb];
                 x->band_lo = any ? s_blo[lb] : 0x7fffffff;
                 x->band_hi = any ? s_bhi[lb] : -1;
                 x->ext[0] = s_ext[0]; x->ext[1] = s_ext[1]; x->ext[2] = s_ext[2]; x->ext[3] = s_ext[3];
-                // parked hits of lower rays on the start row travel too: the upper half writes that row
-                uint32_t nh = 0u;
-                const uint32_t ns = min(s_nspill, RAY_SPILL_CAP);
-                for (uint32_t k = 0; k < ns; ++k) {
-                    const uint32_t e = my_spill[k];
-                    if ((int)((e >> 15) & 0x7fffu) == cy0) { if (nh < HALF_XCHG_HITS) x->hits[nh] = e; nh++; }
-                }
-                if (nh > HALF_XCHG_HITS) atomicAdd(&counters->fuse_overflow, 1ull);
-                x->n_hits = min(nh, HALF_XCHG_HITS);
+                x->n_hits = s_nxhits;
                 // the shared band's old entry, before the upper half replaces it
                 s_eo_shared = (fused && shared_band >= 0) ? bands[shared_band] : 0u;
             }
@@ -1358,11 +1387,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
             if (threadIdx.x == 0) {
                 s_xinfo[0] = __ldcg(&x->band_lo); s_xinfo[1] = __ldcg(&x->band_hi);
                 s_lext[0] = __ldcg(&x->ext[0]); s_lext[1] = __ldcg(&x->ext[1]); s_lext[2] = __ldcg(&x->ext[2]); s_lext[3] = __ldcg(&x->ext[3]);
-                const uint32_t nh = __ldcg(&x->n_hits);
-                for (uint32_t k = 0; k < nh; ++k) {
-                    const uint32_t at = atomicAdd(&s_nspill, 1u);
-                    if (at < RAY_SPILL_CAP) my_spill[at] = __ldcg(&x->hits[k]);
-                }
+                s_nxhits = __ldcg(&x->n_hits);
             }
             __syncthreads();
             if (warp == 0) {   // what the lower rays touched on the start row counts for this half's extents
@@ -1424,6 +1449,14 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
                 const uint32_t x = e & 0x7fffu, y = (e >> 15) & 0x7fffu;
                 if (!upper && (int)y == cy0) continue;
                 global_cell_add(&grid[phys_index(geom, x, y)], (e & 0x40000000u) ? CELL_OCC_INC : CELL_FREE_INC, &saturated);
+            }
+            if (upper && walked && s_nxhits != 0u) {   // and the lower half's, n hits of a cell in one saturating add
+                const uint32_t* occ = reinterpret_cast<const uint32_t*>(xchg[item].occ);
+                const uint32_t rx0 = (uint32_t)(s_row[0].y & 0xffff);
+                for (uint32_t k = threadIdx.x; k < 8u * HALF_XCHG_GROUPS; k += blockDim.x) {
+                    const uint32_t n = (__ldcg(&occ[k >> 1]) >> ((k & 1u) << 4)) & 0xffffu;
+                    if (n != 0u) global_cell_add(&grid[phys_index(geom, rx0 + k, (uint32_t)cy0)], n * CELL_OCC_INC, &saturated);
+                }
             }
         }
         if (helper) {

@@ -20,7 +20,7 @@ from common import SEED, WEIGHT_RTOL, at_scale_config, compare_step, lockstep, m
 pytestmark = pytest.mark.gpu
 
 RAY_PACKED_MAX_BEAMS = 2047                    # kernels_ray.cu: the packed window's 11-bit free field
-RAY_SPILL_CAP = 4 * RAY_PACKED_MAX_BEAMS       # parked hits per work item of the fused ray update
+RAY_SPILL_CAP = 7 * RAY_PACKED_MAX_BEAMS       # parked hits per work item of the fused ray update
 SORT_MAX_BEAMS = 2048                          # k_sort_beams
 LOC_WIN = 1024                                 # k_loc_step: scan beams per window
 FLAGS = {"default": 0, "generic": _lib.FLAG_GENERIC_RAY_KERNEL}
@@ -189,7 +189,7 @@ def _with_beams(obs, dist, valid, angle=None):
 # spends at least 44 (130) cells outside a window sized from the finite distances. The +-inf beams (two thirds) point
 # in every direction, so each half of the disc receives at least 300 of them: on the 512^2 grid, whose tiled slots
 # take the fused ray update, >= 300 x 130 = 39,000 window-bypassing hits per half-particle work item, far above the
-# RAY_SPILL_CAP = 8,188 it can park (the 200^2 grid is not tiled: its packed kernel adds them to the grid directly).
+# RAY_SPILL_CAP = 14,329 it can park (the 200^2 grid is not tiled: its packed kernel adds them to the grid directly).
 N_NONFINITE = 900
 
 

@@ -243,9 +243,7 @@ def quality_run(matcher, n=64, steps=40):
     cfg = GridMapSlamConfig(position=(-12.8, -12.8), width=25.6, height=25.6, resolution=0.05, n_particles=n)
     sim = Simulator(reference_scene(5.0), n_beams=360, scanner_range=6.0, wheel_base=0.1)
     errs = []
-    # the generic ray kernel: the packed one fails on this scene at 64 particles ("more window-bypassing hits than its
-    # scratch holds"), with the matcher off as well; the kernel choice changes no result
-    with GridMapSlam(cfg, GpuPlacement(seed=SEED, flags=_lib.FLAG_GENERIC_RAY_KERNEL)) as g:
+    with GridMapSlam(cfg, GpuPlacement(seed=SEED)) as g:
         g.set_scan_matcher(matcher)
         for _ in range(steps):
             obs, odo = sim.next_scan(0.08, 0.10)
