@@ -74,7 +74,13 @@ enum slamrs_flags {
      * particle survives a later resampling and receives a scan -- which, with thousands of particles
      * and a few hundred survivors per step, most clones never do. The observable state is identical.
      * Whole-grid copies (SLAMRS_FLAG_FULL_GRID_COPY) are always eager. */
-    SLAMRS_FLAG_EAGER_COPY = 16
+    SLAMRS_FLAG_EAGER_COPY = 16,
+    /* Issue every step as the serial kernel sequence: stream events fork the planner off and join it, a separate
+     * kernel commits the step, and profiling records events between the phases. By default a single-GPU step on a
+     * device-resident scan (slamrs_gpu_set_scan_device) with the fused ray update chains its kernels instead: the
+     * ray update's last CTA waits for the planner on the device and commits the step, and profiling reads timestamps
+     * the kernels take. Results are identical either way. */
+    SLAMRS_FLAG_SERIAL_STEPS = SLAMRS_FLAG_EAGER_COPY << 1   /* = 32 */
 };
 
 typedef struct slamrs_gpu_handle slamrs_gpu_handle;
@@ -313,9 +319,13 @@ void* slamrs_gpu_stream(slamrs_gpu_handle* h);
 /* number of kernels this handle has launched since create */
 uint64_t slamrs_gpu_launch_count(const slamrs_gpu_handle* h);
 
-/* Per-phase device timing (CUDA events on the handle's stream). enable, run steps, then read:
+/* Per-phase device timing. enable, run steps, then read:
  * out_ms[SLAMRS_PHASE_COUNT] = summed milliseconds per phase, *out_steps = steps covered.
- * Reading synchronises the stream and resets the accumulation. */
+ * Reading synchronises the stream and resets the accumulation. The serial step sequence (SLAMRS_FLAG_SERIAL_STEPS)
+ * records CUDA events between its phases; a chained step (see that flag) takes %globaltimer stamps inside its
+ * kernels instead, which leaves its kernel chain intact. There RAY_UPDATE is the ray kernel's own span, PULL the
+ * wait of its last CTA for the planner, COPY the commit; phases of overlapping kernels may overlap, and a phase that
+ * another one hides counts 0. */
 enum slamrs_phase {
     SLAMRS_PHASE_MOTION_LIKELIHOOD = 0,
     SLAMRS_PHASE_ALL_GATHER = 1,

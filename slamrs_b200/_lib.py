@@ -19,6 +19,7 @@ FLAG_UPDATE_ALL_PARTICLES = 2
 FLAG_FULL_GRID_COPY = 4
 FLAG_NCCL_EXCHANGE = 8
 FLAG_EAGER_COPY = 16
+FLAG_SERIAL_STEPS = 32
 HISTORY_VALUES = 8
 
 EXPORTS = [

@@ -116,9 +116,15 @@ struct slamrs_gpu_handle {
     const float* ext_angle = nullptr;
     const float* ext_dist = nullptr;
     const uint8_t* ext_valid = nullptr;
-    // profiling: per step SLAMRS_PHASE_COUNT+1 boundary events
+    // profiling: per step SLAMRS_PHASE_COUNT+1 phase boundaries, as events on the stream (serial sequence) or as
+    // %globaltimer stamps written by the kernels themselves (chained sequence, d_prof)
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;   // [PROF_RING][SLAMRS_PHASE_COUNT + 1]
+    unsigned long long* d_prof = nullptr;   // [PROF_RING][SLAMRS_PHASE_COUNT + 1], zero until written
+    std::vector<uint8_t> prof_stamped;      // [PROF_RING]: the step's boundaries are in d_prof
+    bool prof_by_stamps = false;            // the step being issued writes stamps (PROF_MARK records nothing)
+    // chained sequence: the planner's epoch (d_chain[0]) and the ray update's exit counter (d_chain[1])
+    unsigned long long* d_chain = nullptr;
     uint32_t prof_recorded = 0;
     double prof_ms[SLAMRS_PHASE_COUNT] = {0, 0, 0, 0, 0, 0, 0};
     uint64_t prof_steps = 0;
@@ -304,6 +310,7 @@ void free_all(slamrs_gpu_handle* h) {
     cudaFree(h->d_export); cudaFree(h->d_barrier); cudaFree(h->d_peer_cells); cudaFree(h->d_peer_meta);
     cudaFree(h->d_peer_results); cudaFree(h->d_peer_flags); cudaFree(h->d_peer_bands);
     cudaFree(h->d_history);
+    cudaFree(h->d_prof); cudaFree(h->d_chain);
     for (cudaEvent_t e : h->prof_events) cudaEventDestroy(e);
     h->prof_events.clear();
     if (h->h_counters) cudaFreeHost(h->h_counters);
@@ -351,13 +358,20 @@ constexpr uint32_t PROF_MARKS = SLAMRS_PHASE_COUNT + 1;
 int prof_flush(slamrs_gpu_handle* h) {
     if (h->prof_recorded == 0) return SLAMRS_OK;
     CU_TRY(h, cudaStreamSynchronize(h->stream));
+    std::vector<unsigned long long> stamps((size_t)PROF_RING * PROF_MARKS);
+    CU_TRY(h, cudaMemcpy(stamps.data(), h->d_prof, sizeof(unsigned long long) * stamps.size(), cudaMemcpyDeviceToHost));
     for (uint32_t r = 0; r < h->prof_recorded; ++r) {
+        const unsigned long long* t = stamps.data() + (size_t)r * PROF_MARKS;
         for (int p = 0; p < SLAMRS_PHASE_COUNT; ++p) {
             float ms = 0.f;
-            CU_TRY(h, cudaEventElapsedTime(&ms, h->prof_events[r * PROF_MARKS + p], h->prof_events[r * PROF_MARKS + p + 1]));
+            if (h->prof_stamped[r])   // (the kernels of one step may overlap: a phase that another one hides counts 0)
+                ms = t[p + 1] > t[p] ? (float)((double)(t[p + 1] - t[p]) * 1e-6) : 0.f;
+            else
+                CU_TRY(h, cudaEventElapsedTime(&ms, h->prof_events[r * PROF_MARKS + p], h->prof_events[r * PROF_MARKS + p + 1]));
             h->prof_ms[p] += ms;
         }
     }
+    CU_TRY(h, cudaMemset(h->d_prof, 0, sizeof(unsigned long long) * stamps.size()));
     h->prof_steps += h->prof_recorded;
     h->prof_recorded = 0;
     return SLAMRS_OK;
@@ -366,7 +380,7 @@ int prof_flush(slamrs_gpu_handle* h) {
 // records boundary mark `m` of the current step when profiling is on
 #define PROF_MARK(h, m)                                                                                   \
     do {                                                                                                  \
-        if ((h)->profiling) CU_TRY(h, cudaEventRecord((h)->prof_events[(h)->prof_recorded * PROF_MARKS + (m)], (h)->stream)); \
+        if ((h)->profiling && !(h)->prof_by_stamps) CU_TRY(h, cudaEventRecord((h)->prof_events[(h)->prof_recorded * PROF_MARKS + (m)], (h)->stream)); \
     } while (0)
 
 // the copies k_materialize_list has listed: shared grids get their own cells (extent copies)
@@ -419,6 +433,17 @@ int fetch_counters(slamrs_gpu_handle* h) {
     return SLAMRS_OK;
 }
 
+// bookkeeping once every kernel of a SLAM step is queued
+int step_issued(slamrs_gpu_handle* h, int nxt) {
+    CU_TRY(h, cudaGetLastError());
+    h->cur = nxt;
+    h->step++;
+    h->counters_fresh = false;
+    h->mirror_by_step = h->mirror_wanted;
+    h->est_box_stale = false;
+    return SLAMRS_OK;
+}
+
 // One localisation step (localiser mode): motion + likelihood against the term table, then the SLAM step's own
 // weights and resampling kernels without a survivor list -- three launches, chained by programmatic dependent launch.
 int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
@@ -442,7 +467,7 @@ int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
                             h->d_counters);
     h->launches += 3;
     for (uint32_t m = 3; m < PROF_MARKS; ++m) PROF_MARK(h, m);
-    if (h->profiling) h->prof_recorded++;
+    if (h->profiling) h->prof_stamped[h->prof_recorded++] = 0;
     CU_TRY(h, cudaGetLastError());
     h->cur = nxt;
     h->step++;
@@ -669,6 +694,8 @@ int slamrs_gpu_create(const slamrs_gpu_config* cfg, slamrs_gpu_handle** out) {
     CREATE_CU(cudaMemsetAsync(h->d_history, 0xff, sizeof(StepRecord) * STEP_HISTORY, h->stream));
     CREATE_CU(cudaMalloc(&h->d_barrier, sizeof(int)));
     CREATE_CU(cudaMemsetAsync(h->d_barrier, 0, sizeof(int), h->stream));
+    CREATE_CU(cudaMalloc(&h->d_chain, sizeof(unsigned long long) * 2));
+    CREATE_CU(cudaMemsetAsync(h->d_chain, 0, sizeof(unsigned long long) * 2, h->stream));
     launch_init_slots(h->stream, h->d_slot[0], h->n_local, h->d_spare, h->n_spare, h->d_counters, h->rank, h->d_meta, h->d_alias);
     h->launches++;
     CREATE_CU(cudaGetLastError());
@@ -1001,12 +1028,21 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     const uint32_t pull_epoch = flag_pulls ? (uint32_t)(h->step + 1ull) : 0u;
     // (readers | done | xflag | xdone are cleared by k_motion)
     const size_t n_zero = half_items ? 2 * (size_t)h->n_slots + 2 * (size_t)h->n_local : 0;
+    // Chained sequence (one GPU, device-resident scan, fused half-item ray update, no scan matching): between the index
+    // kernel and the next step only kernels sit on the stream. The ray update's last CTA acquires the planner's epoch
+    // and completes the step (RayTail) instead of an event join and a commit launch, and profiling takes %globaltimer
+    // stamps inside the kernels instead of recording events between them. SLAMRS_FLAG_SERIAL_STEPS keeps the serial
+    // sequence (the eager, whole-grid and strict modes have no fused ray update and keep it anyway).
+    const bool chain = h->world == 1 && fuse && half_items && !h->match_on && h->scan_external &&
+                       (h->cfg.flags & SLAMRS_FLAG_SERIAL_STEPS) == 0;
+    h->prof_by_stamps = chain;
+    unsigned long long* prof = (h->profiling && chain) ? h->d_prof + (size_t)h->prof_recorded * PROF_MARKS : nullptr;
     // 1. motion sample + beam-endpoint likelihood (pre-update map) -> results[first .. first+n_local)
     PROF_MARK(h, 0);
     launch_motion_likelihood(s, h->geom, od, scan, h->d_pose[cur], h->d_slot[cur], h->defer ? h->d_alias : nullptr, h->d_cells, h->d_meta, h->cells_per_grid,
                              h->d_results, h->first, h->n_local, caller ? h->d_z : nullptr, h->cfg.seed, h->step, h->d_term_table, h->d_valid_list, h->d_n_valid,
                              h->d_carry, h->d_counters, h->p2p_exchange ? h->d_peer_results : nullptr, res_off, h->rank, h->world,
-                             h->d_readers, (uint32_t)n_zero, h->match_on ? &h->match : nullptr, h->d_match_stats);
+                             h->d_readers, (uint32_t)n_zero, h->match_on ? &h->match : nullptr, h->d_match_stats, prof);
     h->launches += h->match_on ? 3 : 2;   // k_motion (+ k_scan_match) + k_likelihood
     h->match_last_step = h->match_on;
     h->match_last_max_moves = h->match.max_moves;
@@ -1028,7 +1064,8 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     //    which local particles survive
     PROF_MARK(h, 2);
     // (k_weights also zeroes the per-step counters)
-    launch_weights(s, h->d_results, h->n_total, h->d_wnorm, h->d_cum, h->d_fold, (double)h->cfg.resample_threshold, h->d_counters);
+    launch_weights(s, h->d_results, h->n_total, h->d_wnorm, h->d_cum, h->d_fold, (double)h->cfg.resample_threshold, h->d_counters,
+                   prof ? prof + 1 : nullptr);
     // 3b. deferred copies: the clones among the particles about to be written get their own cells. Either the
     //     ray kernel does it while it integrates the scan (fused: k_resample_indices lists the survivors as
     //     clones | owners, no copy kernels), or they are listed now and copied after PROF_MARK 3. Before the
@@ -1074,6 +1111,7 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     pa.step = h->step;
     pa.staged = plan_can_stage(h->n_local, h->n_spare);
     pa.alias_of = h->d_alias; pa.defer = h->defer;
+    pa.done_epoch = chain ? h->d_chain : nullptr;
     launch_plan(h->side_stream, pa);
     h->launches += 3;   // k_weights, k_resample_indices, k_plan
     if (flag_pulls) {
@@ -1083,7 +1121,7 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
                     h->d_readers + h->n_slots);
         h->launches++;
     }
-    CU_TRY(h, cudaEventRecord(h->ev_plan, h->side_stream));
+    if (!chain) CU_TRY(h, cudaEventRecord(h->ev_plan, h->side_stream));
     PROF_MARK(h, 3);
     if (h->defer && !fuse) {
         int mrc = materialize_copies(h, all_particles);
@@ -1095,14 +1133,22 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
         CU_TRY(h, cudaStreamWaitEvent(s, h->ev_sort, 0));
         h->order_pending = false;
     }
+    const RayTail tail{h->d_chain, h->step + 1ull, reinterpret_cast<unsigned int*>(h->d_chain + 1),
+                       h->d_history + (h->step % STEP_HISTORY), h->mirror_wanted ? h->h_counters : nullptr,
+                       prof ? prof + 3 : nullptr, h->barrier_timeout_ns};
     CU_TRY(h, launch_ray_update(s, h->geom, scan, h->d_results, h->first, h->n_local, h->d_alive,
                                 fuse ? h->d_ray_items : nullptr, fuse ? h->d_ray_items + h->n_local : nullptr,
                                 fuse ? h->d_readers : nullptr,
                                 fuse ? h->d_readers + h->n_slots : nullptr, h->d_readers + 2 * (size_t)h->n_slots, h->d_ray_xchg,
                                 h->d_ray_spill, h->d_slot[cur],
                                 h->d_cells, h->d_meta, h->d_bands, h->cells_per_grid, h->radius_cells, h->d_counters, &h->window_cells,
-                                force_generic, h->num_sms, h->d_readers + 2 * (size_t)h->n_slots + h->n_local, pull_epoch));
+                                force_generic, h->num_sms, h->d_readers + 2 * (size_t)h->n_slots + h->n_local, pull_epoch,
+                                chain ? &tail : nullptr));
     h->launches++;
+    if (chain) {   // the ray update has completed the step (RayTail)
+        if (h->profiling) h->prof_stamped[h->prof_recorded++] = 1;
+        return step_issued(h, nxt);
+    }
     PROF_MARK(h, 5);
     CU_TRY(h, cudaStreamWaitEvent(s, h->ev_plan, 0));   // join: the copy lists are ready
     // 6. grid traffic: one launch copies from local and (over NVLink) remote sources alike. Across
@@ -1133,14 +1179,8 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
                         h->boxed_copy, h->d_counters, h->d_history + (h->step % STEP_HISTORY),
                         h->mirror_wanted ? h->h_counters : nullptr);   // (a store over PCIe: only when a sync follows at once)
     h->launches++;
-    if (h->profiling) h->prof_recorded++;
-    CU_TRY(h, cudaGetLastError());
-    h->cur = nxt;
-    h->step++;
-    h->counters_fresh = false;
-    h->mirror_by_step = h->mirror_wanted;
-    h->est_box_stale = false;
-    return SLAMRS_OK;
+    if (h->profiling) h->prof_stamped[h->prof_recorded++] = 0;
+    return step_issued(h, nxt);
 }
 
 int slamrs_gpu_sync(slamrs_gpu_handle* h) {
@@ -1153,6 +1193,8 @@ int slamrs_gpu_sync(slamrs_gpu_handle* h) {
                     h->h_counters->barrier_timeout == 2ull
                         ? "a peer GPU's handle was destroyed (its step failed or its owner left); this handle can only be destroyed"
                         : "a peer GPU did not reach the step barrier within the time limit");
+    if (h->h_counters->chain_timeout)
+        return fail(h, SLAMRS_E_INTERNAL, "the ray update's tail did not see the planner finish within the time limit");
     if (h->h_counters->fuse_overflow)
         return fail(h, SLAMRS_E_INTERNAL, "fused ray update: more window-bypassing hits than its scratch holds");
     if (h->h_counters->window_overflow)
@@ -1389,6 +1431,9 @@ int slamrs_gpu_set_profiling(slamrs_gpu_handle* h, int enabled) {
     if (enabled && h->prof_events.empty()) {
         h->prof_events.resize((size_t)PROF_RING * PROF_MARKS);
         for (auto& e : h->prof_events) CU_TRY(h, cudaEventCreate(&e));
+        h->prof_stamped.assign(PROF_RING, 0);
+        CU_TRY(h, cudaMalloc(&h->d_prof, sizeof(unsigned long long) * PROF_RING * PROF_MARKS));
+        CU_TRY(h, cudaMemset(h->d_prof, 0, sizeof(unsigned long long) * PROF_RING * PROF_MARKS));
     }
     if (!enabled) {
         int rc = prof_flush(h);

@@ -66,6 +66,7 @@ struct StepCounters {
     unsigned long long fold_rounds;      // k_weights: rounds the exact left fold needed (1 = proven at once)
     unsigned long long fold_heads;       // k_weights: chunks resolved by the sequential chain (binade changes)
     unsigned long long fold_fallback;    // k_weights: bit 0 / 1 = the raw-weight sum / the running sum fell back to one thread
+    unsigned long long chain_timeout;    // the ray update's tail gave up waiting for the planner (error)
     int est_box[4];                      // that extent {x0, y0, x1, y1}; -1 when another rank owns the estimate
     double sum;                          // sum of raw weights (particle.rs:50)
     double n_eff;                        // 1 / sum of squared normalised weights (particle.rs:59-65)
@@ -170,7 +171,8 @@ void launch_motion_likelihood(cudaStream_t stream, MapGeom geom, OdomModel od, S
                               uint32_t peer_offset /* records in front of this step's generation */, uint32_t rank,
                               uint32_t world, uint32_t* zero_words /* n_zero words that k_motion clears (may be null with 0) */,
                               uint32_t n_zero, const ScanMatchParams* match /* null: no scan matching */,
-                              uint2* match_stats /* with match: n_local x {moves, poses scored} */);
+                              uint2* match_stats /* with match: n_local x {moves, poses scored} */,
+                              unsigned long long* prof = nullptr /* profiling: k_motion's entry stamp goes to prof[0] */);
 void launch_fill_term_table(cudaStream_t stream, double* table);
 void launch_scan_match(cudaStream_t stream, MapGeom geom, ScanMatchParams mp, OdomModel od, const float* pose_cur,
                        const int32_t* alias_of /* may be null */, const uint32_t* cells, const SlotMeta* meta,
@@ -184,6 +186,19 @@ void launch_peer_barrier(cudaStream_t stream, unsigned long long* const* peer_fl
 void launch_peer_goodbye(cudaStream_t stream, unsigned long long* const* peer_flags, unsigned long long* my_flags,
                          uint32_t rank, uint32_t world, unsigned long long timeout_ns, StepCounters* counters);
 
+// The step's tail folded into the half-item ray update (one GPU, default path; see slamrs_gpu_step_async): the last CTA
+// to leave acquires the planner's epoch and then does what k_commit_boxes does with an empty copy list -- completes the
+// step's history record and, on request, the host's counter mirror -- so that no event join and no commit launch sit
+// on the stream between two steps.
+struct RayTail {
+    const unsigned long long* plan_epoch;   // k_plan publishes `epoch` here (release) once its outputs are written
+    unsigned long long epoch;
+    unsigned int* exit_count;               // CTAs that have left; 0 before the launch, reset by the last CTA
+    StepRecord* record;
+    StepCounters* host_mirror;              // null: no mirror
+    unsigned long long* prof;               // profiling: this step's PROF_MARKS %globaltimer stamps, else null
+    unsigned long long timeout_ns;          // bound of the wait for the planner (counters->chain_timeout on expiry)
+};
 // the fused path applies (packed window kernel, whole-grid tiled slots)
 bool ray_update_can_fuse(const MapGeom& geom, uint32_t n_beams, size_t cells_per_grid, bool force_generic, int radius_cells);
 size_t ray_spill_scratch_words(int num_sms);
@@ -204,7 +219,8 @@ cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan
                               uint32_t* xdone /* per work item, zeroed by the caller */,
 
                               uint32_t signal_epoch /* != 0 (half-item kernel only): every integrated slot's SlotMeta::pad0
-                                                       receives it once both halves are in place (peers that pull the slot wait for it) */);
+                                                       receives it once both halves are in place (peers that pull the slot wait for it) */,
+                              const RayTail* tail = nullptr /* half-item kernel only: the step's tail, folded in */);
 
 // k_weights' launch for a population: a cluster of `cluster` CTAs of `threads` threads, each thread folding `chunk`
 // consecutive elements, held in registers (regs) or re-read from global memory (the generic kernel)
@@ -213,8 +229,10 @@ WeightsShape weights_shape(uint32_t n_total);
 // fold_scratch: weights_scratch_doubles() doubles
 // resample_tau > 0: counters->do_resample = N_eff < tau * N (adaptive resampling; N_eff from the reference's strict
 // left fold of the squares), else 1
+// prof (profiling, may be null): the first CTA stores %globaltimer into prof[0..1] once the weights are in place
 void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t n_total, double* w_norm,
-                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters);
+                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters,
+                    unsigned long long* prof = nullptr);
 size_t weights_scratch_doubles();
 int weights_trace(long long* out64);   // tuning builds (-DSLAMRS_FOLD_TRACE): clock stamps of the last k_weights
 
@@ -257,6 +275,7 @@ struct PlanArgs {
     // k_materialize_list makes a shared grid private when its particle is about to be written.
     int32_t* alias_of;         // n_local + n_spare_cap
     bool defer;
+    unsigned long long* done_epoch;   // may be null: receives step + 1 (release, gpu scope) once every output is written
 };
 void launch_plan(cudaStream_t stream, const PlanArgs& a);
 // Shared grids that are about to be written (local particles selected by the index vector, or all

@@ -432,31 +432,10 @@ __global__ void k_commit_boxes(const CopyItem* __restrict__ items, const unsigne
             items[k].dst_bands[b] = items[k].src_bands[b];
         }
     }
-    if (record && blockIdx.x == 0 && threadIdx.x == 0) {
-        record->copy_bytes = counters->copy_bytes;
-        record->n_alive = counters->n_alive;
-        record->ray_cell_steps = counters->ray_cell_steps;
-        record->ray_copy_bytes = counters->ray_copy_bytes;
-        record->n_copies += counters->n_mat;          // clones made private before the ray update
-        record->n_leaders += counters->n_mat_leaders;
-        // informed extent of the published map, for the windowed read-out (sources are not written here)
-        const SlotMeta* em = reinterpret_cast<const SlotMeta*>((uintptr_t)counters->est_meta_ptr);
-        if (em == nullptr) { counters->est_box[0] = counters->est_box[1] = counters->est_box[2] = counters->est_box[3] = -1; }
-        else {
-            const SlotMeta m = *em;
-            const bool empty = m.x1 <= m.x0 || m.y1 <= m.y0;
-            counters->est_box[0] = empty ? 0 : m.x0; counters->est_box[1] = empty ? 0 : m.y0;
-            counters->est_box[2] = empty ? 0 : m.x1; counters->est_box[3] = empty ? 0 : m.y1;
-        }
-    }
-    // The last kernel of a step leaves the step counters in the host's page-locked mirror (a store through the mapping,
-    // not a memcpy -- see k_publish_counters): the host's wait for the step is then a plain stream synchronisation.
+    if (record && blockIdx.x == 0 && threadIdx.x == 0) commit_step_record(counters, record);
     if (host_mirror != nullptr && blockIdx.x == 0) {
         __syncthreads();   // thread 0's est_box
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(counters);
-        uint32_t* dst = reinterpret_cast<uint32_t*>(host_mirror);
-        for (uint32_t i = threadIdx.x; i < sizeof(StepCounters) / sizeof(uint32_t); i += blockDim.x) dst[i] = __ldcg(src + i);
-        __threadfence_system();
+        publish_mirror(counters, host_mirror);
     }
 }
 void launch_commit_boxes(cudaStream_t stream, const CopyItem* items, const unsigned long long* n_items, uint32_t max_items,

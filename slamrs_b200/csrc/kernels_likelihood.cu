@@ -13,8 +13,10 @@ __global__ void __launch_bounds__(128)
 k_motion(OdomModel od, const float* __restrict__ pose_cur, const int32_t* __restrict__ slot_of,
          ParticleResult* __restrict__ results, uint32_t first_particle, uint32_t n_local,
          const double* __restrict__ z_draws, uint64_t seed, uint64_t step, ScanDevice scan,
-         float2* __restrict__ valid_beams, uint32_t* __restrict__ n_valid, uint32_t* __restrict__ zero_words, uint32_t n_zero) {
+         float2* __restrict__ valid_beams, uint32_t* __restrict__ n_valid, uint32_t* __restrict__ zero_words, uint32_t n_zero,
+         unsigned long long* __restrict__ prof) {
     pdl_launch_dependents();   // k_likelihood may take its place on the SMs now; it waits for this grid before it reads
+    if (prof != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *prof = globaltimer_ns();
     // the ray update's per-step flags and counters start from zero (instead of a memset in front of the step)
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_zero; i += gridDim.x * blockDim.x) zero_words[i] = 0u;
     // Block 0 also compacts the scan's VALID beams, in beam order, for k_likelihood (the likelihood kernel
@@ -114,9 +116,11 @@ void launch_motion_likelihood(cudaStream_t stream, MapGeom geom, OdomModel od, S
                               const double* term_table, float2* valid_beams, uint32_t* n_valid,
                               const double* carry, const StepCounters* counters,
                               ParticleResult* const* peer_results, uint32_t peer_offset, uint32_t rank, uint32_t world,
-                              uint32_t* zero_words, uint32_t n_zero, const ScanMatchParams* match, uint2* match_stats) {
+                              uint32_t* zero_words, uint32_t n_zero, const ScanMatchParams* match, uint2* match_stats,
+                              unsigned long long* prof) {
     k_motion<<<(n_local + 127u) / 128u, 128, 0, stream>>>(od, pose_cur, slot_of, results, first_particle, n_local,
-                                                         z_draws, seed, step, scan, valid_beams, n_valid, zero_words, n_zero);
+                                                         z_draws, seed, step, scan, valid_beams, n_valid, zero_words, n_zero,
+                                                         prof);
     if (match)   // refines the sampled poses in results[] before the likelihood reads them
         launch_scan_match(stream, geom, *match, od, pose_cur, alias_of, cells, meta, cells_per_grid, results, first_particle,
                           n_local, valid_beams, n_valid, match_stats);

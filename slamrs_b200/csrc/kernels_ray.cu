@@ -1076,6 +1076,40 @@ __device__ __noinline__ void ray_half_writeback(const MapGeom& geom, const RayIt
     *moved_p += moved;
 }
 
+// RayTail: the last CTA to leave completes the step. Every CTA's counter updates, box commits and reader signals are
+// issued before its exit is counted (fence + barrier + counted exit, as a grid barrier does); the history record and
+// the estimate's extent also need the planner's outputs, so the last CTA acquires its epoch first -- the planner ran
+// beside this kernel and has almost always finished. The wait is bounded: a planner that does not arrive is reported
+// through counters->chain_timeout instead of holding the GPU.
+__device__ __noinline__ void ray_step_tail(const RayTail& tail, StepCounters* counters) {
+    __shared__ bool s_last;
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = atomicAdd(tail.exit_count, 1u) == gridDim.x - 1u;
+    __syncthreads();
+    if (!s_last) return;
+    if (threadIdx.x == 0) {
+        __threadfence();
+        *tail.exit_count = 0u;   // every other CTA has left: ready for the next step's launch
+        if (tail.prof != nullptr) tail.prof[2] = globaltimer_ns();   // end of the ray update proper
+        const unsigned long long t0 = globaltimer_ns();
+        for (;;) {
+            unsigned long long e;
+            asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(e) : "l"(tail.plan_epoch) : "memory");
+            if (e >= tail.epoch) break;
+            if (globaltimer_ns() - t0 > tail.timeout_ns) { counters->chain_timeout = 1ull; break; }
+            __nanosleep(256);
+        }
+        if (tail.prof != nullptr) tail.prof[3] = globaltimer_ns();   // the planner has joined
+        commit_step_record(counters, tail.record);
+    }
+    if (tail.host_mirror != nullptr) {
+        __syncthreads();   // thread 0's est_box
+        publish_mirror(counters, tail.host_mirror);
+    }
+    if (tail.prof != nullptr && threadIdx.x == 0) tail.prof[4] = globaltimer_ns();
+}
+
 __global__ void __maxnreg__(80)   // 4 CTAs of 192 threads per SM
 k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restrict__ results, uint32_t first_particle,
                   const uint32_t* __restrict__ alive_list, const RayItem* __restrict__ clones, const RayItem* __restrict__ owners,
@@ -1083,7 +1117,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
                   HalfXchg* __restrict__ xchg, uint32_t* __restrict__ spill_scratch, const int32_t* __restrict__ slot_of,
                   uint32_t* __restrict__ cells, SlotMeta* __restrict__ meta, uint32_t* __restrict__ bands_all,
                   size_t cells_per_grid, int radius, uint32_t window_bytes, StepCounters* counters,
-                  uint32_t* __restrict__ xdone, uint32_t n_local, uint32_t signal_epoch) {
+                  uint32_t* __restrict__ xdone, uint32_t n_local, uint32_t signal_epoch, RayTail tail) {
     extern __shared__ __align__(16) uint32_t s_win[];   // two 16-bit cells per word; behind the window: this half's beam list
     uint16_t* s_beam = reinterpret_cast<uint16_t*>(reinterpret_cast<unsigned char*>(s_win) + window_bytes);
     __shared__ uint32_t s_nspill, s_nmine, s_eo_shared, s_nxhits;
@@ -1095,6 +1129,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
     __shared__ RayItem s_item;                          // the item s_next names and its particle's pose, fetched ahead
     __shared__ float s_pose[3];
     __shared__ uint4 s_lrow[HALF_XCHG_GROUPS];
+    if (tail.prof != nullptr && blockIdx.x == 0 && threadIdx.x == 0) tail.prof[0] = tail.prof[1] = globaltimer_ns();
     const unsigned long long n_items = counters->n_alive;
     const int gw = (int)geom.gw, gh = (int)geom.gh;
     const uint32_t win_base = (uint32_t)__cvta_generic_to_shared(s_win);
@@ -1486,6 +1521,7 @@ k_ray_update_half(MapGeom geom, ScanDevice scan, const ParticleResult* __restric
         atomicAdd(&counters->copy_bytes, (unsigned long long)moved * 32ull);
         atomicAdd(&counters->ray_copy_bytes, (unsigned long long)moved * 32ull);
     }
+    if (tail.plan_epoch != nullptr) ray_step_tail(tail, counters);
 }
 
 // =============================================================================== k_sort_beams
@@ -1579,7 +1615,8 @@ cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan
                               const RayItem* clones, const RayItem* owners, const uint32_t* readers, uint32_t* done,
                               uint32_t* xflag, void* xchg, uint32_t* spill_scratch, const int32_t* slot_of, uint32_t* cells,
                               SlotMeta* meta, uint32_t* bands, size_t cells_per_grid, int radius_cells, StepCounters* counters,
-                              uint64_t* window_cells, bool force_generic, int num_sms, uint32_t* xdone, uint32_t signal_epoch) {
+                              uint64_t* window_cells, bool force_generic, int num_sms, uint32_t* xdone, uint32_t signal_epoch,
+                              const RayTail* tail) {
     // half a particle per work item (whole-grid tiled slots whose window holds every reachable cell): 4 CTAs per SM
     if (ray_update_can_fuse(geom, scan.n_beams, cells_per_grid, force_generic, radius_cells)) {
         const int radius = ray_packed_radius(radius_cells);
@@ -1598,7 +1635,8 @@ cudaError_t launch_ray_update(cudaStream_t stream, MapGeom geom, ScanDevice scan
         if (grid > 2u * n_local) grid = 2u * n_local;
         k_ray_update_half<<<grid, threads, smem, stream>>>(geom, scan, results, first_particle, alive_list, clones, owners, readers, done,
                                                            xflag, (HalfXchg*)xchg, spill_scratch, slot_of, cells, meta, bands,
-                                                           cells_per_grid, radius, (uint32_t)wbytes, counters, xdone, n_local, signal_epoch);
+                                                           cells_per_grid, radius, (uint32_t)wbytes, counters, xdone, n_local, signal_epoch,
+                                                           tail ? *tail : RayTail{});
 #ifdef SLAMRS_RAY_TRACE
         ray_log_dump_after_launch(stream);
 #endif

@@ -365,7 +365,8 @@ __device__ bool exact_left_fold(cg::cluster_group& cluster, FoldShared<LREG>& sh
 template <int LREG, int THREADS>
 __global__ void __launch_bounds__(THREADS)
 k_weights(const ParticleResult* __restrict__ results, uint32_t n, double* __restrict__ w_norm,
-          double* __restrict__ cum, double* __restrict__ fold_scratch, double resample_tau, StepCounters* counters) {
+          double* __restrict__ cum, double* __restrict__ fold_scratch, double resample_tau, StepCounters* counters,
+          unsigned long long* __restrict__ prof) {
     cg::cluster_group cluster = cg::this_cluster();
     const uint32_t crank = cluster.block_rank(), C = cluster.num_blocks();
     __shared__ FoldShared<LREG> sh;
@@ -379,6 +380,7 @@ k_weights(const ParticleResult* __restrict__ results, uint32_t n, double* __rest
     pdl_wait();                // every weight of the step is in place (k_likelihood, or the barrier / all-gather behind it)
     FOLD_STAMP(0);
     const uint32_t gt = crank * THREADS + threadIdx.x;
+    if (prof != nullptr && gt == 0) prof[0] = prof[1] = globaltimer_ns();   // the likelihood (+ exchange) phases end here
     const uint32_t L = LREG ? (uint32_t)LREG : (n + C * THREADS - 1u) / (C * THREADS);
     const uint32_t lo = min(n, gt * L), hi = min(n, lo + L), cnt = hi - lo;
 
@@ -610,7 +612,8 @@ WeightsShape weights_shape(uint32_t n_total) {
     return s;
 }
 void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t n_total, double* w_norm,
-                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters) {
+                    double* cum, double* fold_scratch, double resample_tau, StepCounters* counters,
+                    unsigned long long* prof) {
     const WeightsShape shape = weights_shape(n_total);
     const uint32_t c = shape.cluster;
     const bool regs = shape.regs;
@@ -626,8 +629,8 @@ void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 2;
-    if (regs) cudaLaunchKernelEx(&cfg, k_weights<FOLD_LREG, FOLD_THREADS>, results, n_total, w_norm, cum, fold_scratch, resample_tau, counters);
-    else cudaLaunchKernelEx(&cfg, k_weights<0, FOLD_GENERIC_THREADS>, results, n_total, w_norm, cum, fold_scratch, resample_tau, counters);
+    if (regs) cudaLaunchKernelEx(&cfg, k_weights<FOLD_LREG, FOLD_THREADS>, results, n_total, w_norm, cum, fold_scratch, resample_tau, counters, prof);
+    else cudaLaunchKernelEx(&cfg, k_weights<0, FOLD_GENERIC_THREADS>, results, n_total, w_norm, cum, fold_scratch, resample_tau, counters, prof);
 }
 size_t weights_scratch_doubles() { return 2u * FOLD_MAX_CHUNKS; }
 int weights_trace(long long* out64) {
@@ -1082,6 +1085,13 @@ __global__ void __launch_bounds__(1024) k_plan(PlanArgs a) {
             r.step = a.step; r.n_copies = n_copied; r.n_pulls = n_remote; r.distinct = distinct; r.n_leaders = n_lead;
             r.n_alive = 0; r.copy_bytes = 0; r.ray_cell_steps = 0; r.ray_copy_bytes = 0;   // filled in by the step's last kernel (k_commit_boxes)
             a.history[a.step % STEP_HISTORY] = r;
+        }
+    }
+    if (a.done_epoch != nullptr) {   // the ray update's tail acquires this before it completes the step (RayTail)
+        __syncthreads();
+        if (t == 0) {
+            __threadfence();
+            asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(a.done_epoch), "l"(a.step + 1ull) : "memory");
         }
     }
 }
