@@ -371,7 +371,9 @@ int prof_flush(slamrs_gpu_handle* h) {
             h->prof_ms[p] += ms;
         }
     }
-    CU_TRY(h, cudaMemset(h->d_prof, 0, sizeof(unsigned long long) * stamps.size()));
+    // on the handle's stream: a plain cudaMemset runs on the legacy stream, which the (non-blocking) step stream does not
+    // wait for, so it could land after the next step's kernels had stamped their marks
+    CU_TRY(h, cudaMemsetAsync(h->d_prof, 0, sizeof(unsigned long long) * stamps.size(), h->stream));
     h->prof_steps += h->prof_recorded;
     h->prof_recorded = 0;
     return SLAMRS_OK;
@@ -1032,8 +1034,9 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     // kernel and the next step only kernels sit on the stream. The ray update's last CTA acquires the planner's epoch
     // and completes the step (RayTail) instead of an event join and a commit launch, and profiling takes %globaltimer
     // stamps inside the kernels instead of recording events between them. SLAMRS_FLAG_SERIAL_STEPS keeps the serial
-    // sequence (the eager, whole-grid and strict modes have no fused ray update and keep it anyway).
-    const bool chain = h->world == 1 && fuse && half_items && !h->match_on && h->scan_external &&
+    // sequence (the eager, whole-grid and strict modes have no fused ray update and keep it anyway). The chained tail
+    // leaves no host counter mirror; the synchronous update, the one caller that wants it, uploads a host scan.
+    const bool chain = h->world == 1 && fuse && half_items && !h->match_on && h->scan_external && !h->mirror_wanted &&
                        (h->cfg.flags & SLAMRS_FLAG_SERIAL_STEPS) == 0;
     h->prof_by_stamps = chain;
     unsigned long long* prof = (h->profiling && chain) ? h->d_prof + (size_t)h->prof_recorded * PROF_MARKS : nullptr;
@@ -1134,8 +1137,7 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
         h->order_pending = false;
     }
     const RayTail tail{h->d_chain, h->step + 1ull, reinterpret_cast<unsigned int*>(h->d_chain + 1),
-                       h->d_history + (h->step % STEP_HISTORY), h->mirror_wanted ? h->h_counters : nullptr,
-                       prof ? prof + 3 : nullptr, h->barrier_timeout_ns};
+                       h->d_history + (h->step % STEP_HISTORY), prof ? prof + 3 : nullptr, h->barrier_timeout_ns};
     CU_TRY(h, launch_ray_update(s, h->geom, scan, h->d_results, h->first, h->n_local, h->d_alive,
                                 fuse ? h->d_ray_items : nullptr, fuse ? h->d_ray_items + h->n_local : nullptr,
                                 fuse ? h->d_readers : nullptr,
@@ -1433,7 +1435,7 @@ int slamrs_gpu_set_profiling(slamrs_gpu_handle* h, int enabled) {
         for (auto& e : h->prof_events) CU_TRY(h, cudaEventCreate(&e));
         h->prof_stamped.assign(PROF_RING, 0);
         CU_TRY(h, cudaMalloc(&h->d_prof, sizeof(unsigned long long) * PROF_RING * PROF_MARKS));
-        CU_TRY(h, cudaMemset(h->d_prof, 0, sizeof(unsigned long long) * PROF_RING * PROF_MARKS));
+        CU_TRY(h, cudaMemsetAsync(h->d_prof, 0, sizeof(unsigned long long) * PROF_RING * PROF_MARKS, h->stream));
     }
     if (!enabled) {
         int rc = prof_flush(h);

@@ -188,14 +188,14 @@ void launch_peer_goodbye(cudaStream_t stream, unsigned long long* const* peer_fl
 
 // The step's tail folded into the half-item ray update (one GPU, default path; see slamrs_gpu_step_async): the last CTA
 // to leave acquires the planner's epoch and then does what k_commit_boxes does with an empty copy list -- completes the
-// step's history record and, on request, the host's counter mirror -- so that no event join and no commit launch sit
-// on the stream between two steps.
+// step's history record and the estimate's extent -- so that no event join and no commit launch sit on the stream
+// between two steps. It leaves no host counter mirror: only the synchronous update asks for one, and its host scan
+// never takes the chained sequence.
 struct RayTail {
     const unsigned long long* plan_epoch;   // k_plan publishes `epoch` here (release) once its outputs are written
     unsigned long long epoch;
     unsigned int* exit_count;               // CTAs that have left; 0 before the launch, reset by the last CTA
     StepRecord* record;
-    StepCounters* host_mirror;              // null: no mirror
     unsigned long long* prof;               // profiling: this step's PROF_MARKS %globaltimer stamps, else null
     unsigned long long timeout_ns;          // bound of the wait for the planner (counters->chain_timeout on expiry)
 };

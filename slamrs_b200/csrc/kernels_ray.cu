@@ -1102,12 +1102,8 @@ __device__ __noinline__ void ray_step_tail(const RayTail& tail, StepCounters* co
         }
         if (tail.prof != nullptr) tail.prof[3] = globaltimer_ns();   // the planner has joined
         commit_step_record(counters, tail.record);
+        if (tail.prof != nullptr) tail.prof[4] = globaltimer_ns();
     }
-    if (tail.host_mirror != nullptr) {
-        __syncthreads();   // thread 0's est_box
-        publish_mirror(counters, tail.host_mirror);
-    }
-    if (tail.prof != nullptr && threadIdx.x == 0) tail.prof[4] = globaltimer_ns();
 }
 
 __global__ void __maxnreg__(80)   // 4 CTAs of 192 threads per SM
