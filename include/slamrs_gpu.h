@@ -303,12 +303,48 @@ typedef struct slamrs_gpu_sensor_model {
  * slamrs_gpu_map_probability writes). Uses position, resolution, grid size, n_particles, seed, rng_mode, device and
  * resample_threshold of cfg; world_size must be 1 and flags, slot_cells and spare_slots 0. Particles start at
  * Pose::default(); place them with init_uniform or set_poses. update / step_async / pose / weights and the other
- * particle accessors work as on a SLAM handle (step_async launches three kernels); the grid accessors (map_*,
+ * particle accessors work as on a SLAM handle (step_async launches three kernels, four with recovery); the grid accessors (map_*,
  * get_cells, set_cells, get_log_odds, get_extents, get_slots, get_step_history) return SLAMRS_E_INVALID_ARG. */
 int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_sensor_model* model,
                                 const double* map_probability, slamrs_gpu_handle** out);
 /* the localiser's grid_w * grid_h term table (f64, index row * grid_h + column), for tests */
 int slamrs_gpu_get_sensor_terms(slamrs_gpu_handle* h, double* out_cells);
+
+/* Recovery from kidnapping and false convergence: augmented MCL (Probabilistic Robotics, Table 8.3; ROS AMCL's
+ * recovery_alpha_slow / recovery_alpha_fast), bit-exact against the CPU oracle. Off by default; while it is off a
+ * localiser step is unchanged (three launches, the same bits). When it is on, every step does the following after
+ * k_resample_indices, in one more launch (k_loc_recover):
+ *   1. w_avg = sum / N, with sum the strict left fold of this step's raw weights (particle.rs:50, motion term
+ *      included), by __ddiv_rn; nothing below is contracted.
+ *   2. If sum is not finite, the state stays as it is and p = 0. Otherwise
+ *        w_slow = (w_slow == 0) ? w_avg : w_slow + alpha_slow * (w_avg - w_slow)
+ *        w_fast = (w_fast == 0) ? w_avg : w_fast + alpha_fast * (w_avg - w_fast)
+ *        p = (w_slow > 0) ? max(0, 1 - w_fast / w_slow) : 0, NaN mapped to 0.
+ *   3. The free cells are the cells of the loaded map with p < 0.5, in ascending cell index (row * grid_h + column),
+ *      listed once at create (4 bytes per free cell).
+ *   4. Draws from the shared stream keyed by the config seed, in both RNG modes (CALLER mode externalises only the
+ *      reference's own draws). For new particle m at step s, Philox counters (m, s lo32, s hi32, d):
+ *        d = 4: decision u_d = u53(a0, a1), cell u_c = u53(a2, a3);  d = 5: u_x = u53(b0, b1), u_y = u53(b2, b3);
+ *        d = 6: u_t = u53(c0, c1).
+ *   5. Particle m is replaced iff u_d < p, by cell free[min(n_free - 1, (uint32)(u_c * n_free))] at column col and
+ *      row row: x = (float)(pos_x + (col + u_x) * res), y = (float)(pos_y + (row + u_y) * res),
+ *      theta = (float)(-pi + u_t * 2pi), in f64 with pos_x, pos_y and res the config's f32 values.
+ *   6. The estimate (estimated_pose: the resampled pose of max_particle), the indices and the weights are the ones
+ *      resampling recorded: an injected particle never becomes the estimate in the step that creates it.
+ * The cost on a B200 and the behaviour after a kidnapping are in DESIGN.md section 11.1. */
+typedef struct slamrs_gpu_recovery {
+    uint32_t struct_size;   /* = sizeof(slamrs_gpu_recovery) */
+    uint32_t pad;
+    double alpha_slow;      /* (0, alpha_fast) */
+    double alpha_fast;      /* (alpha_slow, 1] */
+} slamrs_gpu_recovery;
+/* Localiser only; NULL turns recovery off; setting it resets w_slow and w_fast; takes effect at the next step.
+ * Returns SLAMRS_E_INVALID_ARG on a SLAM handle, with resample_threshold > 0 (carried weights put the raw sum on
+ * another scale), on a map without free cells, for alphas outside the ranges above and on a struct_size mismatch. */
+int slamrs_gpu_set_recovery(slamrs_gpu_handle* h, const slamrs_gpu_recovery* r);
+/* Last step: {w_slow, w_fast, p_inject} and the number of particles injected (out_injected may be NULL); all zero
+ * when the last step ran without recovery. Synchronises. */
+int slamrs_gpu_get_recovery_state(slamrs_gpu_handle* h, double out[3], uint64_t* out_injected);
 
 /* ------------------------------------------------------------------ introspection (tests, bench) */
 

@@ -102,6 +102,15 @@ pub struct slamrs_gpu_scan_match {
     pub max_moves: u32,
 }
 
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_recovery {
+    pub struct_size: u32,
+    pub pad: u32,
+    pub alpha_slow: f64,
+    pub alpha_fast: f64,
+}
+
 extern "C" {
     pub fn slamrs_gpu_grid_cells(extent: f32, resolution: f32, out_cells: *mut u32) -> c_int;
     pub fn slamrs_gpu_nccl_unique_id(out: *mut u8) -> c_int;
@@ -154,4 +163,6 @@ extern "C" {
     pub fn slamrs_gpu_get_log_odds(h: *mut slamrs_gpu_handle, particle: u64, out_cells: *mut f64) -> c_int;
     pub fn slamrs_gpu_set_scan_match(h: *mut slamrs_gpu_handle, m: *const slamrs_gpu_scan_match) -> c_int;
     pub fn slamrs_gpu_get_scan_match_stats(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
+    pub fn slamrs_gpu_set_recovery(h: *mut slamrs_gpu_handle, r: *const slamrs_gpu_recovery) -> c_int;
+    pub fn slamrs_gpu_get_recovery_state(h: *mut slamrs_gpu_handle, out: *mut f64, out_injected: *mut u64) -> c_int;
 }

@@ -5,7 +5,7 @@ This package is the host-side mirror of the reference interface plus the synthet
 generator. Importing it never falls back to a CPU implementation.
 """
 from .slam import (GpuPlacement, GridData, GridMapLocalizer, GridMapSlam, GridMapSlamConfig, Measurement, Observation,
-                   Odometry, Pose, ScanMatcher, SensorModel, grid_cells, nccl_unique_id)
+                   Odometry, Pose, Recovery, ScanMatcher, SensorModel, grid_cells, nccl_unique_id)
 
 __all__ = ["GpuPlacement", "GridData", "GridMapLocalizer", "GridMapSlam", "GridMapSlamConfig", "Measurement",
-           "Observation", "Odometry", "Pose", "ScanMatcher", "SensorModel", "grid_cells", "nccl_unique_id"]
+           "Observation", "Odometry", "Pose", "Recovery", "ScanMatcher", "SensorModel", "grid_cells", "nccl_unique_id"]

@@ -37,6 +37,7 @@ EXPORTS = [
     "slamrs_gpu_map_probability_async", "slamrs_gpu_map_wait",
     "slamrs_gpu_create_localizer", "slamrs_gpu_get_sensor_terms",
     "slamrs_gpu_set_scan_match", "slamrs_gpu_get_scan_match_stats",
+    "slamrs_gpu_set_recovery", "slamrs_gpu_get_recovery_state",
 ]
 MAP_F64, MAP_F32, MAP_U8 = 0, 1, 2
 SENSOR_BEAM_ENDPOINT, SENSOR_LIKELIHOOD_FIELD = 0, 1
@@ -65,6 +66,10 @@ class SensorModel(C.Structure):
 class ScanMatch(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("radius", C.c_uint32), ("step_xy", C.c_float), ("step_theta", C.c_float),
                 ("levels", C.c_uint32), ("max_moves", C.c_uint32)]
+
+
+class Recovery(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("pad", C.c_uint32), ("alpha_slow", C.c_double), ("alpha_fast", C.c_double)]
 
 
 class Stats(C.Structure):
@@ -144,6 +149,8 @@ def load():
     L.slamrs_gpu_get_sensor_terms.restype = i; L.slamrs_gpu_get_sensor_terms.argtypes = [vp, vp]
     L.slamrs_gpu_set_scan_match.restype = i; L.slamrs_gpu_set_scan_match.argtypes = [vp, C.POINTER(ScanMatch)]
     L.slamrs_gpu_get_scan_match_stats.restype = i; L.slamrs_gpu_get_scan_match_stats.argtypes = [vp, vp]
+    L.slamrs_gpu_set_recovery.restype = i; L.slamrs_gpu_set_recovery.argtypes = [vp, C.POINTER(Recovery)]
+    L.slamrs_gpu_get_recovery_state.restype = i; L.slamrs_gpu_get_recovery_state.argtypes = [vp, vp, C.POINTER(u64)]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
     L.slamrs_gpu_debug_resample_adaptive.restype = i

@@ -140,6 +140,13 @@ struct slamrs_gpu_handle {
     bool localizer = false;
     double* d_loc_terms = nullptr;   // n_cells
     double loc_outside = 0.0;        // term of an endpoint off the grid
+    // augmented-MCL recovery (slamrs_gpu_set_recovery)
+    uint32_t* d_loc_free = nullptr;  // ascending cell indices of the map's free cells (p < 0.5), n_free entries
+    uint32_t n_free = 0;
+    RecoveryState* d_recovery = nullptr;   // 2 entries, by step parity
+    bool recovery_on = false;
+    double alpha_slow = 0.0, alpha_fast = 0.0;
+    bool recovery_last_step = false;       // the last issued step ran k_loc_recover
     // scan-matching pose refinement (slamrs_gpu_set_scan_match)
     bool match_on = false;
     ScanMatchParams match{};
@@ -297,7 +304,7 @@ void free_all(slamrs_gpu_handle* h) {
     cudaFree(h->d_pool);
     cudaFree(h->d_slot[0]); cudaFree(h->d_slot[1]);
     cudaFree(h->d_pose[0]); cudaFree(h->d_pose[1]);
-    cudaFree(h->d_term_table); cudaFree(h->d_loc_terms);
+    cudaFree(h->d_term_table); cudaFree(h->d_loc_terms); cudaFree(h->d_loc_free); cudaFree(h->d_recovery);
     cudaFree(h->d_wnorm); cudaFree(h->d_cum); cudaFree(h->d_idx); cudaFree(h->d_fold); cudaFree(h->d_carry);
     cudaFree(h->d_angle);   // (d_dist and d_valid live in the same allocation)
     if (h->h_scan_stage) cudaFreeHost(h->h_scan_stage);
@@ -447,7 +454,8 @@ int step_issued(slamrs_gpu_handle* h, int nxt) {
 }
 
 // One localisation step (localiser mode): motion + likelihood against the term table, then the SLAM step's own
-// weights and resampling kernels without a survivor list -- three launches, chained by programmatic dependent launch.
+// weights and resampling kernels without a survivor list -- three launches, chained by programmatic dependent launch,
+// and k_loc_recover as a fourth while recovery is on.
 int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
     cudaStream_t s = h->stream;
     if (h->profiling && h->prof_recorded == PROF_RING) {
@@ -468,6 +476,12 @@ int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
                             RayLists{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u}, h->d_wnorm, h->d_carry,
                             h->d_counters);
     h->launches += 3;
+    if (h->recovery_on) {
+        launch_loc_recover(s, h->n_total, h->d_counters, h->d_recovery, h->step, h->alpha_slow, h->alpha_fast, h->cfg.seed,
+                           h->d_loc_free, h->n_free, h->geom, h->d_pose[nxt]);
+        h->launches++;
+    }
+    h->recovery_last_step = h->recovery_on;
     for (uint32_t m = 3; m < PROF_MARKS; ++m) PROF_MARK(h, m);
     if (h->profiling) h->prof_stamped[h->prof_recorded++] = 0;
     CU_TRY(h, cudaGetLastError());
@@ -767,10 +781,13 @@ int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_s
             return fail(nullptr, SLAMRS_E_INVALID_ARG, "occupied_above must lie in [0.5, 1)");
     }
     const size_t n_cells = (size_t)cfg->grid_w * cfg->grid_h;
-    for (size_t i = 0; i < n_cells; ++i)
+    uint32_t n_free = 0;   // cells of the recovery's free-cell list
+    for (size_t i = 0; i < n_cells; ++i) {
         if (!(map_probability[i] >= 0.0 && map_probability[i] <= 1.0))
             return fail(nullptr, SLAMRS_E_INVALID_ARG,
                         "map_probability[" + std::to_string(i) + "] is NaN or outside [0, 1]");
+        n_free += map_probability[i] < 0.5;
+    }
 
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
@@ -790,6 +807,7 @@ int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_s
     h->n_cells = (uint32_t)n_cells;
     h->geom = make_map_geom(cfg->pos_x, cfg->pos_y, cfg->resolution, cfg->grid_w, cfg->grid_h);
     h->loc_outside = field ? log((double)model->z_rand) : 0.0;   // ln(z_rand) / the reference's ln(1) for off-grid endpoints
+    h->n_free = n_free;
 
 #define CREATE_CU(expr)                                                                                   \
     do {                                                                                                  \
@@ -799,12 +817,14 @@ int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_s
             g_create_error = std::string(#expr) + ": " + cudaGetErrorString(_e);                          \
             cudaGetLastError();                                                                           \
             cudaFree(scratch);                                                                            \
+            cudaFree(free_scratch);                                                                       \
             free_all(h);                                                                                  \
             return _code;                                                                                 \
         }                                                                                                 \
     } while (0)
 
     uint32_t* scratch = nullptr;   // the distance transform's column pass (freed before returning)
+    uint32_t* free_scratch = nullptr;   // the free-cell list's tile offsets (freed before returning)
     DeviceGuard guard(device);
     cudaDeviceProp prop;
     CREATE_CU(cudaGetDeviceProperties(&prop, device));
@@ -848,8 +868,18 @@ int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_s
     CREATE_CU(launch_loc_terms(h->stream, h->d_export, cfg->grid_w, field ? 1 : 0, model->sigma, model->z_rand,
                                model->occupied_above, cfg->resolution, scratch, h->d_loc_terms));
     h->launches += field ? 2 : 1;
+    // the free-cell list, from the upload buffer before sim_scan reuses it (4 B per free cell)
+    CREATE_CU(cudaMalloc(&h->d_recovery, sizeof(RecoveryState) * 2));
+    if (n_free) {
+        CREATE_CU(cudaMalloc(&h->d_loc_free, sizeof(uint32_t) * n_free));
+        CREATE_CU(cudaMalloc(&free_scratch, sizeof(uint32_t) * loc_free_scratch_words(n_cells)));
+        launch_loc_free_cells(h->stream, h->d_export, n_cells, free_scratch, h->d_loc_free);
+        CREATE_CU(cudaGetLastError());
+        h->launches += 3;
+    }
     CREATE_CU(cudaStreamSynchronize(h->stream));
     cudaFree(scratch);
+    cudaFree(free_scratch);
 #undef CREATE_CU
     *out = h;
     return SLAMRS_OK;
@@ -861,6 +891,41 @@ int slamrs_gpu_get_sensor_terms(slamrs_gpu_handle* h, double* out_cells) {
     DeviceGuard g(h->device);
     CU_TRY(h, cudaMemcpyAsync(out_cells, h->d_loc_terms, sizeof(double) * h->n_cells, cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_set_recovery(slamrs_gpu_handle* h, const slamrs_gpu_recovery* r) {
+    if (!h) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no recovery (only a localizer has one)");
+    if (!r) {
+        h->recovery_on = false;
+        return SLAMRS_OK;
+    }
+    if (r->struct_size != sizeof(slamrs_gpu_recovery))
+        return fail(h, SLAMRS_E_INVALID_ARG, "slamrs_gpu_recovery struct_size mismatch");
+    if (!(r->alpha_slow > 0.0 && r->alpha_slow < r->alpha_fast && r->alpha_fast <= 1.0))
+        return fail(h, SLAMRS_E_INVALID_ARG, "recovery alphas must satisfy 0 < alpha_slow < alpha_fast <= 1");
+    if (h->cfg.resample_threshold > 0.0f)
+        return fail(h, SLAMRS_E_INVALID_ARG, "recovery needs resample_threshold 0 (adaptive resampling carries weights)");
+    if (h->n_free == 0) return fail(h, SLAMRS_E_INVALID_ARG, "the map has no free cells (p < 0.5) to inject particles into");
+    DeviceGuard g(h->device);
+    CU_TRY(h, cudaMemsetAsync(h->d_recovery, 0, sizeof(RecoveryState) * 2, h->stream));   // behind the steps issued so far
+    h->alpha_slow = r->alpha_slow;
+    h->alpha_fast = r->alpha_fast;
+    h->recovery_on = true;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_get_recovery_state(slamrs_gpu_handle* h, double out[3], uint64_t* out_injected) {
+    if (!h || !out) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no recovery (only a localizer has one)");
+    RecoveryState st{0.0, 0.0, 0.0, 0ull};
+    DeviceGuard g(h->device);
+    if (h->recovery_last_step)
+        CU_TRY(h, cudaMemcpyAsync(&st, h->d_recovery + ((h->step - 1u) & 1u), sizeof(st), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    out[0] = st.w_slow; out[1] = st.w_fast; out[2] = st.p;
+    if (out_injected) *out_injected = st.injected;
     return SLAMRS_OK;
 }
 

@@ -15,6 +15,8 @@
 //   kernels_misc.cu        k_export*       slam.rs:83-88 / map.rs:50-52;  k_sim_scan  simulator/src/sim.rs:134-159
 //   kernels_localize.cu    k_loc_step      localisation on a loaded map: motion + likelihood, one warp per 32 particles;
 //                          k_loc_terms_beam / k_loc_dt_cols / k_loc_dt_rows   sensor-term table at create
+//                          k_loc_free_count / k_loc_free_scan / k_loc_free_cells   free-cell list at create
+//                          k_loc_recover   augmented-MCL recovery behind k_resample_indices (off by default)
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -363,6 +365,20 @@ void launch_loc_step(cudaStream_t stream, MapGeom geom, OdomModel od, ScanDevice
                      ParticleResult* results, uint32_t n, const double* z_draws, uint64_t seed, uint64_t step,
                      const double* terms, double outside, const double* carry /* adaptive resampling, else null */,
                      const StepCounters* counters);
+// Augmented-MCL recovery of the localiser (slamrs_gpu_set_recovery). The ascending list of the map's free cells
+// (p < 0.5, index row * w + column) into free_cells[0, n_free), n_free counted by the host; `scratch` holds
+// loc_free_scratch_words(w * w) words
+size_t loc_free_scratch_words(size_t n_cells);
+void launch_loc_free_cells(cudaStream_t stream, const double* prob, size_t n_cells, uint32_t* scratch, uint32_t* free_cells);
+// One step's recovery state, double-buffered by step parity (state[step & 1] = the state after `step`)
+struct RecoveryState {
+    double w_slow, w_fast, p;       // the averages and the share of particles to replace
+    unsigned long long injected;    // particles replaced in that step
+};
+// behind k_resample_indices: the new averages from counters->sum, then the injections into pose_next
+void launch_loc_recover(cudaStream_t stream, uint32_t n, const StepCounters* counters, RecoveryState* state, uint64_t step,
+                        double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells, uint32_t n_free,
+                        MapGeom geom, float* pose_next);
 
 // test hooks
 void launch_debug_raycast(cudaStream_t stream, const float* x0, const float* y0, const float* x1, const float* y1,

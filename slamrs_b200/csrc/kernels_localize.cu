@@ -1,6 +1,7 @@
 // Monte Carlo localisation against one shared, read-only occupancy map: the per-cell sensor-term table built once
 // at create (k_loc_terms_beam, or k_loc_dt_cols + k_loc_dt_rows for the likelihood field) and the per-step kernel
-// k_loc_step (motion + likelihood, fused). k_weights and k_resample_indices run unchanged behind it.
+// k_loc_step (motion + likelihood, fused). k_weights and k_resample_indices run unchanged behind it, and with
+// recovery on (slamrs_gpu_set_recovery) k_loc_recover behind them, on the free-cell list built at create.
 #include "kernels_common.cuh"
 
 namespace slamrs {
@@ -168,6 +169,99 @@ void launch_loc_step(cudaStream_t stream, MapGeom geom, OdomModel od, ScanDevice
     const size_t smem = scan.n_beams > LOC_WIN ? sizeof(double) * LOC_WARPS * 32u * 32u : 0u;
     k_loc_step<<<(n + per_cta - 1u) / per_cta, per_cta, smem, stream>>>(geom, od, scan, pose_cur, results, n, z_draws, seed,
                                                                          step, terms, outside, carry, counters);
+}
+
+// =============================================================================== recovery (augmented MCL)
+// Free-cell list at create: an ordered compaction of p < 0.5 over the uploaded map in three launches -- the free cells
+// of every tile of FREE_TILE cells (k_loc_free_count), the exclusive scan of those counts (k_loc_free_scan, one CTA)
+// and the write of each tile's cells from its offset (k_loc_free_cells). Thread t of a tile owns its cells 8t .. 8t+7.
+constexpr uint32_t FREE_THREADS = 1024, FREE_PER_THREAD = 8, FREE_TILE = FREE_THREADS * FREE_PER_THREAD;
+
+__device__ __forceinline__ uint32_t free_bits(const double* __restrict__ prob, size_t n_cells, size_t base) {
+    uint32_t bits = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < FREE_PER_THREAD; ++k)
+        if (base + k < n_cells && prob[base + k] < 0.5) bits |= 1u << k;
+    return bits;
+}
+
+__global__ void __launch_bounds__(FREE_THREADS) k_loc_free_count(const double* __restrict__ prob, size_t n_cells,
+                                                                 uint32_t* __restrict__ counts) {
+    __shared__ uint32_t s_tot[33];
+    const size_t base = (size_t)blockIdx.x * FREE_TILE + (size_t)threadIdx.x * FREE_PER_THREAD;
+    uint32_t total;
+    block_excl_scan_u32((uint32_t)__popc(free_bits(prob, n_cells, base)), s_tot, &total);
+    if (threadIdx.x == 0) counts[blockIdx.x] = total;
+}
+
+__global__ void __launch_bounds__(FREE_THREADS) k_loc_free_scan(uint32_t* __restrict__ counts, uint32_t n_tiles) {
+    __shared__ uint32_t s_tot[33];
+    uint32_t carry = 0;
+    for (uint32_t i0 = 0; i0 < n_tiles; i0 += FREE_THREADS) {   // CTA-uniform
+        const uint32_t i = i0 + threadIdx.x;
+        uint32_t total;
+        const uint32_t ex = block_excl_scan_u32(i < n_tiles ? counts[i] : 0u, s_tot, &total);
+        if (i < n_tiles) counts[i] = carry + ex;
+        carry += total;
+    }
+}
+
+__global__ void __launch_bounds__(FREE_THREADS) k_loc_free_cells(const double* __restrict__ prob, size_t n_cells,
+                                                                 const uint32_t* __restrict__ offsets,
+                                                                 uint32_t* __restrict__ free_cells) {
+    __shared__ uint32_t s_tot[33];
+    const size_t base = (size_t)blockIdx.x * FREE_TILE + (size_t)threadIdx.x * FREE_PER_THREAD;
+    uint32_t bits = free_bits(prob, n_cells, base);
+    uint32_t total;
+    uint32_t o = offsets[blockIdx.x] + block_excl_scan_u32((uint32_t)__popc(bits), s_tot, &total);
+    for (; bits; bits &= bits - 1u) free_cells[o++] = (uint32_t)(base + (uint32_t)(__ffs(bits) - 1));
+}
+
+size_t loc_free_scratch_words(size_t n_cells) { return (n_cells + FREE_TILE - 1) / FREE_TILE; }
+
+void launch_loc_free_cells(cudaStream_t stream, const double* prob, size_t n_cells, uint32_t* scratch, uint32_t* free_cells) {
+    const uint32_t n_tiles = (uint32_t)loc_free_scratch_words(n_cells);
+    k_loc_free_count<<<n_tiles, FREE_THREADS, 0, stream>>>(prob, n_cells, scratch);
+    k_loc_free_scan<<<1, FREE_THREADS, 0, stream>>>(scratch, n_tiles);
+    k_loc_free_cells<<<n_tiles, FREE_THREADS, 0, stream>>>(prob, n_cells, scratch, free_cells);
+}
+
+// One thread per new particle, behind k_resample_indices. Every thread computes the same new state from the previous
+// step's (slot (step + 1) & 1); thread 0 stores it in slot step & 1 and clears the other slot's count for the next
+// step. With p > 0 a thread draws its particle's decision (slamrs_stream::recovery_draw) and replaces the resampled
+// pose; each warp adds its injections to the count with one atomic. The estimate, the indices and the weights that
+// k_weights and k_resample_indices recorded stay as they are.
+__global__ void __launch_bounds__(256)
+k_loc_recover(uint32_t n, const StepCounters* __restrict__ counters, RecoveryState* state, uint64_t step, double alpha_slow,
+              double alpha_fast, uint64_t seed, const uint32_t* __restrict__ free_cells, uint32_t n_free, uint32_t grid_h,
+              double pos_x, double pos_y, double res, float* __restrict__ pose_next) {
+    pdl_wait();   // k_resample_indices has completed (it waited for k_weights): counters->sum, the resampled poses
+    RecoveryState* prev = state + ((step + 1u) & 1u);
+    RecoveryState* cur = state + (step & 1u);
+    double w_slow = prev->w_slow, w_fast = prev->w_fast;
+    const double p = slamrs_stream::recovery_update(counters->sum, n, alpha_slow, alpha_fast, &w_slow, &w_fast);
+    const uint32_t m = blockIdx.x * blockDim.x + threadIdx.x;
+    if (m == 0) {
+        cur->w_slow = w_slow; cur->w_fast = w_fast; cur->p = p;
+        prev->injected = 0ull;
+    }
+    if (!(p > 0.0)) return;   // (grid-uniform)
+    float x, y, t;
+    const bool inj = m < n && slamrs_stream::recovery_draw(seed, step, m, p, free_cells, n_free, grid_h, pos_x, pos_y, res,
+                                                           &x, &y, &t);
+    const unsigned mask = __ballot_sync(0xffffffffu, inj);
+    if (inj) {
+        float* q = pose_next + 3 * (size_t)m;
+        q[0] = x; q[1] = y; q[2] = t;
+    }
+    if ((threadIdx.x & 31u) == 0 && mask) atomicAdd(&cur->injected, (unsigned long long)__popc(mask));
+}
+
+void launch_loc_recover(cudaStream_t stream, uint32_t n, const StepCounters* counters, RecoveryState* state, uint64_t step,
+                        double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells, uint32_t n_free,
+                        MapGeom geom, float* pose_next) {
+    launch_pdl(k_loc_recover, dim3((n + 255u) / 256u), dim3(256), 0, stream, n, counters, state, step, alpha_slow, alpha_fast,
+               seed, free_cells, n_free, geom.gh, (double)geom.pos_x, (double)geom.pos_y, (double)geom.res, pose_next);
 }
 
 }  // namespace slamrs

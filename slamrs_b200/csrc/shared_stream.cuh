@@ -11,6 +11,8 @@
 //           r = sqrt(-2 dlog(u1));  z1 = r * dcos(2 pi u2)  (centre distance draw)
 //                                   z2 = r * dsin(2 pi u2)  (heading draw)
 //   uniform counter (0, step lo32, step hi32, 1) -> U = ((x0:x1) >> 11) * 2^-53
+//   start   counter (particle, 0, 0, 2) and (particle, 0, 0, 3): uniform_pose
+//   recover counter (particle, step lo32, step hi32, 4 / 5 / 6): recovery_draw
 //
 // dlog / dsincos2pi are fixed sequences of IEEE binary64 + - * / (explicit round-to-nearest
 // intrinsics on the device, so no FMA contraction), which makes the stream bit-identical on
@@ -188,6 +190,45 @@ SS_HD void uniform_pose(uint64_t seed, uint32_t particle, double x0, double y0, 
     *px = (float)dadd(x0, dmul(u53(a.x[0], a.x[1]), dadd(x1, -x0)));
     *py = (float)dadd(y0, dmul(u53(a.x[2], a.x[3]), dadd(y1, -y0)));
     *ptheta = (float)dadd(-0x1.921fb54442d18p+1, dmul(u53(b.x[0], b.x[1]), 0x1.921fb54442d18p+2));
+}
+
+// Augmented-MCL recovery (slamrs_gpu_set_recovery). The averages of the raw weights, from the step's weight sum `sum`
+// over n particles: w_avg = sum / n; w = (w == 0) ? w_avg : w + alpha (w_avg - w) for both averages; the share of
+// particles to replace is p = max(0, 1 - w_fast / w_slow) (0 when w_slow is not positive, and for NaN). A sum that
+// is not finite leaves both averages as they are and gives p = 0.
+SS_HD double recovery_update(double sum, uint32_t n, double alpha_slow, double alpha_fast, double* w_slow, double* w_fast) {
+    if (!isfinite(sum)) return 0.0;
+    const double w_avg = ddiv(sum, (double)n);
+    *w_slow = *w_slow == 0.0 ? w_avg : dadd(*w_slow, dmul(alpha_slow, dadd(w_avg, -*w_slow)));
+    *w_fast = *w_fast == 0.0 ? w_avg : dadd(*w_fast, dmul(alpha_fast, dadd(w_avg, -*w_fast)));
+    if (!(*w_slow > 0.0)) return 0.0;
+    const double p = dadd(1.0, -ddiv(*w_fast, *w_slow));
+    return p > 0.0 ? p : 0.0;
+}
+// Entry of the free-cell list that the cell uniform u_c in [0, 1) selects. (In round-to-nearest the product stays
+// below n_free for every u_c the stream yields; the clamp keeps the index in range regardless.)
+SS_HD uint32_t recovery_slot(double u_c, uint32_t n_free) {
+    const uint32_t k = (uint32_t)dmul(u_c, (double)n_free);
+    return k < n_free - 1u ? k : n_free - 1u;
+}
+// Is new particle `particle` of step `step` replaced (u_d < p), and by which pose: a cell drawn from the ascending
+// list of free cells (index row * grid_h + column), a position uniform inside that cell and a heading in
+// [-pi, pi) as uniform_pose draws it. Counter domains 4 (u_d, u_c), 5 (u_x, u_y) and 6 (u_t), keyed by the step;
+// pos_x, pos_y and res are the config's f32 values widened. The poses of other particles are not touched.
+SS_HD bool recovery_draw(uint64_t seed, uint64_t step, uint32_t particle, double p, const uint32_t* free_cells,
+                         uint32_t n_free, uint32_t grid_h, double pos_x, double pos_y, double res, float* px, float* py,
+                         float* ptheta) {
+    const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32), s0 = (uint32_t)step, s1 = (uint32_t)(step >> 32);
+    const Words4 a = philox4x32_10(particle, s0, s1, 4u, k0, k1);
+    if (!(u53(a.x[0], a.x[1]) < p)) return false;
+    const uint32_t cell = free_cells[recovery_slot(u53(a.x[2], a.x[3]), n_free)];
+    const Words4 b = philox4x32_10(particle, s0, s1, 5u, k0, k1);
+    const Words4 c = philox4x32_10(particle, s0, s1, 6u, k0, k1);
+    const double col = (double)(cell % grid_h), row = (double)(cell / grid_h);
+    *px = (float)dadd(pos_x, dmul(dadd(col, u53(b.x[0], b.x[1])), res));
+    *py = (float)dadd(pos_y, dmul(dadd(row, u53(b.x[2], b.x[3])), res));
+    *ptheta = (float)dadd(-0x1.921fb54442d18p+1, dmul(u53(c.x[0], c.x[1]), 0x1.921fb54442d18p+2));
+    return true;
 }
 
 }  // namespace slamrs_stream

@@ -142,6 +142,23 @@ class ScanMatcher:
         return m
 
 
+@dataclass
+class Recovery:
+    """Recovery of a GridMapLocalizer from kidnapping and false convergence (slamrs_gpu_recovery; augmented MCL, ROS
+    AMCL's recovery_alpha_slow / recovery_alpha_fast). A short-term (alpha_fast) and a long-term (alpha_slow) average of
+    the mean raw weight are kept; while the short-term one is below the long-term one, a share 1 - w_fast / w_slow of
+    the resampled particles is replaced by poses drawn uniformly over the map's free cells (p < 0.5).
+    0 < alpha_slow < alpha_fast <= 1; the defaults are AMCL's usual values."""
+    alpha_slow: float = 0.001
+    alpha_fast: float = 0.1
+
+    def to_struct(self):
+        r = _lib.Recovery()
+        r.struct_size = C.sizeof(_lib.Recovery)
+        r.alpha_slow, r.alpha_fast = float(self.alpha_slow), float(self.alpha_fast)
+        return r
+
+
 def grid_cells(extent: float, resolution: float) -> int:
     """Map::new grid sizing (map.rs:28-31) as the library computes it."""
     out = C.c_uint32(0)
@@ -510,6 +527,19 @@ class GridMapLocalizer(GridMapSlam):
         out = np.zeros(self.grid_w * self.grid_h, np.float64)
         _lib.check(self._L.slamrs_gpu_get_sensor_terms(self._h, _ptr(out)), self._h)
         return out
+
+    def set_recovery(self, recovery: Optional[Recovery]) -> None:
+        """Recovery from the next update on (resets both averages); None turns it off (the default). Needs
+        resample_threshold 0 and a map with free cells."""
+        r = None if recovery is None else recovery.to_struct()
+        _lib.check(self._L.slamrs_gpu_set_recovery(self._h, None if r is None else C.byref(r)), self._h)
+
+    def recovery_state(self) -> dict:
+        """Of the last update: w_slow, w_fast, p_inject (the share of particles replaced) and injected (how many
+        were); all zero when it ran without recovery. Synchronises."""
+        out = np.zeros(3, np.float64); k = C.c_uint64(0)
+        _lib.check(self._L.slamrs_gpu_get_recovery_state(self._h, _ptr(out), C.byref(k)), self._h)
+        return {"w_slow": float(out[0]), "w_fast": float(out[1]), "p_inject": float(out[2]), "injected": int(k.value)}
 
 
 # ---------------------------------------------------------------------- kernel-level hooks
