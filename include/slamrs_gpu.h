@@ -169,7 +169,8 @@ void slamrs_gpu_destroy(slamrs_gpu_handle* h);
  *   valid      : Measurement.valid (robot.rs:93)
  *   dist_left / dist_right / wheel_dist : the three Odometry floats (robot.rs:115-123); the two
  *                Normal distributions are derived inside exactly as Odometry::new does (:132-150)
- *   z_draws    : rng_mode CALLER: 2*n_particles standard normals, particle-major
+ *   z_draws    : rng_mode CALLER: 2*n_particles standard normals, particle-major (a localiser: 2*N_t, two per
+ *                particle of its current generation, see slamrs_gpu_set_kld)
  *                (centre-distance draw, heading draw -- the draw order of robot.rs:175-176);
  *                every rank passes the full array. NULL in SHARED_STREAM mode.
  *   resample_u : rng_mode CALLER: pointer to the uniform [0,1) of particle.rs:84. NULL otherwise.
@@ -229,7 +230,7 @@ int slamrs_gpu_map_window(slamrs_gpu_handle* h, uint32_t format, int32_t x0, int
 
 /* ParticleFilter::number_of_effective_particles, particle.rs:59-65, evaluated on the normalised
  * weights of the last update BEFORE resampling (the reference never calls it; after resampling it
- * is trivially N). N before the first update. */
+ * is trivially N). N before the first update. A localiser: over the last step's N_t particles. */
 int slamrs_gpu_effective_particles(slamrs_gpu_handle* h, double* out);
 
 /* Global-localisation-style start (README.md:45 lists it as an idea; SURVEY.md 8(f)4): every particle of this
@@ -303,7 +304,8 @@ typedef struct slamrs_gpu_sensor_model {
  * slamrs_gpu_map_probability writes). Uses position, resolution, grid size, n_particles, seed, rng_mode, device and
  * resample_threshold of cfg; world_size must be 1 and flags, slot_cells and spare_slots 0. Particles start at
  * Pose::default(); place them with init_uniform or set_poses. update / step_async / pose / weights and the other
- * particle accessors work as on a SLAM handle (step_async launches three kernels, four with recovery); the grid accessors (map_*,
+ * particle accessors work as on a SLAM handle (step_async launches three kernels, four with recovery, one more with
+ * KLD-sampling; the particle accessors' sizes follow the population, see slamrs_gpu_set_kld); the grid accessors (map_*,
  * get_cells, set_cells, get_log_odds, get_extents, get_slots, get_step_history) return SLAMRS_E_INVALID_ARG. */
 int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_sensor_model* model,
                                 const double* map_probability, slamrs_gpu_handle** out);
@@ -346,6 +348,55 @@ int slamrs_gpu_set_recovery(slamrs_gpu_handle* h, const slamrs_gpu_recovery* r);
  * when the last step ran without recovery. Synchronises. */
 int slamrs_gpu_get_recovery_state(slamrs_gpu_handle* h, double out[3], uint64_t* out_injected);
 
+/* Adaptive population: KLD-sampling (Fox 2003; ROS AMCL's min_particles / max_particles / kld_err / kld_z), bit-exact
+ * against the CPU oracle. Off by default; while it is off a localiser step is unchanged (three launches, four with
+ * recovery, the same bits) and draws n_particles new particles. cfg.n_particles is the capacity C: every buffer is
+ * sized for it at create. The population N_t is the size of the current generation; it starts at C. A step with
+ * KLD-sampling on:
+ *   1. k = the number of distinct bins occupied by the N_t poses the step starts from (what the previous step,
+ *      recovery included, or init_uniform / set_poses left). A pose's cell is the one the likelihood gives a beam
+ *      endpoint at (x, y) (world_to_grid, is_valid, `as usize`); heading bin: t = fmod((double)theta, 2pi), t += 2pi
+ *      if t < 0, h = min(theta_bins - 1, (uint32)((t * theta_bins) / 2pi)) for 0 <= t < 2pi, else 0 (NaN, inf), in
+ *      f64 with 2pi = 0x1.921fb54442d18p+2. Bin ((row / bin_cells) * nbx + column / bin_cells) * theta_bins + h with
+ *      nbx = ceil(grid_w / bin_cells); every pose off the grid falls into the one bin nbx * nby * theta_bins.
+ *   2. N_{t+1} = n_min for k <= 1; otherwise, in f64 in AMCL's order (pf_resample_limit), uncontracted:
+ *      b = 2 / (9 (k - 1)), x = 1 - b + sqrt(b) z, n = (((k - 1) / (2 err)) x) x x, N_{t+1} = clamp(ceil(n), n_min,
+ *      n_max), n_max for a non-finite n or one >= n_max.
+ *   3. Motion, likelihood and weights over the N_t particles, as without KLD-sampling.
+ *   4. M = N_{t+1} draws (particle.rs:78-101 with M wherever N counts draws: r = U * 1.0 / M, u_m = r + (m - 1) * 1.0
+ *      / M); the walk over the running sum of the N_t normalised weights and its clamp at N_t - 1 are unchanged.
+ *   5. The estimate is new particle floor(max_particle * M / N_t) (64-bit integers), the same cumulative-mass position
+ *      as the reference's new[max_particle].
+ *   6. Recovery (if on) averages sum / N_t and injects over the M new particles.
+ * The size of a step lags AMCL's by one: AMCL counts the bins of the set it draws and stops once the bound is met;
+ * here a step draws what the bins of the set it starts from demand (see DESIGN.md section 11.2).
+ * One more kernel in front of the step (k_loc_kld: four launches, five with recovery). The host waits for it, so
+ * step_async on a handle with KLD-sampling on returns only once that kernel (not the step) has completed.
+ * Sizes of the particle accessors on a localiser: get_poses, set_poses and init_uniform use N (the current
+ * generation); get_weights and effective_particles the last step's N_t; get_resample_indices its M; a CALLER-mode
+ * z_draws holds 2 N_t normals. */
+typedef struct slamrs_gpu_kld {
+    uint32_t struct_size;   /* = sizeof(slamrs_gpu_kld) */
+    uint32_t n_min;         /* 1 <= n_min <= n_max */
+    uint32_t n_max;         /* <= n_particles (the capacity) */
+    uint32_t pad;
+    double err;             /* finite, (0, 1] */
+    double z;               /* finite, >= 0: the upper (1 - delta) quantile of the standard normal */
+    uint32_t bin_cells;     /* >= 1: grid cells per bin side */
+    uint32_t theta_bins;    /* 1..3600 */
+} slamrs_gpu_kld;
+/* Localiser only; takes effect at the next step; NULL turns it off (the next step then draws n_particles from N_t,
+ * and every step after it is the fixed-size step). Returns SLAMRS_E_INVALID_ARG on a SLAM handle, with
+ * resample_threshold > 0 (carried weights assume a fixed population), for fields outside the ranges above, for a bin
+ * bitmap of more than 2^28 bits and on a struct_size mismatch. */
+int slamrs_gpu_set_kld(slamrs_gpu_handle* h, const slamrs_gpu_kld* k);
+/* Last step: {N_t particles weighted, k occupied bins, N_{t+1} particles drawn}; all zero when it ran without
+ * KLD-sampling. Synchronises. */
+int slamrs_gpu_get_kld_state(slamrs_gpu_handle* h, uint64_t out[3]);
+/* The size of the current generation: the localiser's population N (n_particles until KLD-sampling changes it); a SLAM
+ * handle's n_local. */
+int slamrs_gpu_get_population(slamrs_gpu_handle* h, uint64_t* out);
+
 /* ------------------------------------------------------------------ introspection (tests, bench) */
 
 const char* slamrs_gpu_last_error(const slamrs_gpu_handle* h); /* never NULL; "" when none */
@@ -386,15 +437,15 @@ int slamrs_gpu_get_phase_ms(slamrs_gpu_handle* h, double out_ms[SLAMRS_PHASE_COU
 #define SLAMRS_HISTORY_VALUES 8
 int slamrs_gpu_get_step_history(slamrs_gpu_handle* h, uint64_t first_step, uint32_t count, uint64_t* out_values);
 
-/* current generation, this rank's shard: n_local * {x, y, theta} */
+/* current generation, this rank's shard: n_local * {x, y, theta} (a localiser: N, see slamrs_gpu_get_population) */
 int slamrs_gpu_get_poses(slamrs_gpu_handle* h, float* out_xyt);
 int slamrs_gpu_set_poses(slamrs_gpu_handle* h, const float* xyt);
 /* the resampler's bookkeeping: physical grid slot of every local particle (n_local entries) and the
  * list of spare slots (*out_n_spare entries; pass a buffer of spare_slots entries, or NULL) */
 int slamrs_gpu_get_slots(slamrs_gpu_handle* h, int32_t* out_slot_of, int32_t* out_spare, uint32_t* out_n_spare);
-/* last step, all N particles in pre-resample order: normalised and raw (un-normalised) weights */
+/* last step, all N particles in pre-resample order: normalised and raw (un-normalised) weights (a localiser: N_t) */
 int slamrs_gpu_get_weights(slamrs_gpu_handle* h, double* out_norm, double* out_raw);
-/* last step's resample source index for every new particle (N entries) and the stored argmax */
+/* last step's resample source index for every new particle (N entries; a localiser: M) and the stored argmax */
 int slamrs_gpu_get_resample_indices(slamrs_gpu_handle* h, uint32_t* out_idx);
 int slamrs_gpu_get_max_particle(slamrs_gpu_handle* h, uint64_t* out);
 /* one particle's grid as packed hit counters: low 16 bits = free updates, high 16 = occupied

@@ -111,6 +111,19 @@ pub struct slamrs_gpu_recovery {
     pub alpha_fast: f64,
 }
 
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_kld {
+    pub struct_size: u32,
+    pub n_min: u32,
+    pub n_max: u32,
+    pub pad: u32,
+    pub err: f64,
+    pub z: f64,
+    pub bin_cells: u32,
+    pub theta_bins: u32,
+}
+
 extern "C" {
     pub fn slamrs_gpu_grid_cells(extent: f32, resolution: f32, out_cells: *mut u32) -> c_int;
     pub fn slamrs_gpu_nccl_unique_id(out: *mut u8) -> c_int;
@@ -165,4 +178,7 @@ extern "C" {
     pub fn slamrs_gpu_get_scan_match_stats(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
     pub fn slamrs_gpu_set_recovery(h: *mut slamrs_gpu_handle, r: *const slamrs_gpu_recovery) -> c_int;
     pub fn slamrs_gpu_get_recovery_state(h: *mut slamrs_gpu_handle, out: *mut f64, out_injected: *mut u64) -> c_int;
+    pub fn slamrs_gpu_set_kld(h: *mut slamrs_gpu_handle, k: *const slamrs_gpu_kld) -> c_int;
+    pub fn slamrs_gpu_get_kld_state(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
+    pub fn slamrs_gpu_get_population(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
 }

@@ -38,6 +38,7 @@ EXPORTS = [
     "slamrs_gpu_create_localizer", "slamrs_gpu_get_sensor_terms",
     "slamrs_gpu_set_scan_match", "slamrs_gpu_get_scan_match_stats",
     "slamrs_gpu_set_recovery", "slamrs_gpu_get_recovery_state",
+    "slamrs_gpu_set_kld", "slamrs_gpu_get_kld_state", "slamrs_gpu_get_population",
 ]
 MAP_F64, MAP_F32, MAP_U8 = 0, 1, 2
 SENSOR_BEAM_ENDPOINT, SENSOR_LIKELIHOOD_FIELD = 0, 1
@@ -70,6 +71,11 @@ class ScanMatch(C.Structure):
 
 class Recovery(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("pad", C.c_uint32), ("alpha_slow", C.c_double), ("alpha_fast", C.c_double)]
+
+
+class Kld(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("n_min", C.c_uint32), ("n_max", C.c_uint32), ("pad", C.c_uint32),
+                ("err", C.c_double), ("z", C.c_double), ("bin_cells", C.c_uint32), ("theta_bins", C.c_uint32)]
 
 
 class Stats(C.Structure):
@@ -151,6 +157,9 @@ def load():
     L.slamrs_gpu_get_scan_match_stats.restype = i; L.slamrs_gpu_get_scan_match_stats.argtypes = [vp, vp]
     L.slamrs_gpu_set_recovery.restype = i; L.slamrs_gpu_set_recovery.argtypes = [vp, C.POINTER(Recovery)]
     L.slamrs_gpu_get_recovery_state.restype = i; L.slamrs_gpu_get_recovery_state.argtypes = [vp, vp, C.POINTER(u64)]
+    L.slamrs_gpu_set_kld.restype = i; L.slamrs_gpu_set_kld.argtypes = [vp, C.POINTER(Kld)]
+    L.slamrs_gpu_get_kld_state.restype = i; L.slamrs_gpu_get_kld_state.argtypes = [vp, vp]
+    L.slamrs_gpu_get_population.restype = i; L.slamrs_gpu_get_population.argtypes = [vp, C.POINTER(u64)]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
     L.slamrs_gpu_debug_resample_adaptive.restype = i

@@ -147,6 +147,17 @@ struct slamrs_gpu_handle {
     bool recovery_on = false;
     double alpha_slow = 0.0, alpha_fast = 0.0;
     bool recovery_last_step = false;       // the last issued step ran k_loc_recover
+    // generation sizes: the current generation (the localiser's population N), the particles the last step weighted
+    // (N_t) and the new particles it drew (M). A SLAM handle keeps n_local, n_total and n_total.
+    uint32_t pop = 0, pop_weighted = 0, pop_drawn = 0;
+    // KLD-sampling (slamrs_gpu_set_kld)
+    bool kld_on = false;
+    KldParams kld{};
+    uint32_t* d_kld = nullptr;         // k_loc_kld's header + bin bitmap, kld_alloc_words words
+    size_t kld_words = 0, kld_alloc_words = 0;   // words zeroed per step (current bins) / allocated
+    KldResult* h_kld = nullptr;        // page-locked: k_loc_kld's last CTA writes the step's result here
+    cudaEvent_t ev_kld = nullptr;      // behind k_loc_kld
+    KldResult kld_last{0ull, 0ull, 0ull};   // the last step's result (zero when it ran without KLD-sampling)
     // scan-matching pose refinement (slamrs_gpu_set_scan_match)
     bool match_on = false;
     ScanMatchParams match{};
@@ -305,6 +316,9 @@ void free_all(slamrs_gpu_handle* h) {
     cudaFree(h->d_slot[0]); cudaFree(h->d_slot[1]);
     cudaFree(h->d_pose[0]); cudaFree(h->d_pose[1]);
     cudaFree(h->d_term_table); cudaFree(h->d_loc_terms); cudaFree(h->d_loc_free); cudaFree(h->d_recovery);
+    cudaFree(h->d_kld);
+    if (h->h_kld) cudaFreeHost(h->h_kld);
+    if (h->ev_kld) cudaEventDestroy(h->ev_kld);
     cudaFree(h->d_wnorm); cudaFree(h->d_cum); cudaFree(h->d_idx); cudaFree(h->d_fold); cudaFree(h->d_carry);
     cudaFree(h->d_angle);   // (d_dist and d_valid live in the same allocation)
     if (h->h_scan_stage) cudaFreeHost(h->h_scan_stage);
@@ -455,7 +469,10 @@ int step_issued(slamrs_gpu_handle* h, int nxt) {
 
 // One localisation step (localiser mode): motion + likelihood against the term table, then the SLAM step's own
 // weights and resampling kernels without a survivor list -- three launches, chained by programmatic dependent launch,
-// and k_loc_recover as a fourth while recovery is on.
+// and k_loc_recover as a fourth while recovery is on. The step weights the pop = N_t particles of the current
+// generation and draws M new ones: the capacity n_total while KLD-sampling is off, else the size k_loc_kld computes
+// in front of k_loc_step from the bins of the current generation. The host waits for k_loc_kld (it finishes while
+// k_loc_step runs), so the launches behind k_weights get their size from the host.
 int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
     cudaStream_t s = h->stream;
     if (h->profiling && h->prof_recorded == PROF_RING) {
@@ -465,23 +482,41 @@ int loc_step_async(slamrs_gpu_handle* h, const OdomModel& od, bool caller) {
     const int cur = h->cur, nxt = cur ^ 1;
     const ScanDevice scan = h->scan_external ? ScanDevice{h->ext_angle, h->ext_dist, h->ext_valid, h->n_beams, nullptr}
                                              : ScanDevice{h->d_angle, h->d_dist, h->d_valid, h->n_beams, nullptr};
+    const uint32_t n = h->pop;
+    uint32_t m = h->n_total;
     PROF_MARK(h, 0);
-    launch_loc_step(s, h->geom, od, scan, h->d_pose[cur], h->d_results, h->n_total, caller ? h->d_z : nullptr, h->cfg.seed,
+    if (h->kld_on) {
+        CU_TRY(h, cudaMemsetAsync(h->d_kld, 0, sizeof(uint32_t) * h->kld_words, s));
+        launch_loc_kld(s, h->d_pose[cur], n, h->geom, h->kld, h->d_kld, h->h_kld);
+        CU_TRY(h, cudaEventRecord(h->ev_kld, s));
+        h->launches++;
+    }
+    launch_loc_step(s, h->geom, od, scan, h->d_pose[cur], h->d_results, n, caller ? h->d_z : nullptr, h->cfg.seed,
                     h->step, h->d_loc_terms, h->loc_outside, h->d_carry, h->d_counters);
     PROF_MARK(h, 1);
     PROF_MARK(h, 2);
-    launch_weights(s, h->d_results, h->n_total, h->d_wnorm, h->d_cum, h->d_fold, (double)h->cfg.resample_threshold, h->d_counters);
-    launch_resample_indices(s, h->d_results, h->d_cum, h->n_total, caller ? h->d_u : nullptr, h->cfg.seed, h->step, h->d_idx,
-                            h->d_pose[nxt], 0, h->n_total, false, nullptr,
+    launch_weights(s, h->d_results, n, h->d_wnorm, h->d_cum, h->d_fold, (double)h->cfg.resample_threshold, h->d_counters);
+    h->kld_last = KldResult{0ull, 0ull, 0ull};
+    if (h->kld_on) {
+        CU_TRY(h, cudaEventSynchronize(h->ev_kld));
+        const volatile KldResult* r = h->h_kld;
+        h->kld_last = KldResult{r->n_weighted, r->k, r->m};
+        m = (uint32_t)h->kld_last.m;
+    }
+    launch_resample_indices(s, h->d_results, h->d_cum, n, m, caller ? h->d_u : nullptr, h->cfg.seed, h->step, h->d_idx,
+                            h->d_pose[nxt], 0, m, false, nullptr,
                             RayLists{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u}, h->d_wnorm, h->d_carry,
                             h->d_counters);
     h->launches += 3;
     if (h->recovery_on) {
-        launch_loc_recover(s, h->n_total, h->d_counters, h->d_recovery, h->step, h->alpha_slow, h->alpha_fast, h->cfg.seed,
+        launch_loc_recover(s, n, m, h->d_counters, h->d_recovery, h->step, h->alpha_slow, h->alpha_fast, h->cfg.seed,
                            h->d_loc_free, h->n_free, h->geom, h->d_pose[nxt]);
         h->launches++;
     }
     h->recovery_last_step = h->recovery_on;
+    h->pop_weighted = n;
+    h->pop_drawn = m;
+    h->pop = m;
     for (uint32_t m = 3; m < PROF_MARKS; ++m) PROF_MARK(h, m);
     if (h->profiling) h->prof_stamped[h->prof_recorded++] = 0;
     CU_TRY(h, cudaGetLastError());
@@ -575,6 +610,8 @@ int slamrs_gpu_create(const slamrs_gpu_config* cfg, slamrs_gpu_handle** out) {
     h->n_total = (uint32_t)cfg->n_particles;
     h->n_local = h->n_total / h->world;
     h->first = h->rank * h->n_local;
+    h->pop = h->n_local;
+    h->pop_weighted = h->pop_drawn = h->n_total;
     h->n_cells = cfg->grid_w * cfg->grid_h;
     h->geom = make_map_geom(cfg->pos_x, cfg->pos_y, cfg->resolution, cfg->grid_w, cfg->grid_h, cfg->slot_cells);
     // a slot holds pw x ph cells: the whole grid, or (windowed slots) a power-of-two torus of it
@@ -804,6 +841,7 @@ int slamrs_gpu_create_localizer(const slamrs_gpu_config* cfg, const slamrs_gpu_s
     h->localizer = true;
     h->device = device;
     h->n_total = h->n_local = (uint32_t)cfg->n_particles;
+    h->pop = h->pop_weighted = h->pop_drawn = h->n_total;
     h->n_cells = (uint32_t)n_cells;
     h->geom = make_map_geom(cfg->pos_x, cfg->pos_y, cfg->resolution, cfg->grid_w, cfg->grid_h);
     h->loc_outside = field ? log((double)model->z_rand) : 0.0;   // ln(z_rand) / the reference's ln(1) for off-grid endpoints
@@ -929,6 +967,62 @@ int slamrs_gpu_get_recovery_state(slamrs_gpu_handle* h, double out[3], uint64_t*
     return SLAMRS_OK;
 }
 
+int slamrs_gpu_set_kld(slamrs_gpu_handle* h, const slamrs_gpu_kld* k) {
+    if (!h) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no KLD-sampling (only a localizer has one)");
+    if (!k) {
+        h->kld_on = false;
+        return SLAMRS_OK;
+    }
+    if (k->struct_size != sizeof(slamrs_gpu_kld)) return fail(h, SLAMRS_E_INVALID_ARG, "slamrs_gpu_kld struct_size mismatch");
+    if (h->cfg.resample_threshold > 0.0f)
+        return fail(h, SLAMRS_E_INVALID_ARG,
+                    "KLD-sampling needs resample_threshold 0 (carried weights assume a fixed population)");
+    if (!(k->n_min >= 1u && k->n_min <= k->n_max && k->n_max <= h->n_total))
+        return fail(h, SLAMRS_E_INVALID_ARG, "KLD n_min and n_max must satisfy 1 <= n_min <= n_max <= n_particles");
+    if (!(isfinite(k->err) && k->err > 0.0 && k->err <= 1.0))
+        return fail(h, SLAMRS_E_INVALID_ARG, "KLD err must be finite and lie in (0, 1]");
+    if (!(isfinite(k->z) && k->z >= 0.0)) return fail(h, SLAMRS_E_INVALID_ARG, "KLD z must be finite and >= 0");
+    if (k->bin_cells < 1u) return fail(h, SLAMRS_E_INVALID_ARG, "KLD bin_cells must be >= 1");
+    if (k->theta_bins < 1u || k->theta_bins > 3600u)
+        return fail(h, SLAMRS_E_INVALID_ARG, "KLD theta_bins must lie in 1..3600");
+    const uint64_t nb = ((uint64_t)h->geom.gw + k->bin_cells - 1u) / k->bin_cells;   // (square grid)
+    const uint64_t bits = nb * nb * k->theta_bins + 1u;                                // + the off-grid bin
+    if (bits > (1ull << 28))
+        return fail(h, SLAMRS_E_INVALID_ARG, "KLD bin bitmap above 2^28 bits: raise bin_cells or lower theta_bins");
+    const size_t words = KLD_HEADER_WORDS + (size_t)((bits + 31u) / 32u);
+    DeviceGuard g(h->device);
+    if (!h->h_kld) CU_TRY(h, cudaMallocHost(&h->h_kld, sizeof(KldResult)));
+    if (!h->ev_kld) CU_TRY(h, cudaEventCreateWithFlags(&h->ev_kld, cudaEventDisableTiming));
+    if (words > h->kld_alloc_words) {
+        CU_TRY(h, cudaStreamSynchronize(h->stream));   // no issued step still uses the old bitmap
+        cudaFree(h->d_kld);
+        h->d_kld = nullptr;
+        h->kld_alloc_words = 0;
+        CU_TRY(h, cudaMalloc(&h->d_kld, sizeof(uint32_t) * words));
+        h->kld_alloc_words = words;
+    }
+    h->kld = KldParams{k->n_min, k->n_max, k->err, k->z, k->bin_cells, k->theta_bins, (uint32_t)nb, (uint32_t)nb};
+    h->kld_words = words;
+    h->kld_on = true;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_get_kld_state(slamrs_gpu_handle* h, uint64_t out[3]) {
+    if (!h || !out) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no KLD-sampling (only a localizer has one)");
+    DeviceGuard g(h->device);
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    out[0] = h->kld_last.n_weighted; out[1] = h->kld_last.k; out[2] = h->kld_last.m;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_get_population(slamrs_gpu_handle* h, uint64_t* out) {
+    if (!h || !out) return SLAMRS_E_INVALID_ARG;
+    *out = h->pop;
+    return SLAMRS_OK;
+}
+
 int slamrs_gpu_set_scan_match(slamrs_gpu_handle* h, const slamrs_gpu_scan_match* m) {
     if (!h) return SLAMRS_E_INVALID_ARG;
     if (h->localizer) return fail(h, SLAMRS_E_INVALID_ARG, "a localizer does not scan-match");
@@ -1051,8 +1145,9 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     DeviceGuard g(h->device);
     cudaStream_t s = h->stream;
     const OdomModel od = odometry_new(dist_left, dist_right, wheel_dist);
-    if (caller) {
-        CU_TRY(h, cudaMemcpyAsync(h->d_z, z_draws, sizeof(double) * 2 * h->n_total, cudaMemcpyHostToDevice, s));
+    if (caller) {   // (a localiser draws for the particles of its current generation)
+        CU_TRY(h, cudaMemcpyAsync(h->d_z, z_draws, sizeof(double) * 2 * (h->localizer ? h->pop : h->n_total),
+                                  cudaMemcpyHostToDevice, s));
         CU_TRY(h, cudaMemcpyAsync(h->d_u, resample_u, sizeof(double), cudaMemcpyHostToDevice, s));
     }
     if (h->localizer) return loc_step_async(h, od, caller);
@@ -1141,7 +1236,7 @@ int slamrs_gpu_step_async(slamrs_gpu_handle* h, float dist_left, float dist_righ
     RayLists ray{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u};
     if (fuse) ray = RayLists{h->d_ray_items, h->d_ray_items + h->n_local, h->d_slot[cur], h->d_alias, h->d_readers, h->d_meta,
                              h->n_local, flag_pulls ? 1u : 0u};
-    launch_resample_indices(s, h->d_results, h->d_cum, h->n_total, caller ? h->d_u : nullptr, h->cfg.seed, h->step,
+    launch_resample_indices(s, h->d_results, h->d_cum, h->n_total, h->n_total, caller ? h->d_u : nullptr, h->cfg.seed, h->step,
                             h->d_idx, h->d_pose[nxt], h->first, h->n_local, !all_particles, h->d_alive, ray, h->d_wnorm, h->d_carry,
                             h->d_counters);
     if (all_particles) {
@@ -1546,7 +1641,7 @@ uint64_t slamrs_gpu_launch_count(const slamrs_gpu_handle* h) { return h ? h->lau
 int slamrs_gpu_get_poses(slamrs_gpu_handle* h, float* out_xyt) {
     if (!h || !out_xyt) return SLAMRS_E_INVALID_ARG;
     DeviceGuard g(h->device);
-    CU_TRY(h, cudaMemcpyAsync(out_xyt, h->d_pose[h->cur], sizeof(float) * 3 * h->n_local, cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(out_xyt, h->d_pose[h->cur], sizeof(float) * 3 * h->pop, cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     return SLAMRS_OK;
 }
@@ -1568,7 +1663,7 @@ int slamrs_gpu_init_uniform(slamrs_gpu_handle* h, const float box[4]) {
     if (!h || !box) return SLAMRS_E_INVALID_ARG;
     if (!(box[2] >= box[0] && box[3] >= box[1])) return fail(h, SLAMRS_E_INVALID_ARG, "empty box");
     DeviceGuard g(h->device);
-    launch_init_uniform(h->stream, h->cfg.seed, h->first, h->n_local, box[0], box[1], box[2], box[3], h->d_pose[h->cur]);
+    launch_init_uniform(h->stream, h->cfg.seed, h->first, h->pop, box[0], box[1], box[2], box[3], h->d_pose[h->cur]);
     h->launches++;
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     CU_TRY(h, cudaGetLastError());
@@ -1578,7 +1673,7 @@ int slamrs_gpu_init_uniform(slamrs_gpu_handle* h, const float box[4]) {
 int slamrs_gpu_set_poses(slamrs_gpu_handle* h, const float* xyt) {
     if (!h || !xyt) return SLAMRS_E_INVALID_ARG;
     DeviceGuard g(h->device);
-    CU_TRY(h, cudaMemcpyAsync(h->d_pose[h->cur], xyt, sizeof(float) * 3 * h->n_local, cudaMemcpyHostToDevice, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(h->d_pose[h->cur], xyt, sizeof(float) * 3 * h->pop, cudaMemcpyHostToDevice, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     return SLAMRS_OK;
 }
@@ -1587,10 +1682,10 @@ int slamrs_gpu_get_weights(slamrs_gpu_handle* h, double* out_norm, double* out_r
     if (!h) return SLAMRS_E_INVALID_ARG;
     DeviceGuard g(h->device);
     if (out_norm)
-        CU_TRY(h, cudaMemcpyAsync(out_norm, h->d_wnorm, sizeof(double) * h->n_total, cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(out_norm, h->d_wnorm, sizeof(double) * h->pop_weighted, cudaMemcpyDeviceToHost, h->stream));
     if (out_raw)
         CU_TRY(h, cudaMemcpy2DAsync(out_raw, sizeof(double), h->d_results, sizeof(ParticleResult), sizeof(double),
-                                    h->n_total, cudaMemcpyDeviceToHost, h->stream));
+                                    h->pop_weighted, cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     return SLAMRS_OK;
 }
@@ -1598,7 +1693,7 @@ int slamrs_gpu_get_weights(slamrs_gpu_handle* h, double* out_norm, double* out_r
 int slamrs_gpu_get_resample_indices(slamrs_gpu_handle* h, uint32_t* out_idx) {
     if (!h || !out_idx) return SLAMRS_E_INVALID_ARG;
     DeviceGuard g(h->device);
-    CU_TRY(h, cudaMemcpyAsync(out_idx, h->d_idx, sizeof(uint32_t) * h->n_total, cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(out_idx, h->d_idx, sizeof(uint32_t) * h->pop_drawn, cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     return SLAMRS_OK;
 }
@@ -1822,7 +1917,7 @@ int slamrs_gpu_debug_resample_adaptive(int device, const double* raw_weights, ui
         cudaEventRecord(ev[0], nullptr);
         launch_weights(nullptr, res.p, n, wn.p, cum.p, fold.p, tau, cnt.p);
         cudaEventRecord(ev[1], nullptr);
-        launch_resample_indices(nullptr, res.p, cum.p, n, u.p, 0, 0, idx.p, nullptr, 0, 0, false, nullptr,
+        launch_resample_indices(nullptr, res.p, cum.p, n, n, u.p, 0, 0, idx.p, nullptr, 0, 0, false, nullptr,
                                 RayLists{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0u, 0u}, wn.p, nullptr, cnt.p);
         cudaEventRecord(ev[2], nullptr);
         cudaError_t e = cudaDeviceSynchronize();

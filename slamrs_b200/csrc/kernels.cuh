@@ -17,6 +17,7 @@
 //                          k_loc_terms_beam / k_loc_dt_cols / k_loc_dt_rows   sensor-term table at create
 //                          k_loc_free_count / k_loc_free_scan / k_loc_free_cells   free-cell list at create
 //                          k_loc_recover   augmented-MCL recovery behind k_resample_indices (off by default)
+//                          k_loc_kld       KLD-sampling: bins of the starting generation and the next one's size (off by default)
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -238,8 +239,9 @@ void launch_weights(cudaStream_t stream, const ParticleResult* results, uint32_t
 size_t weights_scratch_doubles();
 int weights_trace(long long* out64);   // tuning builds (-DSLAMRS_FOLD_TRACE): clock stamps of the last k_weights
 
+// m_draws new particles from the n_total weights (the localiser's KLD-sampling; every other caller passes n_total)
 void launch_resample_indices(cudaStream_t stream, const ParticleResult* results, const double* cum,
-                             uint32_t n_total, const double* u01_caller, uint64_t seed, uint64_t step,
+                             uint32_t n_total, uint32_t m_draws, const double* u01_caller, uint64_t seed, uint64_t step,
                              uint32_t* idx, float* pose_next, uint32_t first_particle, uint32_t n_local,
                              bool build_alive /* also list the surviving local particles */,
                              uint32_t* alive_list, RayLists ray, const double* w_norm, double* carry /* may be null */,
@@ -375,10 +377,27 @@ struct RecoveryState {
     double w_slow, w_fast, p;       // the averages and the share of particles to replace
     unsigned long long injected;    // particles replaced in that step
 };
-// behind k_resample_indices: the new averages from counters->sum, then the injections into pose_next
-void launch_loc_recover(cudaStream_t stream, uint32_t n, const StepCounters* counters, RecoveryState* state, uint64_t step,
-                        double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells, uint32_t n_free,
-                        MapGeom geom, float* pose_next);
+// behind k_resample_indices: the new averages from counters->sum of the n weighted particles, then the injections into
+// the m_draws new poses of pose_next
+void launch_loc_recover(cudaStream_t stream, uint32_t n, uint32_t m_draws, const StepCounters* counters, RecoveryState* state,
+                        uint64_t step, double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells,
+                        uint32_t n_free, MapGeom geom, float* pose_next);
+// KLD-sampling of the localiser (slamrs_gpu_set_kld): the bins and the bound (nbx = nby = ceil(w / bin_cells))
+struct KldParams {
+    uint32_t n_min, n_max;
+    double err, z;
+    uint32_t bin_cells, theta_bins, nbx, nby;
+};
+// {particles weighted, occupied bins, particles to draw} of one step, written by k_loc_kld's last CTA
+struct KldResult {
+    unsigned long long n_weighted, k, m;
+};
+// k_loc_kld's state: [bin count, CTA ticket, padding] then the bitmap; all of it zeroed before every launch
+constexpr uint32_t KLD_HEADER_WORDS = 32;
+// in front of k_loc_step: the bins of the n poses of `pose` and the size of the next generation into *host_out
+// (page-locked host memory)
+void launch_loc_kld(cudaStream_t stream, const float* pose, uint32_t n, MapGeom geom, const KldParams& kp, uint32_t* state,
+                    KldResult* host_out);
 
 // test hooks
 void launch_debug_raycast(cudaStream_t stream, const float* x0, const float* y0, const float* x1, const float* y1,

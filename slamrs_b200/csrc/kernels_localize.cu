@@ -1,7 +1,8 @@
 // Monte Carlo localisation against one shared, read-only occupancy map: the per-cell sensor-term table built once
 // at create (k_loc_terms_beam, or k_loc_dt_cols + k_loc_dt_rows for the likelihood field) and the per-step kernel
 // k_loc_step (motion + likelihood, fused). k_weights and k_resample_indices run unchanged behind it, and with
-// recovery on (slamrs_gpu_set_recovery) k_loc_recover behind them, on the free-cell list built at create.
+// recovery on (slamrs_gpu_set_recovery) k_loc_recover behind them, on the free-cell list built at create. With
+// KLD-sampling on (slamrs_gpu_set_kld) k_loc_kld runs in front of k_loc_step and sizes the next generation.
 #include "kernels_common.cuh"
 
 namespace slamrs {
@@ -231,10 +232,12 @@ void launch_loc_free_cells(cudaStream_t stream, const double* prob, size_t n_cel
 // step. With p > 0 a thread draws its particle's decision (slamrs_stream::recovery_draw) and replaces the resampled
 // pose; each warp adds its injections to the count with one atomic. The estimate, the indices and the weights that
 // k_weights and k_resample_indices recorded stay as they are.
+// n particles were weighted (w_avg = sum / n) and m new ones drawn (the injection candidates); m = n unless KLD-sampling
+// sized the new generation.
 __global__ void __launch_bounds__(256)
-k_loc_recover(uint32_t n, const StepCounters* __restrict__ counters, RecoveryState* state, uint64_t step, double alpha_slow,
-              double alpha_fast, uint64_t seed, const uint32_t* __restrict__ free_cells, uint32_t n_free, uint32_t grid_h,
-              double pos_x, double pos_y, double res, float* __restrict__ pose_next) {
+k_loc_recover(uint32_t n, uint32_t m_draws, const StepCounters* __restrict__ counters, RecoveryState* state, uint64_t step,
+              double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* __restrict__ free_cells, uint32_t n_free,
+              uint32_t grid_h, double pos_x, double pos_y, double res, float* __restrict__ pose_next) {
     pdl_wait();   // k_resample_indices has completed (it waited for k_weights): counters->sum, the resampled poses
     RecoveryState* prev = state + ((step + 1u) & 1u);
     RecoveryState* cur = state + (step & 1u);
@@ -247,7 +250,7 @@ k_loc_recover(uint32_t n, const StepCounters* __restrict__ counters, RecoverySta
     }
     if (!(p > 0.0)) return;   // (grid-uniform)
     float x, y, t;
-    const bool inj = m < n && slamrs_stream::recovery_draw(seed, step, m, p, free_cells, n_free, grid_h, pos_x, pos_y, res,
+    const bool inj = m < m_draws && slamrs_stream::recovery_draw(seed, step, m, p, free_cells, n_free, grid_h, pos_x, pos_y, res,
                                                            &x, &y, &t);
     const unsigned mask = __ballot_sync(0xffffffffu, inj);
     if (inj) {
@@ -257,11 +260,84 @@ k_loc_recover(uint32_t n, const StepCounters* __restrict__ counters, RecoverySta
     if ((threadIdx.x & 31u) == 0 && mask) atomicAdd(&cur->injected, (unsigned long long)__popc(mask));
 }
 
-void launch_loc_recover(cudaStream_t stream, uint32_t n, const StepCounters* counters, RecoveryState* state, uint64_t step,
-                        double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells, uint32_t n_free,
-                        MapGeom geom, float* pose_next) {
-    launch_pdl(k_loc_recover, dim3((n + 255u) / 256u), dim3(256), 0, stream, n, counters, state, step, alpha_slow, alpha_fast,
-               seed, free_cells, n_free, geom.gh, (double)geom.pos_x, (double)geom.pos_y, (double)geom.res, pose_next);
+void launch_loc_recover(cudaStream_t stream, uint32_t n, uint32_t m_draws, const StepCounters* counters, RecoveryState* state,
+                        uint64_t step, double alpha_slow, double alpha_fast, uint64_t seed, const uint32_t* free_cells,
+                        uint32_t n_free, MapGeom geom, float* pose_next) {
+    launch_pdl(k_loc_recover, dim3((m_draws + 255u) / 256u), dim3(256), 0, stream, n, m_draws, counters, state, step, alpha_slow,
+               alpha_fast, seed, free_cells, n_free, geom.gh, (double)geom.pos_x, (double)geom.pos_y, (double)geom.res, pose_next);
+}
+
+// =============================================================================== KLD-sampling (adaptive population)
+// The bin of a pose: the cell the likelihood would give a beam endpoint at (x, y), coarsened to bin_cells x bin_cells
+// cells, times theta_bins headings; every pose off the grid shares the one bin nbx * nby * theta_bins.
+constexpr double KLD_TWO_PI = 0x1.921fb54442d18p+2;
+
+__device__ __forceinline__ uint32_t kld_bin(float x, float y, float theta, const MapGeom& geom, const KldParams& kp) {
+    const float gx = world_to_grid(x, geom.pos_x, geom.res);
+    const float gy = world_to_grid(y, geom.pos_y, geom.res);
+    if (!grid_is_valid(gx, gy, geom.gw, geom.gh)) return kp.nbx * kp.nby * kp.theta_bins;
+    const uint32_t cx = (uint32_t)f32_as_usize(gx), cy = (uint32_t)f32_as_usize(gy);
+    double t = fmod((double)theta, KLD_TWO_PI);   // (exact)
+    if (t < 0.0) t = __dadd_rn(t, KLD_TWO_PI);
+    uint32_t hb = 0;   // NaN / infinite headings, and a negative one that rounds up to 2 pi, fall into heading bin 0
+    if (t >= 0.0 && t < KLD_TWO_PI)
+        hb = min(kp.theta_bins - 1u, (uint32_t)__ddiv_rn(__dmul_rn(t, (double)kp.theta_bins), KLD_TWO_PI));
+    return ((cy / kp.bin_cells) * kp.nbx + cx / kp.bin_cells) * kp.theta_bins + hb;
+}
+
+// The particle count of the next generation for k occupied bins: AMCL's pf_resample_limit in its order of operations
+// (n_min instead of max_particles for k <= 1).
+__device__ __forceinline__ uint32_t kld_bound(uint32_t k, const KldParams& kp) {
+    if (k <= 1u) return kp.n_min;
+    const double km1 = (double)(k - 1u);
+    const double b = __ddiv_rn(2.0, __dmul_rn(9.0, km1));
+    const double x = __dadd_rn(__dsub_rn(1.0, b), __dmul_rn(__dsqrt_rn(b), kp.z));
+    const double n = __dmul_rn(__dmul_rn(__dmul_rn(__ddiv_rn(km1, __dmul_rn(2.0, kp.err)), x), x), x);
+    if (!(n < (double)kp.n_max)) return kp.n_max;   // (also NaN and infinity)
+    const double c = ceil(n);
+    return c < (double)kp.n_min ? kp.n_min : (uint32_t)c;
+}
+
+// One thread per pose of the starting generation: marks its bin in the bitmap (state + KLD_HEADER_WORDS, zeroed with the
+// header before the launch) and each warp adds the bits it set first to state[0]. The last CTA to finish (ticket
+// state[1]) evaluates the bound and leaves {n, k, N_next} in the host's page-locked result. A converged cloud puts
+// nearly every pose into a few bins: only one lane per distinct bin of a warp touches the bitmap, and it reads the word
+// before its atomicOr, so only the first warps to reach a bin contend for that word.
+__global__ void __launch_bounds__(256)
+k_loc_kld(const float* __restrict__ pose, uint32_t n, MapGeom geom, KldParams kp, uint32_t* state, KldResult* host_out) {
+    __shared__ bool s_last;
+    uint32_t* bits = state + KLD_HEADER_WORDS;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t b = 0xffffffffu;   // (no bin: bins stay below 2^28)
+    if (i < n) {
+        const float* q = pose + 3 * (size_t)i;
+        b = kld_bin(q[0], q[1], q[2], geom, kp);
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, b);
+    bool fresh = false;
+    if (i < n && (threadIdx.x & 31u) == (unsigned)(__ffs(peers) - 1)) {
+        const uint32_t bit = 1u << (b & 31u);
+        uint32_t* w = &bits[b >> 5];
+        if ((*(volatile const uint32_t*)w & bit) == 0u) fresh = (atomicOr(w, bit) & bit) == 0u;
+    }
+    const unsigned mask = __ballot_sync(0xffffffffu, fresh);
+    if ((threadIdx.x & 31u) == 0 && mask) atomicAdd(&state[0], (uint32_t)__popc(mask));
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = atomicAdd(&state[1], 1u) == gridDim.x - 1u;
+    __syncthreads();
+    if (!s_last || threadIdx.x != 0) return;
+    __threadfence();
+    const uint32_t k = atomicAdd(&state[0], 0u);
+    host_out->n_weighted = n;
+    host_out->k = k;
+    host_out->m = kld_bound(k, kp);
+    __threadfence_system();
+}
+
+void launch_loc_kld(cudaStream_t stream, const float* pose, uint32_t n, MapGeom geom, const KldParams& kp, uint32_t* state,
+                    KldResult* host_out) {
+    k_loc_kld<<<(n + 255u) / 256u, 256, 0, stream>>>(pose, n, geom, kp, state, host_out);
 }
 
 }  // namespace slamrs

@@ -644,9 +644,9 @@ int weights_trace(long long* out64) {
 
 // =============================================================================== k_resample_indices
 
-// u_m of particle.rs:84, 89 for the zero-based new-particle index m0
-__device__ __forceinline__ double resample_threshold(uint32_t n, double U, uint32_t m0) {
-    const double num = (double)n;
+// u_m of particle.rs:84, 89 for the zero-based new-particle index m0 of m_draws draws (N wherever N counts draws)
+__device__ __forceinline__ double resample_threshold(uint32_t m_draws, double U, uint32_t m0) {
+    const double num = (double)m_draws;
     const double r = __ddiv_rn(__dmul_rn(U, 1.0), num);   // particle.rs:84: r = rand::random::<f64>() * 1.0 / N
     // particle.rs:89: u = r + (m as f64 - 1.0) * 1.0 / N with m = m0 + 1
     return __dadd_rn(r, __ddiv_rn(__dmul_rn(__dsub_rn((double)(m0 + 1u), 1.0), 1.0), num));
@@ -677,8 +677,11 @@ constexpr uint32_t RS_COARSE = 2048;
 // into the fused ray update's work lists (kernels_ray.cu): a clone (grid still an alias of its source's
 // slot) is listed in ray.clones, counts itself as a reader of its root and becomes private; a particle
 // that owns its slot is listed in ray.owners.
+// m draws from the n weights (the localiser's KLD-sampling draws m != n; every other caller passes m = n): the
+// thresholds step by 1/m, the walk and its clamp stay on the n running sums, and the estimate is new particle
+// floor(max_particle * m / n), the same cumulative-mass position (max_particle itself when m = n).
 __global__ void __launch_bounds__(256)
-k_resample_indices(const ParticleResult* __restrict__ results, const double* __restrict__ cum, uint32_t n,
+k_resample_indices(const ParticleResult* __restrict__ results, const double* __restrict__ cum, uint32_t n, uint32_t m,
                    const double* __restrict__ u01_caller, uint64_t seed, uint64_t step, uint32_t* __restrict__ idx,
                    float* __restrict__ pose_next, uint32_t first_particle, uint32_t n_local, bool build_alive,
                    uint32_t* __restrict__ alive_list, RayLists ray, const double* __restrict__ w_norm,
@@ -693,8 +696,8 @@ k_resample_indices(const ParticleResult* __restrict__ results, const double* __r
     const uint32_t m0 = blockIdx.x * blockDim.x + threadIdx.x;  // zero-based new-particle index
     const double U = u01_caller ? *u01_caller : slamrs_stream::resample_uniform(seed, step);
     const int lane = threadIdx.x & 31;
-    auto source_of = [&](uint32_t m, bool* ran_off) {
-        const double u = resample_threshold(n, U, m);
+    auto source_of = [&](uint32_t j, bool* ran_off) {
+        const double u = resample_threshold(m, U, j);
         const uint32_t blk = first_not_below(s_coarse, 0u, n_coarse, u);
         *ran_off = blk >= n_coarse;   // the reference would index out of bounds and panic; clamp and flag
         if (blk >= n_coarse) return n - 1u;
@@ -702,7 +705,7 @@ k_resample_indices(const ParticleResult* __restrict__ results, const double* __r
     };
     bool ran_off = false;
     uint32_t src_idx = 0xffffffffu;
-    if (m0 < n) {
+    if (m0 < m) {
         if (resample) src_idx = source_of(m0, &ran_off); else src_idx = m0;
         if (carry != nullptr) carry[m0] = w_norm[m0];     // read by the next update only if this one did not resample
         if (m0 == 0u) counters->carry_active = resample ? 0ull : 1ull;
@@ -714,17 +717,18 @@ k_resample_indices(const ParticleResult* __restrict__ results, const double* __r
             q[0] = src.x; q[1] = src.y; q[2] = src.theta;
         }
         // estimated_pose(), slam.rs:77-81: new generation indexed by the pre-resample argmax
-        if ((unsigned long long)m0 == counters->max_particle) {
+        const unsigned long long mp = counters->max_particle;
+        if ((unsigned long long)m0 == (m == n ? mp : mp * m / n)) {
             counters->est_pose[0] = src.x; counters->est_pose[1] = src.y; counters->est_pose[2] = src.theta;
         }
     }
     if (!build_alive) return;   // uniform over the grid
     uint32_t prev = __shfl_up_sync(0xffffffffu, src_idx, 1);
-    if (lane == 0 && m0 > 0 && m0 < n) {
+    if (lane == 0 && m0 > 0 && m0 < m) {
         bool dummy;
         prev = resample ? source_of(m0 - 1u, &dummy) : m0 - 1u;
     }
-    const bool alive = m0 < n && (m0 == 0 || prev != src_idx) && src_idx >= first_particle &&
+    const bool alive = m0 < m && (m0 == 0 || prev != src_idx) && src_idx >= first_particle &&
                        src_idx < first_particle + n_local;
     // warp-aggregated appends (order is irrelevant: particles are independent)
     if (ray.clones == nullptr) {
@@ -746,7 +750,7 @@ k_resample_indices(const ParticleResult* __restrict__ results, const double* __r
         // itself, or the run of selectors reaches past the end of this rank's range.
         const uint32_t end = first_particle + n_local;
         remote = !(m0 >= first_particle && m0 < end);
-        if (!remote && end < n) {
+        if (!remote && end < m) {
             bool dummy;
             remote = (resample ? source_of(end, &dummy) : end) == src_idx;
         }
@@ -796,11 +800,11 @@ k_resample_indices(const ParticleResult* __restrict__ results, const double* __r
 }
 
 void launch_resample_indices(cudaStream_t stream, const ParticleResult* results, const double* cum,
-                             uint32_t n_total, const double* u01_caller, uint64_t seed, uint64_t step,
+                             uint32_t n_total, uint32_t m_draws, const double* u01_caller, uint64_t seed, uint64_t step,
                              uint32_t* idx, float* pose_next, uint32_t first_particle, uint32_t n_local,
                              bool build_alive, uint32_t* alive_list, RayLists ray, const double* w_norm, double* carry,
                              StepCounters* counters) {
-    launch_pdl(k_resample_indices, dim3((n_total + 255) / 256), dim3(256), 0, stream, results, cum, n_total, u01_caller, seed, step, idx,
+    launch_pdl(k_resample_indices, dim3((m_draws + 255) / 256), dim3(256), 0, stream, results, cum, n_total, m_draws, u01_caller, seed, step, idx,
                pose_next, first_particle, n_local, build_alive, alive_list, ray, w_norm, carry, counters);
 }
 

@@ -159,6 +159,34 @@ class Recovery:
         return r
 
 
+@dataclass
+class Kld:
+    """Adaptive population of a GridMapLocalizer: KLD-sampling (Fox 2003; slamrs_gpu_kld, ROS AMCL's min_particles /
+    max_particles / kld_err / kld_z). Each step draws as many particles as the spread of the cloud it starts from needs:
+    with k distinct bins occupied (cells of bin_xy metres, theta_bins headings), N = (k - 1) / (2 err) * (1 - b +
+    sqrt(b) z)^3 with b = 2 / (9 (k - 1)), clamped to [n_min, n_max] (n_min for k <= 1). n_max None is the capacity
+    (the config's n_particles). z is the upper (1 - delta) quantile of the standard normal: 2.326 for delta = 0.01.
+    ROS AMCL passes its kld_z parameter (default 0.99) where z belongs, which draws about 0.6x as many particles for
+    small k; pass z=0.99 to match its populations."""
+    n_min: int = 256
+    n_max: Optional[int] = None
+    err: float = 0.01
+    z: float = 2.326
+    bin_xy: float = 0.5        # metres; bin_cells = max(1, round(bin_xy / resolution))
+    theta_bins: int = 36
+
+    def bin_cells(self, resolution: float) -> int:
+        return max(1, int(round(self.bin_xy / resolution)))
+
+    def to_struct(self, capacity: int, resolution: float):
+        k = _lib.Kld()
+        k.struct_size = C.sizeof(_lib.Kld)
+        k.n_min, k.n_max = int(self.n_min), int(capacity if self.n_max is None else self.n_max)
+        k.err, k.z = float(self.err), float(self.z)
+        k.bin_cells, k.theta_bins = self.bin_cells(resolution), int(self.theta_bins)
+        return k
+
+
 def grid_cells(extent: float, resolution: float) -> int:
     """Map::new grid sizing (map.rs:28-31) as the library computes it."""
     out = C.c_uint32(0)
@@ -515,6 +543,7 @@ class GridMapLocalizer(GridMapSlam):
         self._map = np.ascontiguousarray(data, np.float64).reshape(-1)
         self.model = model or SensorModel()
         super().__init__(config, placement)
+        self._n_weighted = self.n_particles   # the particles the last step weighted (weights() reads that many)
 
     def _create(self, cfg) -> None:
         if self._map.size != cfg.grid_w * cfg.grid_h:
@@ -540,6 +569,68 @@ class GridMapLocalizer(GridMapSlam):
         out = np.zeros(3, np.float64); k = C.c_uint64(0)
         _lib.check(self._L.slamrs_gpu_get_recovery_state(self._h, _ptr(out), C.byref(k)), self._h)
         return {"w_slow": float(out[0]), "w_fast": float(out[1]), "p_inject": float(out[2]), "injected": int(k.value)}
+
+    # ------------------------------------------------------------------ adaptive population (KLD-sampling)
+    # n_particles is the capacity. The population (the current generation's size) starts there and changes only in a
+    # step: poses / set_poses / init_uniform use it, weights the size the last step weighted, resample_indices the
+    # size it drew (the population after it), and caller-mode z_draws holds 2 * population normals.
+    def set_kld(self, kld: Optional[Kld]) -> None:
+        """KLD-sampling from the next update on; None turns it off (the default): the next update then draws
+        n_particles particles, and every later one is the fixed-size step. Needs resample_threshold 0."""
+        k = None if kld is None else kld.to_struct(self.n_particles, self.config.resolution)
+        _lib.check(self._L.slamrs_gpu_set_kld(self._h, None if k is None else C.byref(k)), self._h)
+
+    def kld_state(self) -> dict:
+        """Of the last update: n_weighted (the particles it weighted), k (the bins they occupied) and n_drawn (the
+        particles it drew); all zero when it ran without KLD-sampling. Synchronises."""
+        out = np.zeros(3, np.uint64)
+        _lib.check(self._L.slamrs_gpu_get_kld_state(self._h, _ptr(out)), self._h)
+        return dict(zip(("n_weighted", "k", "n_drawn"), (int(v) for v in out)))
+
+    @property
+    def population(self) -> int:
+        out = C.c_uint64(0)
+        _lib.check(self._L.slamrs_gpu_get_population(self._h, C.byref(out)), self._h)
+        return int(out.value)
+
+    def update(self, z: Observation, u: Odometry, z_draws: Optional[np.ndarray] = None,
+               resample_u: Optional[float] = None) -> None:
+        angle, dist, valid = self._scan_arrays(z)
+        n = self.population
+        zd = None if z_draws is None else np.ascontiguousarray(z_draws, np.float64)
+        if zd is not None and zd.size != 2 * n:
+            raise ValueError("z_draws must hold 2 * population values")
+        ru = None if resample_u is None else np.array([resample_u], np.float64)
+        _lib.check(self._L.slamrs_gpu_update(self._h, _ptr(angle), _ptr(dist), _ptr(valid), angle.size,
+                                             u.distance_left, u.distance_right, u.wheel_distance,
+                                             _ptr(zd), _ptr(ru)), self._h)
+        self._n_weighted = n
+
+    def step_async(self, u: Odometry, z_draws: Optional[np.ndarray] = None, resample_u: Optional[float] = None) -> None:
+        n = self.population
+        if z_draws is not None and np.asarray(z_draws).size != 2 * n:
+            raise ValueError("z_draws must hold 2 * population values")
+        super().step_async(u, z_draws, resample_u)
+        self._n_weighted = n
+
+    def poses(self) -> np.ndarray:
+        out = np.zeros((self.population, 3), np.float32)
+        _lib.check(self._L.slamrs_gpu_get_poses(self._h, _ptr(out)), self._h)
+        return out
+
+    def set_poses(self, xyt) -> None:
+        a = np.ascontiguousarray(xyt, np.float32).reshape(self.population, 3)
+        _lib.check(self._L.slamrs_gpu_set_poses(self._h, _ptr(a)), self._h)
+
+    def weights(self):
+        norm = np.zeros(self._n_weighted, np.float64); raw = np.zeros(self._n_weighted, np.float64)
+        _lib.check(self._L.slamrs_gpu_get_weights(self._h, _ptr(norm), _ptr(raw)), self._h)
+        return norm, raw
+
+    def resample_indices(self) -> np.ndarray:
+        out = np.zeros(self.population, np.uint32)
+        _lib.check(self._L.slamrs_gpu_get_resample_indices(self._h, _ptr(out)), self._h)
+        return out
 
 
 # ---------------------------------------------------------------------- kernel-level hooks
