@@ -397,6 +397,58 @@ int slamrs_gpu_get_kld_state(slamrs_gpu_handle* h, uint64_t out[3]);
  * handle's n_local. */
 int slamrs_gpu_get_population(slamrs_gpu_handle* h, uint64_t* out);
 
+/* Pose hypotheses: clusters of the localiser's current generation with their mean and covariance (ROS AMCL's
+ * pf_cluster_stats and the estimate it publishes). Computed on the device on request; DESIGN.md section 11.3.
+ *   1. Input: the N poses get_poses returns (the previous step's resampled, injected set, or what init_uniform /
+ *      set_poses left), each of weight 1/N. The call is enqueued behind any step_async and synchronises once. It
+ *      changes no filter state: poses, weights, indices, estimate, recovery and KLD state, and the launches of the
+ *      steps are those of a handle that never calls it.
+ *   2. A pose is excluded if any of x, y, theta is not finite or its cell is off the grid (the likelihood's is_valid);
+ *      excluded poses are counted in n_excluded and belong to no cluster and not to `overall`.
+ *   3. A pose's bin is KLD-sampling's (slamrs_gpu_set_kld, item 1) with these bin_cells and theta_bins:
+ *      ((row / bin_cells) * nbx + column / bin_cells) * theta_bins + h.
+ *   4. Two occupied bins are adjacent when their (bx, by) differ by at most 1 each and their heading bins differ by at
+ *      most 1 modulo theta_bins (AMCL's 3x3x3 neighbourhood, except that the heading wraps: a cloud facing +-pi is one
+ *      cluster). A cluster is a connected component of occupied bins; its label is the smallest bin id in it.
+ *   5. Clusters are ranked by count (descending), then label (ascending); out_clusters[0, min(K, n_clusters)) receives
+ *      the first ones, the rest of its K entries are zeroed. Entry 0 is the estimate AMCL publishes.
+ *   6. Moments of each reported cluster and of `overall`, in f64 from the widened f32 coordinates: mean x, y = sums /
+ *      count; S = sum sin(theta), C = sum cos(theta); mean theta = atan2(S, C); var_theta = -2 ln(sqrt(S^2 + C^2) /
+ *      count). The covariance is centred, in a second pass over the poses: cov_xy = sum (x - mean x)(y - mean y) / count
+ *      (AMCL computes E[xy] - E[x]E[y] in one pass). No theta-x or theta-y covariance, as in AMCL. A set without poses
+ *      (every pose excluded) reports all zeros.
+ *   7. The integer outputs (n_bins, n_clusters, counts, labels, order) are exact; the f64 moments are sums folded in a
+ *      fixed order (no floating-point atomics), so every call on the same poses returns the same bits.
+ * Returns SLAMRS_E_INVALID_ARG on a SLAM handle, for a NULL c, out or out_clusters, for fields outside the ranges
+ * below, for a bin space nbx * nby * theta_bins above 2^28 and on a struct_size mismatch. The device scratch (about
+ * 17 bytes per particle of capacity plus 2 bits per bin, at most) is allocated by the first call and kept until destroy. */
+typedef struct slamrs_gpu_clustering {
+    uint32_t struct_size;   /* = sizeof(slamrs_gpu_clustering) */
+    uint32_t bin_cells;     /* >= 1: grid cells per bin side */
+    uint32_t theta_bins;    /* 1..3600 */
+    uint32_t max_clusters;  /* K, 1..64: clusters reported */
+} slamrs_gpu_clustering;
+
+typedef struct slamrs_gpu_pose_cluster {
+    uint64_t count;          /* poses in the cluster */
+    uint64_t label;          /* smallest bin id in the cluster */
+    double weight;           /* count / N */
+    double mean[3];          /* x, y (m), theta = atan2(S, C) in (-pi, pi] */
+    double cov_xx, cov_xy, cov_yy;  /* centred, divided by count */
+    double var_theta;        /* -2 ln(R), R = sqrt(S^2 + C^2) / count (AMCL's cov[2][2]) */
+} slamrs_gpu_pose_cluster;
+
+typedef struct slamrs_gpu_pose_stats {
+    uint64_t n_poses;        /* N, the current generation */
+    uint64_t n_excluded;     /* off the grid or a non-finite component */
+    uint64_t n_bins;         /* distinct occupied bins */
+    uint64_t n_clusters;     /* all clusters, not only the K reported */
+    slamrs_gpu_pose_cluster overall;  /* every non-excluded pose as one set (label 0) */
+} slamrs_gpu_pose_stats;
+
+int slamrs_gpu_pose_clusters(slamrs_gpu_handle* h, const slamrs_gpu_clustering* c, slamrs_gpu_pose_stats* out,
+                             slamrs_gpu_pose_cluster* out_clusters /* K entries */);
+
 /* ------------------------------------------------------------------ introspection (tests, bench) */
 
 const char* slamrs_gpu_last_error(const slamrs_gpu_handle* h); /* never NULL; "" when none */

@@ -124,6 +124,38 @@ pub struct slamrs_gpu_kld {
     pub theta_bins: u32,
 }
 
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_clustering {
+    pub struct_size: u32,
+    pub bin_cells: u32,
+    pub theta_bins: u32,
+    pub max_clusters: u32,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_pose_cluster {
+    pub count: u64,
+    pub label: u64,
+    pub weight: f64,
+    pub mean: [f64; 3],
+    pub cov_xx: f64,
+    pub cov_xy: f64,
+    pub cov_yy: f64,
+    pub var_theta: f64,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct slamrs_gpu_pose_stats {
+    pub n_poses: u64,
+    pub n_excluded: u64,
+    pub n_bins: u64,
+    pub n_clusters: u64,
+    pub overall: slamrs_gpu_pose_cluster,
+}
+
 extern "C" {
     pub fn slamrs_gpu_grid_cells(extent: f32, resolution: f32, out_cells: *mut u32) -> c_int;
     pub fn slamrs_gpu_nccl_unique_id(out: *mut u8) -> c_int;
@@ -181,4 +213,5 @@ extern "C" {
     pub fn slamrs_gpu_set_kld(h: *mut slamrs_gpu_handle, k: *const slamrs_gpu_kld) -> c_int;
     pub fn slamrs_gpu_get_kld_state(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
     pub fn slamrs_gpu_get_population(h: *mut slamrs_gpu_handle, out: *mut u64) -> c_int;
+    pub fn slamrs_gpu_pose_clusters(h: *mut slamrs_gpu_handle, c: *const slamrs_gpu_clustering, out: *mut slamrs_gpu_pose_stats, out_clusters: *mut slamrs_gpu_pose_cluster) -> c_int;
 }

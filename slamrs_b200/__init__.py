@@ -4,8 +4,8 @@ The compute path is libslamrs_gpu.so (hand-written sm_100a CUDA behind include/s
 This package is the host-side mirror of the reference interface plus the synthetic-input
 generator. Importing it never falls back to a CPU implementation.
 """
-from .slam import (GpuPlacement, GridData, GridMapLocalizer, GridMapSlam, GridMapSlamConfig, Kld, Measurement, Observation,
+from .slam import (Clustering, GpuPlacement, GridData, GridMapLocalizer, GridMapSlam, GridMapSlamConfig, Kld, Measurement, Observation,
                    Odometry, Pose, Recovery, ScanMatcher, SensorModel, grid_cells, nccl_unique_id)
 
-__all__ = ["GpuPlacement", "GridData", "GridMapLocalizer", "GridMapSlam", "GridMapSlamConfig", "Kld", "Measurement",
+__all__ = ["Clustering", "GpuPlacement", "GridData", "GridMapLocalizer", "GridMapSlam", "GridMapSlamConfig", "Kld", "Measurement",
            "Observation", "Odometry", "Pose", "Recovery", "ScanMatcher", "SensorModel", "grid_cells", "nccl_unique_id"]

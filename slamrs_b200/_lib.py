@@ -39,6 +39,7 @@ EXPORTS = [
     "slamrs_gpu_set_scan_match", "slamrs_gpu_get_scan_match_stats",
     "slamrs_gpu_set_recovery", "slamrs_gpu_get_recovery_state",
     "slamrs_gpu_set_kld", "slamrs_gpu_get_kld_state", "slamrs_gpu_get_population",
+    "slamrs_gpu_pose_clusters",
 ]
 MAP_F64, MAP_F32, MAP_U8 = 0, 1, 2
 SENSOR_BEAM_ENDPOINT, SENSOR_LIKELIHOOD_FIELD = 0, 1
@@ -76,6 +77,21 @@ class Recovery(C.Structure):
 class Kld(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("n_min", C.c_uint32), ("n_max", C.c_uint32), ("pad", C.c_uint32),
                 ("err", C.c_double), ("z", C.c_double), ("bin_cells", C.c_uint32), ("theta_bins", C.c_uint32)]
+
+
+class Clustering(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("bin_cells", C.c_uint32), ("theta_bins", C.c_uint32),
+                ("max_clusters", C.c_uint32)]
+
+
+class PoseCluster(C.Structure):
+    _fields_ = [("count", C.c_uint64), ("label", C.c_uint64), ("weight", C.c_double), ("mean", C.c_double * 3),
+                ("cov_xx", C.c_double), ("cov_xy", C.c_double), ("cov_yy", C.c_double), ("var_theta", C.c_double)]
+
+
+class PoseStats(C.Structure):
+    _fields_ = [("n_poses", C.c_uint64), ("n_excluded", C.c_uint64), ("n_bins", C.c_uint64), ("n_clusters", C.c_uint64),
+                ("overall", PoseCluster)]
 
 
 class Stats(C.Structure):
@@ -160,6 +176,8 @@ def load():
     L.slamrs_gpu_set_kld.restype = i; L.slamrs_gpu_set_kld.argtypes = [vp, C.POINTER(Kld)]
     L.slamrs_gpu_get_kld_state.restype = i; L.slamrs_gpu_get_kld_state.argtypes = [vp, vp]
     L.slamrs_gpu_get_population.restype = i; L.slamrs_gpu_get_population.argtypes = [vp, C.POINTER(u64)]
+    L.slamrs_gpu_pose_clusters.restype = i
+    L.slamrs_gpu_pose_clusters.argtypes = [vp, C.POINTER(Clustering), C.POINTER(PoseStats), vp]
     L.slamrs_gpu_debug_resample.restype = i
     L.slamrs_gpu_debug_resample.argtypes = [i, vp, u32, C.c_double, vp, C.POINTER(u64), vp, vp, vp, vp]
     L.slamrs_gpu_debug_resample_adaptive.restype = i

@@ -158,6 +158,10 @@ struct slamrs_gpu_handle {
     KldResult* h_kld = nullptr;        // page-locked: k_loc_kld's last CTA writes the step's result here
     cudaEvent_t ev_kld = nullptr;      // behind k_loc_kld
     KldResult kld_last{0ull, 0ull, 0ull};   // the last step's result (zero when it ran without KLD-sampling)
+    // pose clusters (slamrs_gpu_pose_clusters): device scratch allocated by the first call, grown when a call needs more
+    void* d_cl = nullptr;
+    size_t cl_bytes = 0;
+    ClusterOutput* h_cl = nullptr;     // page-locked: the last kernel leaves the result here
     // scan-matching pose refinement (slamrs_gpu_set_scan_match)
     bool match_on = false;
     ScanMatchParams match{};
@@ -319,6 +323,8 @@ void free_all(slamrs_gpu_handle* h) {
     cudaFree(h->d_kld);
     if (h->h_kld) cudaFreeHost(h->h_kld);
     if (h->ev_kld) cudaEventDestroy(h->ev_kld);
+    cudaFree(h->d_cl);
+    if (h->h_cl) cudaFreeHost(h->h_cl);
     cudaFree(h->d_wnorm); cudaFree(h->d_cum); cudaFree(h->d_idx); cudaFree(h->d_fold); cudaFree(h->d_carry);
     cudaFree(h->d_angle);   // (d_dist and d_valid live in the same allocation)
     if (h->h_scan_stage) cudaFreeHost(h->h_scan_stage);
@@ -1020,6 +1026,45 @@ int slamrs_gpu_get_kld_state(slamrs_gpu_handle* h, uint64_t out[3]) {
 int slamrs_gpu_get_population(slamrs_gpu_handle* h, uint64_t* out) {
     if (!h || !out) return SLAMRS_E_INVALID_ARG;
     *out = h->pop;
+    return SLAMRS_OK;
+}
+
+int slamrs_gpu_pose_clusters(slamrs_gpu_handle* h, const slamrs_gpu_clustering* c, slamrs_gpu_pose_stats* out,
+                             slamrs_gpu_pose_cluster* out_clusters) {
+    if (!h) return SLAMRS_E_INVALID_ARG;
+    if (!h->localizer)
+        return fail(h, SLAMRS_E_INVALID_ARG, "a SLAM handle has no pose clusters (only a localizer has them)");
+    if (!c || !out || !out_clusters) return fail(h, SLAMRS_E_INVALID_ARG, "null clustering, stats or clusters pointer");
+    if (c->struct_size != sizeof(slamrs_gpu_clustering))
+        return fail(h, SLAMRS_E_INVALID_ARG, "slamrs_gpu_clustering struct_size mismatch");
+    if (c->bin_cells < 1u) return fail(h, SLAMRS_E_INVALID_ARG, "clustering bin_cells must be >= 1");
+    if (c->theta_bins < 1u || c->theta_bins > 3600u)
+        return fail(h, SLAMRS_E_INVALID_ARG, "clustering theta_bins must lie in 1..3600");
+    if (c->max_clusters < 1u || c->max_clusters > CLUSTER_MAX_K)
+        return fail(h, SLAMRS_E_INVALID_ARG, "clustering max_clusters must lie in 1..64");
+    const uint64_t nb = ((uint64_t)h->geom.gw + c->bin_cells - 1u) / c->bin_cells;   // (square grid)
+    const uint64_t bin_space = nb * nb * c->theta_bins;
+    if (bin_space > (1ull << 28))
+        return fail(h, SLAMRS_E_INVALID_ARG, "clustering bin space above 2^28 bins: raise bin_cells or lower theta_bins");
+    DeviceGuard g(h->device);
+    const size_t bytes = cluster_scratch_bytes(h->n_total, bin_space);
+    if (!h->h_cl) CU_TRY(h, cudaMallocHost(&h->h_cl, sizeof(ClusterOutput)));
+    if (bytes > h->cl_bytes) {
+        CU_TRY(h, cudaStreamSynchronize(h->stream));   // no issued call still uses the old scratch
+        cudaFree(h->d_cl);
+        h->d_cl = nullptr;
+        h->cl_bytes = 0;
+        CU_TRY(h, cudaMalloc(&h->d_cl, bytes));
+        h->cl_bytes = bytes;
+    }
+    const KldParams bins{0u, 0u, 0.0, 0.0, c->bin_cells, c->theta_bins, (uint32_t)nb, (uint32_t)nb};
+    uint64_t launched = 0;
+    CU_TRY(h, launch_pose_clusters(h->stream, h->d_pose[h->cur], h->pop, h->n_total, h->geom, bins, c->max_clusters, h->d_cl,
+                                   h->h_cl, &launched));
+    h->launches += launched;
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    *out = h->h_cl->stats;
+    memcpy(out_clusters, h->h_cl->clusters, sizeof(slamrs_gpu_pose_cluster) * c->max_clusters);
     return SLAMRS_OK;
 }
 

@@ -18,9 +18,11 @@
 //                          k_loc_free_count / k_loc_free_scan / k_loc_free_cells   free-cell list at create
 //                          k_loc_recover   augmented-MCL recovery behind k_resample_indices (off by default)
 //                          k_loc_kld       KLD-sampling: bins of the starting generation and the next one's size (off by default)
+//   kernels_cluster.cu     k_cl_*          pose clusters of the localiser's generation (AMCL's pf_cluster_stats), on request
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/slamrs_gpu.h"
 #include "slam_device.cuh"
 
 namespace slamrs {
@@ -398,6 +400,24 @@ constexpr uint32_t KLD_HEADER_WORDS = 32;
 // (page-locked host memory)
 void launch_loc_kld(cudaStream_t stream, const float* pose, uint32_t n, MapGeom geom, const KldParams& kp, uint32_t* state,
                     KldResult* host_out);
+// counts[0, n_tiles) -> their exclusive prefix sums, in place (k_loc_free_scan: one CTA; the free-cell list's and the
+// pose clusters' ordered compactions)
+void launch_tile_offsets(cudaStream_t stream, uint32_t* counts, uint32_t n_tiles);
+
+// Pose clusters of the localiser's current generation (slamrs_gpu_pose_clusters, kernels_cluster.cu). The bins are
+// KLD-sampling's (bins.bin_cells, theta_bins, nbx, nby; the other fields are unused).
+constexpr uint32_t CLUSTER_MAX_K = 64;
+struct ClusterOutput {   // what the last kernel leaves in page-locked host memory
+    slamrs_gpu_pose_stats stats;
+    slamrs_gpu_pose_cluster clusters[CLUSTER_MAX_K];
+};
+// device scratch for `capacity` poses and a bin space of bin_space bins
+size_t cluster_scratch_bytes(uint32_t capacity, uint64_t bin_space);
+// the n poses of `pose` (n <= capacity) into *host_out; `k` clusters reported (1..CLUSTER_MAX_K); returns the number of
+// kernels launched through *launches
+cudaError_t launch_pose_clusters(cudaStream_t stream, const float* pose, uint32_t n, uint32_t capacity, MapGeom geom,
+                                 const KldParams& bins, uint32_t k, void* scratch, ClusterOutput* host_out,
+                                 uint64_t* launches);
 
 // test hooks
 void launch_debug_raycast(cudaStream_t stream, const float* x0, const float* y0, const float* x1, const float* y1,

@@ -200,6 +200,24 @@ __device__ __forceinline__ uint32_t block_compact_valid_beams(const ScanDevice& 
     return s_base;
 }
 
+// The bin of a pose (KLD-sampling's k_loc_kld and the pose clusters): the cell the likelihood would give a beam
+// endpoint at (x, y), coarsened to bin_cells x bin_cells cells, times theta_bins headings; every pose off the grid
+// shares the one bin nbx * nby * theta_bins.
+constexpr double KLD_TWO_PI = 0x1.921fb54442d18p+2;
+
+__device__ __forceinline__ uint32_t kld_bin(float x, float y, float theta, const MapGeom& geom, const KldParams& kp) {
+    const float gx = world_to_grid(x, geom.pos_x, geom.res);
+    const float gy = world_to_grid(y, geom.pos_y, geom.res);
+    if (!grid_is_valid(gx, gy, geom.gw, geom.gh)) return kp.nbx * kp.nby * kp.theta_bins;
+    const uint32_t cx = (uint32_t)f32_as_usize(gx), cy = (uint32_t)f32_as_usize(gy);
+    double t = fmod((double)theta, KLD_TWO_PI);   // (exact)
+    if (t < 0.0) t = __dadd_rn(t, KLD_TWO_PI);
+    uint32_t hb = 0;   // NaN / infinite headings, and a negative one that rounds up to 2 pi, fall into heading bin 0
+    if (t >= 0.0 && t < KLD_TWO_PI)
+        hb = min(kp.theta_bins - 1u, (uint32_t)__ddiv_rn(__dmul_rn(t, (double)kp.theta_bins), KLD_TWO_PI));
+    return ((cy / kp.bin_cells) * kp.nbx + cx / kp.bin_cells) * kp.theta_bins + hb;
+}
+
 struct alignas(32) V8 {
     uint4 a, b;
 };

@@ -227,6 +227,10 @@ void launch_loc_free_cells(cudaStream_t stream, const double* prob, size_t n_cel
     k_loc_free_cells<<<n_tiles, FREE_THREADS, 0, stream>>>(prob, n_cells, scratch, free_cells);
 }
 
+void launch_tile_offsets(cudaStream_t stream, uint32_t* counts, uint32_t n_tiles) {
+    k_loc_free_scan<<<1, FREE_THREADS, 0, stream>>>(counts, n_tiles);
+}
+
 // One thread per new particle, behind k_resample_indices. Every thread computes the same new state from the previous
 // step's (slot (step + 1) & 1); thread 0 stores it in slot step & 1 and clears the other slot's count for the next
 // step. With p > 0 a thread draws its particle's decision (slamrs_stream::recovery_draw) and replaces the resampled
@@ -268,23 +272,6 @@ void launch_loc_recover(cudaStream_t stream, uint32_t n, uint32_t m_draws, const
 }
 
 // =============================================================================== KLD-sampling (adaptive population)
-// The bin of a pose: the cell the likelihood would give a beam endpoint at (x, y), coarsened to bin_cells x bin_cells
-// cells, times theta_bins headings; every pose off the grid shares the one bin nbx * nby * theta_bins.
-constexpr double KLD_TWO_PI = 0x1.921fb54442d18p+2;
-
-__device__ __forceinline__ uint32_t kld_bin(float x, float y, float theta, const MapGeom& geom, const KldParams& kp) {
-    const float gx = world_to_grid(x, geom.pos_x, geom.res);
-    const float gy = world_to_grid(y, geom.pos_y, geom.res);
-    if (!grid_is_valid(gx, gy, geom.gw, geom.gh)) return kp.nbx * kp.nby * kp.theta_bins;
-    const uint32_t cx = (uint32_t)f32_as_usize(gx), cy = (uint32_t)f32_as_usize(gy);
-    double t = fmod((double)theta, KLD_TWO_PI);   // (exact)
-    if (t < 0.0) t = __dadd_rn(t, KLD_TWO_PI);
-    uint32_t hb = 0;   // NaN / infinite headings, and a negative one that rounds up to 2 pi, fall into heading bin 0
-    if (t >= 0.0 && t < KLD_TWO_PI)
-        hb = min(kp.theta_bins - 1u, (uint32_t)__ddiv_rn(__dmul_rn(t, (double)kp.theta_bins), KLD_TWO_PI));
-    return ((cy / kp.bin_cells) * kp.nbx + cx / kp.bin_cells) * kp.theta_bins + hb;
-}
-
 // The particle count of the next generation for k occupied bins: AMCL's pf_resample_limit in its order of operations
 // (n_min instead of max_particles for k <= 1).
 __device__ __forceinline__ uint32_t kld_bound(uint32_t k, const KldParams& kp) {

@@ -187,6 +187,35 @@ class Kld:
         return k
 
 
+@dataclass
+class Clustering:
+    """How GridMapLocalizer.pose_clusters groups the poses (slamrs_gpu_clustering; ROS AMCL's pf_cluster_stats): bins of
+    bin_xy metres (bin_cells = max(1, round(bin_xy / resolution)), as Kld) and theta_bins headings; occupied bins that
+    touch (3 x 3 x 3, the heading wrapping around) form a cluster. The defaults are AMCL's 0.5 m / 10 degree bins.
+    max_clusters (1..64) clusters are reported, the heaviest first."""
+    bin_xy: float = 0.5
+    theta_bins: int = 36
+    max_clusters: int = 16
+
+    def bin_cells(self, resolution: float) -> int:
+        return max(1, int(round(self.bin_xy / resolution)))
+
+    def to_struct(self, resolution: float):
+        c = _lib.Clustering()
+        c.struct_size = C.sizeof(_lib.Clustering)
+        c.bin_cells, c.theta_bins, c.max_clusters = self.bin_cells(resolution), int(self.theta_bins), int(self.max_clusters)
+        return c
+
+
+def _pose_cluster(c) -> dict:
+    """One slamrs_gpu_pose_cluster as a dict; `cov` is the 3 x 3 covariance as AMCL publishes it: x-y block, var_theta
+    at [2, 2], no theta-x or theta-y terms."""
+    cov = np.zeros((3, 3), np.float64)
+    cov[0, 0], cov[0, 1], cov[1, 0], cov[1, 1], cov[2, 2] = c.cov_xx, c.cov_xy, c.cov_xy, c.cov_yy, c.var_theta
+    return {"count": int(c.count), "label": int(c.label), "weight": float(c.weight),
+            "mean": np.array([c.mean[0], c.mean[1], c.mean[2]], np.float64), "cov": cov}
+
+
 def grid_cells(extent: float, resolution: float) -> int:
     """Map::new grid sizing (map.rs:28-31) as the library computes it."""
     out = C.c_uint32(0)
@@ -592,6 +621,25 @@ class GridMapLocalizer(GridMapSlam):
         out = C.c_uint64(0)
         _lib.check(self._L.slamrs_gpu_get_population(self._h, C.byref(out)), self._h)
         return int(out.value)
+
+    # ------------------------------------------------------------------ pose hypotheses (AMCL's cluster statistics)
+    def pose_clusters(self, clustering: Optional[Clustering] = None):
+        """Clusters of the current generation (the poses poses() returns, each of weight 1 / population), computed on
+        the device behind the updates issued so far; changes no filter state. Returns (overall, clusters):
+        overall = {n_poses, n_excluded (off the grid or not finite), n_bins, n_clusters, and the moments of every
+        non-excluded pose}; clusters = up to max_clusters dicts, heaviest first (ties: smallest label), each {count,
+        label (smallest bin id), weight, mean (x, y, theta), cov (3 x 3, as AMCL publishes it)}. clusters[0]['mean']
+        is the pose AMCL publishes."""
+        cl = clustering or Clustering()
+        c = cl.to_struct(self.config.resolution)
+        stats = _lib.PoseStats()
+        arr = (_lib.PoseCluster * max(1, int(cl.max_clusters)))()
+        _lib.check(self._L.slamrs_gpu_pose_clusters(self._h, C.byref(c), C.byref(stats), arr), self._h)
+        overall = _pose_cluster(stats.overall)
+        del overall["label"]
+        overall.update(n_poses=int(stats.n_poses), n_excluded=int(stats.n_excluded), n_bins=int(stats.n_bins),
+                       n_clusters=int(stats.n_clusters))
+        return overall, [_pose_cluster(arr[j]) for j in range(min(int(cl.max_clusters), int(stats.n_clusters)))]
 
     def update(self, z: Observation, u: Odometry, z_draws: Optional[np.ndarray] = None,
                resample_u: Optional[float] = None) -> None:
